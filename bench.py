@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the sknnr query-time hot path (kneighbors + predict, k=7) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[2], "C3"): EuclideanKNNRegressor, 10M query rows x
 50k reference plots x 32 features, k=7, predict(weights="distance") over 8 targets; synthetic
@@ -24,6 +24,11 @@ under the next chunks' kernels (default), or stored by the finishing kernels the
             Hamming search), each with its own roofline and CPU baseline.
 `cpu_baseline` / `--impl reference`: the UNMODIFIED reference package (oracle/_ref/sknnr, installed
             by __graft_entry__.build()) on the box's host cores, on a bounded sample.
+
+--steps K sets the number of timed steps of every leg.  --dump-outputs DIR writes, after each leg's
+timed steps, what its last step returned - (dist, idx, pred) of a fixed, seeded sample of rows and the
+sample's row numbers - as DIR/<leg>_<name>.npy in float64 (64 MB in all at most).  The inputs depend on
+the arguments only, so two builds can be compared output for output.
 """
 
 from __future__ import annotations
@@ -83,7 +88,13 @@ def parse_args():
     ap.add_argument("--gather", default="auto", choices=["auto", "fused", "copy"],
                     help="N > 1: how a rank's rows reach rank 0's arrays - fused = the finishing kernels store "
                          "over NVLink; copy = per-chunk copy-engine peer copies on the chunk's stream")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write a seeded sample of each leg's last timed step's results to DIR/<leg>_<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes what this project's timed path returns; --impl reference has no such path")
     if a.gather == "auto":
         # measured on 8 GPUs (profiles/r02_multi_gpu_gather.md): copy 83.4 ms per step against 88.6 fused and
         # 82.4 on one GPU - the ranks run in step, so seven ranks' finishing kernels store into rank 0 at
@@ -360,6 +371,21 @@ class SharedResults:
                                                 C.c_void_p(self.ptr(i, rank)), out.nbytes, 2, None))
         return out
 
+    def rows_to_host(self, rows, k, n_out):
+        """(dist, idx, pred) of the job-wide row numbers `rows`, gathered on the device so that only those
+        rows are copied (rank 0 only).  The arrays are the library's allocations, seen by torch through the
+        CUDA array interface."""
+        import torch
+
+        sel = torch.from_numpy(rows).to(torch.device("cuda", self.dev))
+        out = []
+        for i, typestr, width in ((0, "<f8", k), (1, "<i8", k), (2, "<f8", n_out)):
+            iface = {"data": (self.base[i].value, False), "shape": (self.world * self.rows, width),
+                     "typestr": typestr, "strides": None, "version": 3}
+            whole = torch.as_tensor(type("LibraryArray", (), {"__cuda_array_interface__": iface})())
+            out.append(whole[sel].cpu().numpy())
+        return out
+
     def close(self):
         for i in range(3):
             if self.base[i].value:
@@ -368,6 +394,23 @@ class SharedResults:
                 else:
                     self.lib.sknnr_device_free(self.dev, self.base[i])
                 self.base[i] = C.c_void_p(None)
+
+
+DUMP_BYTES = {"c3": 32_000_000, "c5": 15_000_000, "c4": 15_000_000}     # --dump-outputs: under 64 MB in all
+
+
+def dump_outputs(a, leg, n_rows, k, n_out, fetch):
+    """--dump-outputs: DIR/<leg>_{rows,dist,idx,pred}.npy for a fixed, seeded sample of the `n_rows` result
+    rows (all of them when they fit DUMP_BYTES[leg]); `fetch(rows)` returns (dist, idx, pred) of those rows.
+    Everything is stored as float64 (indices and row numbers are exact in it)."""
+    m = DUMP_BYTES[leg] // (8 * (1 + 2 * k + n_out))
+    if m >= n_rows:
+        rows = np.arange(n_rows)
+    else:
+        rows = np.unique(np.random.default_rng(20261020).integers(0, n_rows, size=m))
+    os.makedirs(a.dump_outputs, exist_ok=True)
+    for name, arr in zip(("rows", "dist", "idx", "pred"), (rows, *fetch(rows))):
+        np.save(os.path.join(a.dump_outputs, f"{leg}_{name}.npy"), np.asarray(arr, dtype=np.float64))
 
 
 def measure_gemm_peaks(dev):
@@ -572,6 +615,8 @@ def bench_c3(a, rank, world, local_rank, dev, stream, lib, L, KNNIndex, barrier,
     clocks = sampler.stop() if rank == 0 else None
     value = world * n_q * a.steps / (ms_total * 1e-3)
     barrier()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a, "c3", world * n_q, k, n_out, lambda rows: shared.rows_to_host(rows, k, n_out))
     headline_launches = int(index.stats()["kernel_launches"])   # of one headline step (this rank)
 
     # out-of-band verification of the fused gather: every rank repeats its block into local memory and
@@ -637,7 +682,7 @@ def bench_c3(a, rank, world, local_rank, dev, stream, lib, L, KNNIndex, barrier,
         step_host()
         barrier()
         t0 = time.perf_counter()
-        e2e_steps = max(1, min(a.steps, 3))
+        e2e_steps = a.steps
         for _ in range(e2e_steps):
             step_host()
         barrier()
@@ -661,7 +706,7 @@ def bench_c3(a, rank, world, local_rank, dev, stream, lib, L, KNNIndex, barrier,
             pred = est.predict(X_np)
         barrier()
         t0 = time.perf_counter()
-        est_steps = max(1, min(a.steps, 3))
+        est_steps = a.steps
         per_call = []
         for _ in range(est_steps):
             t1 = time.perf_counter()
@@ -758,8 +803,12 @@ def bench_c5(a, rank, world, local_rank, dev, stream, lib, L, barrier, timed, pe
                            pred_ptr=shared.ptr(2), weights="distance", row_offset=lo, stream=stream.cuda_stream)
 
     step()
-    steps = max(1, min(a.steps, 2))
+    steps = a.steps
     ms = timed(step, steps)
+    if a.dump_outputs:
+        if rank == 0:
+            dump_outputs(a, "c5", total, k, n_out, lambda rows: shared.rows_to_host(rows, k, n_out))
+        barrier()      # the next step() of the other ranks stores into the arrays read here
     step()
     barrier()
     st = index.stats()
@@ -855,8 +904,11 @@ def bench_c4(a, rank, world, local_rank, dev, stream, lib, L, barrier, timed, di
             L.W_UNIFORM, C.c_void_p(o_pred.data_ptr()), C.c_void_p(stream.cuda_stream)))
 
     step()
-    steps = max(1, min(a.steps, 2))
+    steps = a.steps
     ms = timed(step, steps)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a, "c4", n_q, k, n_t, lambda rows: [t[torch.from_numpy(rows).to(dev)].cpu().numpy()
+                                                         for t in (o_dist, o_idx, o_pred)])
     step()
     barrier()
     st = index.stats()

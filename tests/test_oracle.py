@@ -225,7 +225,7 @@ def test_oracle_matches_installed_reference_on_fresh_random_data(est_name, weigh
     state from the reference's own transformer, so what is compared is the query-time path."""
     sknnr = _installed_reference()
     if sknnr is None:
-        pytest.skip("oracle/_ref is not installed (run __graft_entry__.build() where /root/reference exists)")
+        pytest.skip("the unmodified reference package is not installed under oracle/_ref/sknnr")
     rng = np.random.default_rng(20260)
     n_ref, d, n_out, k = 600, 6, 3, 5
     A = rng.standard_normal((d, d))
@@ -266,7 +266,7 @@ def test_hamming_oracle_matches_installed_reference_on_fresh_forests(est_name):
     order) and tie-aware equal neighbours, for target rows and for the X=None self-query."""
     sknnr = _installed_reference()
     if sknnr is None:
-        pytest.skip("oracle/_ref is not installed (run __graft_entry__.build() where /root/reference exists)")
+        pytest.skip("the unmodified reference package is not installed under oracle/_ref/sknnr")
     rng = np.random.default_rng(7)
     n_ref, d, k = 250, 5, 5
     R = rng.standard_normal((n_ref, d))
@@ -297,3 +297,95 @@ def test_hamming_oracle_matches_installed_reference_on_fresh_forests(est_name):
     same = (oi == ri).all(axis=1)
     assert same.sum() >= 20
     np.testing.assert_allclose(orc.predict(st, ids_q, k=k)[same], rp[same], rtol=1e-12)
+
+
+def _fresh_float_data():
+    rng = np.random.default_rng(20260)
+    n_ref, d, n_out = 600, 6, 3
+    A = rng.standard_normal((d, d))
+    R = rng.standard_normal((n_ref, d)) @ A + rng.standard_normal(d) * 3.0
+    R[50:60] = R[40:50]                                   # duplicated plots: exact distance ties
+    y = rng.standard_normal((n_ref, n_out))
+    Q = rng.standard_normal((400, d)) @ A
+    Q[:20] = R[100:120]                                   # queries on top of plots: zero distances
+    return R, y, Q
+
+
+@pytest.mark.parametrize(("transformer", "weights"), [
+    ("StandardScalerWithDOF", "distance"), ("StandardScalerWithDOF", "uniform"),
+    ("MahalanobisTransformer", "distance"), (None, "uniform"),
+])
+def test_oracle_matches_scikit_learn_on_fresh_random_data(transformer, weights):
+    """The data of test_oracle_matches_installed_reference_on_fresh_random_data without the reference
+    package: the oracle against scikit-learn's brute KNeighborsRegressor, the code the reference hands its
+    transformed plots to (ref:src/sknnr/_base.py:162-164), on the same feature space.  Ties between
+    duplicated plots, zero distances under weights='distance' and the X=None self-query."""
+    from sklearn.neighbors import KNeighborsRegressor
+
+    import sknnr_b200.transformers as T
+
+    R, y, Q = _fresh_float_data()
+    k = 5
+    center = scale = proj = None
+    if transformer is not None:
+        kw = {"ddof": 1} if transformer == "StandardScalerWithDOF" else {}
+        center, scale, proj, _ = getattr(T, transformer)(**kw).fit(R, y)._affine()
+    st = orc.FittedState(kind="euclidean", fit_Z=orc.affine_project(R, center, scale, proj), y=y,
+                         center=center, scale=scale, proj=proj)
+    skl = KNeighborsRegressor(n_neighbors=k, weights=weights, algorithm="brute").fit(st.fit_Z, y)
+    Zq = orc.affine_project(Q, center, scale, proj)
+    for X, Z in ((Q, Zq), (None, None)):
+        rd, ri = skl.kneighbors(Z)
+        od, oi = orc.kneighbors(st, X, k, deterministic=False)
+        orc.assert_tie_aware_equal(od, oi, rd, ri, rtol=1e-7, atol=5e-7)
+        # scikit-learn leaves the order of exactly tied plots to its heap: only duplicated plots may trade places
+        assert np.isin(oi[oi != ri], np.r_[40:60]).all()
+    rp = skl.predict(Zq)
+    op = orc.predict(st, Q, k, weights=weights, deterministic=False)
+    ok = np.isclose(op, rp, rtol=1e-6, atol=1e-6).all(axis=1)
+    assert (~ok).sum() <= 12, int((~ok).sum())
+    assert ok[:20].all()
+
+
+@pytest.mark.parametrize("est_name", ["RFNNRegressor", "GBNNRegressor"])
+def test_hamming_oracle_matches_scikit_learn_on_fresh_forests(est_name):
+    """The forests of test_hamming_oracle_matches_installed_reference_on_fresh_forests without the
+    reference package: node IDs from scikit-learn's own Tree.apply, tree weights from this package's
+    fit side (pinned against the reference in test_host.py), and the oracle against scikit-learn's brute
+    weighted-Hamming KNeighborsRegressor - bit-equal distances, tie-aware neighbours, X=None included."""
+    import warnings
+
+    from sklearn.neighbors import KNeighborsRegressor
+
+    import sknnr_b200 as S
+
+    rng = np.random.default_rng(7)
+    n_ref, d, k = 250, 5, 5
+    R = rng.standard_normal((n_ref, d))
+    y = np.column_stack([R[:, 0] + 0.3 * rng.standard_normal(n_ref), R[:, 1] * R[:, 2], rng.standard_normal(n_ref)])
+    Q = rng.standard_normal((120, d))
+    est = getattr(S, est_name)(n_neighbors=k, n_estimators=12 if est_name == "RFNNRegressor" else 8, random_state=3)
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore", FutureWarning)
+        est.transformer_ = est._get_transformer().fit(R, y)
+    w = est._get_hamming_weights()
+    trees = est.transformer_._trees()
+    ids_ref = np.stack([t.apply(R.astype(np.float32)) for t in trees], axis=1).astype(np.int64)
+    ids_q = np.stack([t.apply(Q.astype(np.float32)) for t in trees], axis=1).astype(np.int64)
+    assert ids_ref.shape[1] == len(w) and abs(w.sum() - 1.0) < 1e-9
+    if est_name == "GBNNRegressor":
+        assert len(np.unique(w)) > 3   # genuinely unequal weights
+    st = orc.FittedState(kind="hamming", fit_Z=ids_ref, y=y, hamming_w=w)
+    skl = KNeighborsRegressor(n_neighbors=k, metric="hamming", metric_params={"w": w}, algorithm="brute").fit(ids_ref, y)
+    for X, ids in ((ids_q, ids_q), (None, None)):
+        rd, ri = skl.kneighbors(ids)
+        od, oi = orc.kneighbors(st, X, k=k, deterministic=False)
+        assert np.array_equal(od, rd)
+        orc.assert_tie_aware_equal(od, oi, rd, ri, rtol=0, atol=0, gap_rtol=0)
+    rd, ri = skl.kneighbors(ids_q)
+    od, oi = orc.kneighbors(st, ids_q, k=k, deterministic=False)
+    rp = skl.predict(ids_q)
+    np.testing.assert_allclose(orc.weighted_average(y, ri), rp, rtol=1e-12)
+    same = (oi == ri).all(axis=1)
+    assert same.sum() >= 20
+    np.testing.assert_allclose(orc.predict(st, ids_q, k=k, deterministic=False)[same], rp[same], rtol=1e-12)
