@@ -91,8 +91,7 @@ int sknnr_device_count(int *count);
 /* Global knobs (environment-style; never estimator constructor arguments):
  *   "engine"      SKNNR_ENGINE_*           (default AUTO)
  *   "chunk_rows"  rows per internal chunk  (default 1<<20; device-pointer calls use twice that)
- *   "host_slots"  chunks of a host-buffer call in flight, 1..8 (default 8: measured 60 / 71 / 76 /
- *                 82 M queries/s with 2 / 3 / 4 / 8; 12 or 16 are slower again)
+ *   "host_slots"  1..8: a host-buffer call keeps min(4, value) chunks in flight (default 8)
  *   "timing"      0/1 record search_ms     (default 0)
  *   "kc"          0/8/16/32 minimum length of the FP32 (SIMT) search's candidate list (default 16);
  *                 0 picks the smallest list that holds k+1 (longer lists = fewer certificate
@@ -102,23 +101,6 @@ int sknnr_device_count(int *count);
  *   "tc_seed_stride" 0..64: the tensor engine pre-scans one reference tile in n to seed its
  *                 thresholds (default 4; 0 = the default too: the engine never starts cold, and
  *                 reference sets below 192 / 64 tiles are pre-scanned at stride <= 2 / 1)
- *   "tail_priority" 0/1 the cascade's tail streams (second pass, FP32 and exhaustive stages of the uncertified
- *                 rows) get the highest stream priority; read when an index is created (default 1)
- *   "host_nt"     0/1 staging copies of pageable caller buffers use streaming (non-temporal) stores (default 1)
- *   "host_pipeline" 0/1 host-buffer calls run as a three-stage pipeline: one in-order H2D stream, one compute
- *                 stream, one D2H stream over up to four slots of buffers (default 1); 0: every chunk in
- *                 flight has a stream of its own for copies and kernels (round 1's layout)
- *   "simt_min_rows" 0..2^20: when fewer rows than this are still uncertified after the tensor engine,
- *                 they skip the FP32 engine (one warp would scan the whole reference set for them)
- *                 and go to the exhaustive float64 kernel (default 256)
- *   "tc_retry"    0/1 after its two-stream layout (k (+1) <= 7) the tensor engine runs a second pass,
- *                 one stream of 16, over the rows the first pass could not certify, each from the
- *                 threshold the first pass proved sufficient, before the FP32 engine sees what is
- *                 left (default 1)
- *   "tail_spread" 0/1 the second (FP32) stage of the cascade deals its few rows out over all SMs,
- *                 one warp of 32 rows at a time (default 1; 0 = one CTA per 384 rows)
- *   "host_threads" workers that stage pageable caller buffers through page-locked slot buffers
- *                 (default 0 = min(16, 3/4 of the cores); read when the first pageable call starts them)
  *   "stage_rows"  rows per chunk of a call with pageable buffers (default 1<<19)
  *   "tc_debug"    timing experiments only (bit 0 skips the hit path, bit 2 skips the tile
  *                 loads: results are wrong)                                             */
@@ -165,7 +147,7 @@ int sknnr_index_destroy(sknnr_index *index);
  * Without SKNNR_DEVICE_PTRS the call is synchronous and every pointer may be a pageable host,
  * page-locked host or device pointer (unified addressing; a peer GPU's memory mapped with
  * sknnr_ipc_open included): device-resident X is read in place, results bound for device memory
- * leave each chunk as one copy-engine transfer on the chunk's stream.                          */
+ * leave each chunk as one copy-engine transfer.                                               */
 int sknnr_kneighbors(sknnr_index *index, const void *X, int32_t x_dtype, int64_t n_q,
                      int64_t ldx, int64_t row_offset, int32_t k, uint32_t flags,
                      int32_t decimals, double *out_dist, int64_t *out_idx, int32_t weights,

@@ -44,7 +44,7 @@ def _stale(target: str, deps: list[str]) -> bool:
 
 
 def build(verbose: bool = False, force: bool = False, variant: str = "", extra_flags=()) -> str:
-    """``variant``: build into lib/libsknnr_b200_<variant>.so with ``extra_flags`` (e.g. -DSK_TC_JOINT=10)."""
+    """``variant``: build into lib/libsknnr_b200_<variant>.so with ``extra_flags`` (e.g. -DSK_CHECKS)."""
     nvcc = nvcc_path()
     objdir = os.path.join(HERE, "build" + ("_" + variant if variant else ""))
     os.makedirs(objdir, exist_ok=True)

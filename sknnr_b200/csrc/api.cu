@@ -50,15 +50,8 @@ struct Options {
     int64_t timing = 0;
     int64_t kc = 16; // minimum candidate-list length of the float search (0 = smallest that fits k+1)
     int64_t tc_streams = 0;     // tensor engine: candidate streams per query (0 = automatic, else 1 or 2)
-    int64_t host_slots = 8;     // chunks of a host-buffer call in flight (1..8)
-    int64_t tail_priority = 1;  // the slots' tail streams are created with the highest stream priority (read at index creation)
-    int64_t host_nt = 1;        // staging copies of pageable buffers use streaming stores
-    int64_t host_pipeline = 1;  // host-buffer calls: one compute stream fed by an in-order H2D stream, drained by a D2H stream
-    int64_t simt_min_rows = 256; // cascade: fewer uncertified rows than this skip the FP32 engine (exhaustive kernel instead)
-    int64_t tc_retry = 1;       // tensor engine: second pass over the uncertified rows before the FP32 stage
-    int64_t tail_spread = 1;    // second stage: deal the uncertified rows out over all SMs (0: one CTA per 384 rows)
+    int64_t host_slots = 8;     // a host-buffer call keeps min(4, host_slots) chunks in flight (1..8)
     int64_t tc_seed_stride = 4; // tensor engine: pre-scan every n-th reference tile to seed thresholds (0 = default)
-    int64_t host_threads = 0;   // workers that stage pageable host buffers (0 = automatic)
     int64_t stage_rows = 1 << 19; // rows per chunk of a call whose buffers are pageable
 } g_opt;
 
@@ -96,11 +89,8 @@ public:
     int size() const { return (int)th_.size(); }
     static HostPool &get() {
         static HostPool *pool = [] {
-            int n = (int)g_opt.host_threads;
-            if (n <= 0) {
-                const unsigned hw = std::thread::hardware_concurrency();
-                n = (int)std::min(16u, std::max(2u, hw * 3 / 4));
-            }
+            const unsigned hw = std::thread::hardware_concurrency();
+            const int n = (int)std::min(16u, std::max(2u, hw * 3 / 4));
             return new HostPool(n - 1);   // the calling thread takes a share as well
         }();
         return *pool;
@@ -134,7 +124,7 @@ public:
 // line, a third of the copy's memory traffic (8 threads on the build host: 21 -> 27 GB/s).
 void stream_copy(unsigned char *d, const unsigned char *s, size_t n) {
 #if defined(__SSE2__)
-    if (g_opt.host_nt && n >= (256u << 10)) {
+    if (n >= (256u << 10)) {
         while (n && ((uintptr_t)d & 15)) { *d++ = *s++; --n; }
         for (size_t i = n / 64; i; --i, s += 64, d += 64) {
             const __m128i a = _mm_loadu_si128((const __m128i *)s), b = _mm_loadu_si128((const __m128i *)(s + 16));
@@ -253,7 +243,6 @@ struct DevBuf {
 // per-chunk device buffers + the stream the chunk runs on
 struct Slot {
     cudaStream_t stream = nullptr;
-    bool own_stream = false;
     // the cascade's tail (SIMT re-search + exhaustive search of uncertified rows) runs on its own
     // stream so that a handful of slow CTAs overlap the next chunk's first stage
     cudaStream_t tail_stream = nullptr;
@@ -291,10 +280,11 @@ struct Slot {
     long long rows_in_flight = 0;
     DevBuf<int> nonfinite;         // [0] != 0: a query value of the chunk in flight is NaN / inf
     bool flag_pending = false;
-    // device-pointer calls are not synchronised: the slot's scratch stays in use until ev_last
+    // the slot's scratch stays in use until ev_last (the D2H of a host-buffer call's chunk, the end of a
+    // device-pointer call's chunk on the caller's stream: such calls are not synchronised)
     cudaEvent_t ev_last = nullptr;
     bool last_pending = false;
-    // host-buffer calls (pipelined): the chunk's input has arrived / its first stage is through
+    // host-buffer calls: the chunk's input has arrived / its first stage is through
     cudaEvent_t ev_in = nullptr, ev_out = nullptr;
     // page-locked staging of pageable caller buffers (one chunk in, one chunk out) and the copy-out
     // that is still owed to the caller once the slot's stream has drained
@@ -322,7 +312,7 @@ struct Slot {
         if (ev_in) cudaEventDestroy(ev_in);
         if (ev_out) cudaEventDestroy(ev_out);
         ev_in = ev_out = nullptr;
-        if (own_stream && stream) cudaStreamDestroy(stream);
+        if (stream) cudaStreamDestroy(stream);
         if (tail_stream) cudaStreamDestroy(tail_stream);
         if (ev_stage1) cudaEventDestroy(ev_stage1);
         if (ev_tail) cudaEventDestroy(ev_tail);
@@ -393,10 +383,9 @@ struct IndexBase {
         CK(cudaStreamCreateWithFlags(&d2h_stream, cudaStreamNonBlocking));
         for (auto &s : slots) {
             CK(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
-            s.own_stream = true;
             // (the tail's few CTAs go ahead of the thousands the next chunk's first stage has queued:
             // the chunk's results are complete, and its slot free, a whole first stage earlier)
-            CK(cudaStreamCreateWithPriority(&s.tail_stream, cudaStreamNonBlocking, g_opt.tail_priority ? prio_hi : prio_lo));
+            CK(cudaStreamCreateWithPriority(&s.tail_stream, cudaStreamNonBlocking, prio_hi));
             CK(cudaEventCreateWithFlags(&s.ev_stage1, cudaEventDisableTiming));
             CK(cudaEventCreateWithFlags(&s.ev_tail, cudaEventDisableTiming));
             CK(cudaHostAlloc((void **)&s.h_fb, 4 * sizeof(int), cudaHostAllocDefault));
@@ -673,25 +662,9 @@ int sknnr_set_option(const char *name, int64_t value) {
     } else if (!strcmp(name, "host_slots")) {
         if (value < 1 || value > IndexBase::kSlots) return fail(SKNNR_EINVAL, "host_slots must be 1..8");
         g_opt.host_slots = value;
-    } else if (!strcmp(name, "host_threads")) {
-        if (value < 0 || value > 64) return fail(SKNNR_EINVAL, "host_threads must be 0..64");
-        g_opt.host_threads = value;   // read when the staging pool starts (first pageable call)
     } else if (!strcmp(name, "stage_rows")) {
         if (value < 1024) return fail(SKNNR_EINVAL, "stage_rows must be >= 1024");
         g_opt.stage_rows = (value + 1023) / 1024 * 1024;
-    } else if (!strcmp(name, "tail_priority")) {
-        g_opt.tail_priority = value ? 1 : 0;
-    } else if (!strcmp(name, "host_nt")) {
-        g_opt.host_nt = value ? 1 : 0;
-    } else if (!strcmp(name, "host_pipeline")) {
-        g_opt.host_pipeline = value ? 1 : 0;
-    } else if (!strcmp(name, "simt_min_rows")) {
-        if (value < 0 || value > (1 << 20)) return fail(SKNNR_EINVAL, "simt_min_rows must be 0..2^20");
-        g_opt.simt_min_rows = value;
-    } else if (!strcmp(name, "tc_retry")) {
-        g_opt.tc_retry = value ? 1 : 0;
-    } else if (!strcmp(name, "tail_spread")) {
-        g_opt.tail_spread = value ? 1 : 0;
     } else if (!strcmp(name, "tc_seed_stride")) {
         if (value < 0 || value > 64) return fail(SKNNR_EINVAL, "tc_seed_stride must be 0..64");
         g_opt.tc_seed_stride = value;
@@ -1025,12 +998,12 @@ static int run_chunk(sknnr_index *ix, Slot &s, const void *dX, int x_f32, int64_
         int ns = kk <= 7 ? 2 : 1;   // a stream's list keeps at most 7 (ns = 2) / 15 (ns = 1) candidates
         if (g_opt.tc_streams == 1) ns = 1;
         CK(launch_search_tc(s.qimg_tc.p, ix->d_rimg_tc, ix->kc_tot, ix->n_rtiles_tc, rows, ns, ix->tc_nstage,
-                            (int)g_opt.tc_seed_stride, ix->tc_wide_joint || g_opt.tc_retry == 0, s.cand_idx.p,
+                            (int)g_opt.tc_seed_stride, ix->tc_wide_joint, s.cand_idx.p,
                             s.cand_thr.p, nullptr, nullptr, st));
         if (g_opt.timing) CK(s.mark(st));
         // (a second pass only pays after the two-stream layout: its joint list holds 11 candidates, the
         // second pass's single stream 15 - the one-stream layout would meet the same 15 again)
-        const bool retry = g_opt.tc_retry != 0 && ns == 2;
+        const bool retry = ns == 2;
         if (retry) {
             CK(s.fb_thr.reserve((size_t)rows));
             CK(s.fbm.reserve((size_t)rows + 1));
@@ -1097,10 +1070,11 @@ static int run_chunk(sknnr_index *ix, Slot &s, const void *dX, int x_f32, int64_
     // stage 2 (or the only fast stage): FP32 SIMT engine
     if (g_opt.timing && !use_tc) CK(s.mark(st));
     // (a handful of rows is not worth a scan of the whole reference set by one warp per row block: below
-    // simt_min_rows the stage passes its rows straight on to the exhaustive kernel)
-    const int bypass = stage2_count ? (int)g_opt.simt_min_rows : 0;
+    // kSimtMinRows the stage passes its rows straight on to the exhaustive kernel)
+    constexpr int kSimtMinRows = 256;
+    const int bypass = stage2_count ? kSimtMinRows : 0;
     CK(launch_search_simt(s.qimg.p, ix->d_rimg, ix->dpad, ix->n_rtiles, rows, kc, s.cand_idx.p,
-                          s.cand_thr.p, stage2_count, g_opt.tail_spread && ix->spread_tail ? ix->n_sm : 0, bypass, st));
+                          s.cand_thr.p, stage2_count, ix->spread_tail ? ix->n_sm : 0, bypass, st));
     if (g_opt.timing && !use_tc) CK(s.mark(st));
     FinishParams fp2 = fp;
     fp2.row_map = stage2_list;
@@ -1167,8 +1141,8 @@ int sknnr_kneighbors(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_
     const size_t esz = x_dtype == SKNNR_F32 ? 4 : 8;
     // A synchronous call takes any mix of host and device pointers (unified addressing): device
     // resident X is read in place, and results bound for device memory - this GPU's or a peer's
-    // mapped through sknnr_ipc_open - leave each chunk as one copy-engine transfer on the chunk's
-    // slot stream, under the kernels of the following chunks.
+    // mapped through sknnr_ipc_open - leave each chunk as one copy-engine transfer on the D2H
+    // stream, under the kernels of the following chunks.
     if (!dev_ptrs && !x_on_device && is_device_ptr(X)) x_on_device = true;
 
     cudaStream_t user_stream = dev_ptrs ? (cudaStream_t)stream : nullptr;
@@ -1202,8 +1176,7 @@ int sknnr_kneighbors(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_
     // tails; measured +1.8 %), while host buffers prefer the shorter pipeline ramp of the smaller one
     int64_t chunk = dev_ptrs ? 2 * g_opt.chunk_rows : (staged ? std::min(g_opt.stage_rows, g_opt.chunk_rows) : g_opt.chunk_rows);
     chunk = std::min<int64_t>(chunk, (n_q + 255) / 256 * 256);
-    const bool piped = !dev_ptrs && g_opt.host_pipeline != 0;
-    const int n_slots = dev_ptrs ? 2 : (staged || piped ? std::min<int>(4, (int)g_opt.host_slots) : (int)g_opt.host_slots);
+    const int n_slots = dev_ptrs ? 2 : std::min<int>(4, (int)g_opt.host_slots);
     // Host buffers: the first chunk's H2D copy and the last chunk's D2H copy cannot overlap any
     // kernel, so the stream of chunks ramps up (1/4, 1/2, 1, ...) and down (..., 1/2, 1/4).
     const bool ramp = ramp_applies(dev_ptrs, n_q, chunk);
@@ -1240,12 +1213,12 @@ int sknnr_kneighbors(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_
                 ix->tensor_demoted[ix->ns_in_use] = true;
         }
         // (the chunk's kernels run on the caller's stream / the pipeline's compute stream, lent to the slot)
-        StreamLoan loan(s, piped ? ix->host_compute : user_stream, dev_ptrs || piped);
+        StreamLoan loan(s, dev_ptrs ? user_stream : ix->host_compute, true);
         if (dev_ptrs && s.tail_pending) {   // the slot's buffers are free once its previous tail is done
             CK(cudaStreamWaitEvent(user_stream, s.ev_tail, 0));
             s.tail_pending = false;
         }
-        const cudaStream_t cin = piped ? ix->h2d_stream : s.stream, cout = piped ? ix->d2h_stream : s.stream;
+        const cudaStream_t cin = ix->h2d_stream, cout = ix->d2h_stream;
         const void *dX;
         int64_t dld = ldx;
         if (tracing) {
@@ -1268,10 +1241,8 @@ int sknnr_kneighbors(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_
                 CK(cudaMemcpy2DAsync(s.x.p, (size_t)cols * esz, src, (size_t)ldx * esz, (size_t)cols * esz,
                                      (size_t)rows, cudaMemcpyDefault, cin));
             }
-            if (piped) {
-                CK(cudaEventRecord(s.ev_in, cin));
-                CK(cudaStreamWaitEvent(s.stream, s.ev_in, 0));
-            }
+            CK(cudaEventRecord(s.ev_in, cin));
+            CK(cudaStreamWaitEvent(s.stream, s.ev_in, 0));
             ix->stats.h2d_bytes += rows * cols * (int64_t)esz;
             dX = s.x.p;
             dld = cols;
@@ -1295,10 +1266,9 @@ int sknnr_kneighbors(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_
                        flags, decimals, weights, o_dist, o_idx, o_pred, check_finite);
         if (rc != SKNNR_OK) return rc;
         if (!dev_ptrs) {
-            if (piped) {   // the D2H stream picks the results up behind the first stage and the slot's tail
-                CK(cudaEventRecord(s.ev_out, s.stream));
-                CK(cudaStreamWaitEvent(cout, s.ev_out, 0));
-            }
+            // the D2H stream picks the results up behind the first stage and the slot's tail
+            CK(cudaEventRecord(s.ev_out, s.stream));
+            CK(cudaStreamWaitEvent(cout, s.ev_out, 0));
             if (s.tail_pending) CK(cudaStreamWaitEvent(cout, s.ev_tail, 0));  // results complete
             CK(trace_mark(2, cout));
             // D2H straight into page-locked caller memory, else into the slot's staging buffer (the
@@ -1318,14 +1288,11 @@ int sknnr_kneighbors(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_
             if (out_idx) CK(deliver(out_idx + r0 * k, o_idx, (size_t)rows * k * 8, stage_idx, s.h_idx));
             if (o_pred) CK(deliver(out_pred + r0 * ix->n_out, o_pred, (size_t)rows * ix->n_out * 8, stage_pred, s.h_pred));
             CK(trace_mark(3, cout));
-            if (piped) {   // what finish_slot waits for before the slot's buffers are reused
-                CK(cudaEventRecord(s.ev_last, cout));
-                s.last_pending = true;
-            }
+            CK(cudaEventRecord(s.ev_last, cout));
         } else {
             CK(cudaEventRecord(s.ev_last, user_stream));
-            s.last_pending = true;
         }
+        s.last_pending = true;   // the slot's buffers are free for reuse once ev_last has passed
     }
     if (!dev_ptrs) {
         for (auto &s : ix->slots) CK(ix->finish_slot(s));

@@ -24,10 +24,7 @@ namespace sk {
 
 constexpr int FOREST_THREADS = 256;  // queries per CTA
 constexpr int FOREST_TG = 32;        // trees per staging group
-#ifndef SK_FOREST_ILP
-#define SK_FOREST_ILP 2
-#endif
-constexpr int FOREST_ILP = SK_FOREST_ILP;   // trees walked concurrently by one thread
+constexpr int FOREST_ILP = 2;        // trees walked concurrently by one thread
 
 template <typename TX>
 __global__ void __launch_bounds__(FOREST_THREADS)

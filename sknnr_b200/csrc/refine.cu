@@ -96,15 +96,7 @@ __device__ __forceinline__ double sqrt_padded(double d2) {
 // top k has approximate score <= (kth - |q|^2 + E) / thr_scale, E = eps_s (|q|^2 + max|r|^2).  A second pass
 // that lists everything below a threshold a hair above that (rounded up to float) finds all of them, and
 // its own certificate  kth' < thr * thr_scale + |q|^2 - E  then holds because kth' <= kth.
-#ifdef SK_RETRY_STATS
-__device__ unsigned long long g_retry_stats[4];
-#endif
 __device__ __forceinline__ float retry_threshold(double kth, double qn, const RefineArgs &a) {
-#ifdef SK_RETRY_STATS
-    atomicAdd(&g_retry_stats[0], 1ull);
-    if (!(kth < SK_INF_D)) atomicAdd(&g_retry_stats[1], 1ull);
-    if (!(qn < a.qn_limit)) atomicAdd(&g_retry_stats[2], 1ull);
-#endif
     if (!(kth < SK_INF_D)) return SK_INF_F;   // fewer than k candidates so far (or NaN): start cold
     const double span = qn + a.r2max;
     double t = (kth - qn + a.eps_s * span) / a.thr_scale;
@@ -285,12 +277,6 @@ refine2_kernel(RefineArgs a, FinishParams fp) {
     finish_query_w<16>(fp, q, sqrt_padded(d2), id, hl, live && ok);
 }
 
-#ifdef SK_RETRY_STATS
-extern "C" void sk_retry_stats(unsigned long long *out) {
-    cudaDeviceSynchronize();
-    cudaMemcpyFromSymbol(out, g_retry_stats, sizeof(g_retry_stats));
-}
-#endif
 cudaError_t launch_refine(const RefineArgs &a, const FinishParams &fp, cudaStream_t st) {
     if (a.n_q <= 0) return cudaSuccess;
     if (a.kc <= 16 && a.d <= 64) {

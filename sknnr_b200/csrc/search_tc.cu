@@ -88,22 +88,9 @@ __device__ unsigned long long g_tc_counters[8];
 
 // rank (in the union of both streams' lists) of the score the joint threshold is set to: the k-th
 // neighbour must clear it by the certificate's error margin, so it sits a few ranks above k
-#ifndef SK_TC_JOINT
-#define SK_TC_JOINT 10
-#endif
-// ... and the rank an index falls back to when too many of its rows fail rank SK_TC_JOINT (api.cu, tc_wide_joint)
-#ifndef SK_TC_JOINT_WIDE
-#define SK_TC_JOINT_WIDE 12
-#endif
-// hit path of a chunk: 0 = every lane runs the predicated parking code of all four octets, 1 = a
-// vote per octet first (octets nobody hits are skipped), 2 = a vote per pair of octets
-#ifndef SK_TC_OCTVOTE
-#define SK_TC_OCTVOTE 1
-#endif
-// jobs between two resolutions of the pending queues (0 = 8 with queues of four octets, 2 with queues of two)
-#ifndef SK_TC_DRAIN_EVERY
-#define SK_TC_DRAIN_EVERY 0
-#endif
+constexpr int TC_JOINT = 10;
+// ... and the rank an index falls back to when too many of its rows fail rank TC_JOINT (api.cu, tc_wide_joint)
+constexpr int TC_JOINT_WIDE = 12;
 
 // ---- per-thread selection state (thread <-> (query, stream) = column `col` of every array) ----
 //   candidates  buf_s / buf_i [CAP][LD]: unsorted (score, index) entries; the count lives in
@@ -242,22 +229,14 @@ __device__ __forceinline__ void tc_chunk(const uint32_t (&r)[32], int idb, uint3
     } else {
         if (!__any_sync(SK_FULL, hit)) return;   // vote straight into a predicate
     }
-#if SK_TC_OCTVOTE == 1
     // which octets hold a hit somewhere in the warp (votes against the threshold on entry: it only
     // falls inside, so a vote can only be a false alarm); octets without one are skipped, branch uniform
     unsigned ov[4];
 #pragma unroll
     for (int o = 0; o < 4; ++o) ov[o] = __ballot_sync(SK_FULL, g[o] < thr);
-#elif SK_TC_OCTVOTE == 2
-    unsigned ov[4];
-    ov[0] = ov[1] = __ballot_sync(SK_FULL, fminf(g[0], g[1]) < thr);
-    ov[2] = ov[3] = __ballot_sync(SK_FULL, fminf(g[2], g[3]) < thr);
-#endif
 #pragma unroll
     for (int o = 0; o < 4; ++o) {
-#if SK_TC_OCTVOTE
         if (ov[o] == 0u) continue;
-#endif
         const bool p = g[o] < thr;
         const bool room = pqo < PQ_END;
         SK_CHECK(pqo < PQ_END + ES);
@@ -549,7 +528,7 @@ search_tc_kernel(const __half *__restrict__ qimg, const __half *__restrict__ rim
             // every job when each warp takes it whenever its own queues fill up (measured: 32.5 ->
             // 30.1 ms per 4M rows).  A lane whose queue fills up inside a period drops octets, which
             // only lowers its threshold.
-            constexpr int DRAIN_EVERY = SK_TC_DRAIN_EVERY > 0 ? SK_TC_DRAIN_EVERY : 8;
+            constexpr int DRAIN_EVERY = 8;   // jobs between two scheduled resolutions (a power of two)
             // The schedule is global (job number modulo the period).  On top of it a warp whose queues
             // were (nearly) full at its last resolution comes back after one or two jobs: early in the
             // pass and on small reference sets the thresholds are loose and a full period would overflow
@@ -686,7 +665,7 @@ static cudaError_t launch_tc(const __half *qimg, const __half *rimg, int kc_tot,
                              const float *init_thr, const int *n_rows_dev, cudaStream_t st) {
     // rank of the joint threshold: the certificate's margin grows with the contraction depth
     // (eps * (|q|^2 + max|r|^2)), so deep spaces keep the streams' own KC-th best (rank 2 KC = off)
-    constexpr int JLO = NS == 2 ? SK_TC_JOINT : 1, JMID = NS == 2 ? SK_TC_JOINT_WIDE : 1, JHI = NS == 2 ? 2 * KC : 1;
+    constexpr int JLO = NS == 2 ? TC_JOINT : 1, JMID = NS == 2 ? TC_JOINT_WIDE : 1, JHI = NS == 2 ? 2 * KC : 1;
     const bool deep = kc_tot > 6;   // more than 48 FP16 elements, i.e. d' > 45 (search_tc_smem_bytes knows the same rule)
 #define SK_TC_GO(CAPE_, J_, DBG_)                                                                                  \
     return launch_tc_dbg<KC, MT, NS, CAP, CAPE_, J_, DBG_>(qimg, rimg, kc_tot, n_rtiles, nstage, seed_stride, n_q, \

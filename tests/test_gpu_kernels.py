@@ -919,10 +919,11 @@ def test_tensor_engine_certifies_nearly_every_row_and_stays_selected(k, n_ref):
 
 @pytest.mark.parametrize(("k", "n_ref", "exclude_self"), [(5, 30_000, False), (7, 30_000, False), (12, 30_000, False),
                                                            (6, 8_000, True)])
-def test_tensor_second_pass_equals_fp32_stage_and_takes_most_of_its_rows(k, n_ref, exclude_self):
+def test_tensor_second_pass_equals_exact_engine_and_takes_most_of_its_rows(k, n_ref, exclude_self):
     """Stage 1b of the cascade (the tensor engine once more over its uncertified rows, each from the
     threshold the first pass proved sufficient) must change nothing but who certifies a row: results
-    are bit-equal with and without it, and it leaves the FP32 engine fewer rows than the first pass did."""
+    are bit-equal with the exhaustive float64 engine's, and it leaves the FP32 engine fewer rows than
+    the first pass did."""
     from sknnr_b200._engine import KNNIndex
 
     rng = np.random.default_rng(31)
@@ -931,27 +932,22 @@ def test_tensor_second_pass_equals_fp32_stage_and_takes_most_of_its_rows(k, n_re
     Q = None if exclude_self else rng.standard_normal((150_000, 32))
     ix = KNNIndex(R, None, None, None, y)
     kw = dict(exclude_self=True) if exclude_self else dict(transformed=True)
-    try:
-        L.set_option("tc_retry", 0)
-        d0, i0, p0 = ix.query(Q, k, weights="distance", with_pred=True, **kw)
-        c0 = ix.cascade_counts()
-        L.set_option("tc_retry", 1)
-        d1, i1, p1 = ix.query(Q, k, weights="distance", with_pred=True, **kw)
-        c1 = ix.cascade_counts()
-    finally:
-        L.set_option("tc_retry", 1)
+    d1, i1, p1 = ix.query(Q, k, weights="distance", with_pred=True, **kw)
+    c1 = ix.cascade_counts()
     assert ix.stats()["engine"] == L.ENGINE_TENSOR
+    L.set_option("engine", L.ENGINE_EXACT)
+    try:
+        d0, i0, p0 = ix.query(Q, k, weights="distance", with_pred=True, **kw)
+        assert ix.stats()["engine"] == L.ENGINE_EXACT
+    finally:
+        L.set_option("engine", L.ENGINE_AUTO)
     assert np.array_equal(i0, i1) and np.array_equal(d0, d1) and np.array_equal(p0, p1)
-    # (without a second pass behind it the first pass sets its joint threshold at rank 12 instead of
-    # 10, so the two calls' first-pass counts are not comparable; what reaches the FP32 engine is)
-    assert c0["after_tensor"] == c0["to_fp32"], (c0, c1)
     assert c1["to_fp32"] <= c1["after_tensor"]
-    assert c1["to_fp32"] <= c0["to_fp32"], (c0, c1)
     if k + int(exclude_self) > 7:
         # one stream of 16 in the first pass already: a second pass would meet the same list, so there is none
-        assert c1["to_fp32"] == c1["after_tensor"], (c0, c1)
+        assert c1["to_fp32"] == c1["after_tensor"], c1
     elif c1["after_tensor"] >= 50:
-        assert c1["to_fp32"] < 0.2 * c1["after_tensor"], (c0, c1)
+        assert c1["to_fp32"] < 0.2 * c1["after_tensor"], c1
 
 
 def test_joint_threshold_rank_adapts_to_crowded_neighbourhoods():
@@ -975,12 +971,11 @@ def test_joint_threshold_rank_adapts_to_crowded_neighbourhoods():
 
 
 @pytest.mark.parametrize("pinned", [True, False])
-def test_host_pipeline_equals_one_stream_per_chunk(pinned):
+def test_host_call_many_chunks_equal_one_chunk(pinned):
     """Host-buffer calls run as a three-stage pipeline (in-order H2D stream, compute stream, D2H
     stream; csrc/api.cu).  Many ramped chunks, more chunks than slots, a ragged last chunk, tensor
-    and FP32 engines, a NaN row under the device-side finite check: all bit-equal with the layout
-    that gives every chunk a stream of its own, and a second call on the same index reuses the
-    slots cleanly."""
+    and FP32 engines, a NaN row under the device-side finite check: all bit-equal with the same query
+    made as a single chunk, and a second call on the same index reuses the slots cleanly."""
     from sknnr_b200._engine import KNNIndex, pinned_empty
 
     rng = np.random.default_rng(77)
@@ -994,30 +989,30 @@ def test_host_pipeline_equals_one_stream_per_chunk(pinned):
             Xp[:] = X
             X = Xp
         ix = KNNIndex(R, None, None, None, y)
+
+        def run():
+            out = None
+            if pinned:
+                out = (pinned_empty((n_q, 6)), pinned_empty((n_q, 6), np.int64), pinned_empty((n_q, 3)))
+            got = ix.query(X, 6, transformed=True, weights="distance", with_pred=True, out=out)
+            return [np.array(g) for g in got]
+
+        one = run()                                  # default chunk_rows / stage_rows: a single chunk
         L.set_option("chunk_rows", 4096)
         L.set_option("stage_rows", 2048)
         try:
-            res = {}
-            for mode in (0, 1, 1):
-                L.set_option("host_pipeline", mode)
-                out = None
-                if pinned:
-                    out = (pinned_empty((n_q, 6)), pinned_empty((n_q, 6), np.int64), pinned_empty((n_q, 3)))
-                got = ix.query(X, 6, transformed=True, weights="distance", with_pred=True, out=out)
-                if mode in res:
-                    for a, b in zip(res[mode], got):
-                        assert np.array_equal(a, b)
-                res[mode] = [np.array(g) for g in got]
-            for a, b in zip(res[0], res[1]):
+            many = run()
+            for a, b in zip(one, many):
+                assert np.array_equal(a, b)
+            for a, b in zip(many, run()):
                 assert np.array_equal(a, b)
             Xb = np.array(X)
             Xb[n_q - 3, 1] = np.nan
             with pytest.raises(L.NonFiniteInput):
                 ix.query(Xb, 6, transformed=True, check_finite=True)
             again = ix.query(X, 6, transformed=True, weights="distance", with_pred=True)
-            for a, b in zip(res[1], again):
+            for a, b in zip(many, again):
                 assert np.array_equal(a, b)
         finally:
-            L.set_option("host_pipeline", 1)
             L.set_option("chunk_rows", 1 << 20)
             L.set_option("stage_rows", 1 << 19)

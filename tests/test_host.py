@@ -245,3 +245,23 @@ def test_host_chunk_schedule_ramps_and_covers_every_row():
     assert L.host_chunk_plan(10_000_000, 1 << 20) == [262144, 524288] + [1 << 20] * 8 + [562816, 262144]
     with pytest.raises(ValueError):
         L.host_chunk_plan(-1, 1 << 20)
+
+
+def test_set_option_accepts_the_kept_names_and_rejects_the_retired_ones():
+    """The options that only chose between a measured winner and a measured loser are gone from
+    sknnr_set_option: their names are unknown options now.  The kept ones still take a value."""
+    from sknnr_b200 import _lib as L
+
+    for name in ("host_pipeline", "tail_priority", "tc_retry", "tail_spread", "host_nt", "simt_min_rows",
+                 "host_threads"):
+        with pytest.raises(ValueError, match="unknown option"):
+            L.set_option(name, 1)
+    # (a value other than the default, then the default again)
+    kept = {"engine": (3, 0), "chunk_rows": (4096, 1 << 20), "timing": (1, 0), "kc": (8, 16), "tc_streams": (1, 0),
+            "tc_seed_stride": (2, 4), "tc_debug": (1, 0), "host_slots": (2, 8), "stage_rows": (2048, 1 << 19)}
+    try:
+        for name, (value, _) in kept.items():
+            L.set_option(name, value)
+    finally:
+        for name, (_, default) in kept.items():
+            L.set_option(name, default)
