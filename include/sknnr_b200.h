@@ -68,6 +68,11 @@ extern "C" {
 #define SKNNR_ENGINE_TENSOR 2   /* tcgen05 TF32 filter kernel                              */
 #define SKNNR_ENGINE_EXACT 3    /* FP64 exhaustive kernel (the certificate's fallback)     */
 
+/* distance of a float index (sknnr_index_create_metric) */
+#define SKNNR_METRIC_EUCLIDEAN 0   /* sqrt(sum (x_j - y_j)^2)                                    */
+#define SKNNR_METRIC_MANHATTAN 1   /* sum |x_j - y_j|, summed left to right in float64           */
+#define SKNNR_METRIC_CHEBYSHEV 2   /* max |x_j - y_j|                                            */
+
 typedef struct sknnr_index sknnr_index;           /* Euclidean-space estimators */
 typedef struct sknnr_hamming_index sknnr_hamming_index; /* RFNN node-ID estimators    */
 typedef struct sknnr_forest sknnr_forest;               /* fitted forests of an RFNodeTransformer */
@@ -112,7 +117,7 @@ int sknnr_set_option(const char *name, int64_t value);
  * the last chunk's copy out overlap no kernel. */
 int sknnr_host_chunk_plan(int64_t n_q, int64_t chunk_rows, int64_t *rows_out, int32_t cap, int32_t *n_chunks);
 
-/* ---- Euclidean-space index: Raw / Euclidean / Mahalanobis / MSN / GNN ------------------
+/* ---- Float index: Raw / Euclidean / Mahalanobis / MSN / GNN -----------------------------
  * Fitted state of one estimator.  The four float transformers are one affine map
  *     Z = ((X - center) / scale) @ proj
  * (StandardScalerWithDOF: $SP/sklearn/preprocessing/_data.py:1131-1134 with scale_ from
@@ -130,6 +135,20 @@ int sknnr_index_create(const double *fit_z, int64_t n_ref, int32_t d_out,
                        const double *center, const double *scale, const double *proj,
                        int32_t d_in, const double *y, int32_t n_out, int32_t device,
                        sknnr_index **out);
+/* The same for a search with another distance in the estimator's space (sknnr_index_create is the
+ * SKNNR_METRIC_EUCLIDEAN case).  SKNNR_METRIC_MANHATTAN / _CHEBYSHEV are scikit-learn's
+ * ManhattanDistance64 / ChebyshevDistance64 ($SP/sklearn/metrics/_dist_metrics.pyx.tp), which
+ * KNeighborsRegressor uses for metric="manhattan" / "cityblock" / "l1" / minkowski p=1 and
+ * "chebyshev" / "infinity" / minkowski p=inf: the returned distances are bit-equal to its own (a
+ * sequential float64 sum, resp. maximum, of |x_j - y_j|; no square root).  Such an index searches
+ * with an FP32 filter kernel (SKNNR_ENGINE_SIMT; AUTO and TENSOR select it too) whose candidates a
+ * float64 kernel recomputes and certifies, and with the exhaustive float64 kernel for the rest; every
+ * query call, sknnr_transform and the raster front end take it as they take a Euclidean index.
+ * Another metric code: SKNNR_EINVAL.                                                         */
+int sknnr_index_create_metric(const double *fit_z, int64_t n_ref, int32_t d_out,
+                              const double *center, const double *scale, const double *proj,
+                              int32_t d_in, const double *y, int32_t n_out, int32_t metric,
+                              int32_t device, sknnr_index **out);
 int sknnr_index_destroy(sknnr_index *index);
 
 /* kneighbors (+ optional predict) for n_q query rows.  Replaces S2+S1(+S3) in one call.

@@ -80,8 +80,9 @@ class RawKNNRegressor(DFIndexCrosswalkMixin, IndependentPredictorMixin, KNeighbo
     """``KNeighborsRegressor`` with independent prediction / score, dataframe-index crosswalk
     and deterministic neighbour ordering (mirrors ref:src/sknnr/_base.py:43-182), searching on
     the B200.  Supported searches: brute Euclidean (``metric='minkowski', p=2`` or
-    ``'euclidean'``) and weighted Hamming (``metric='hamming'``); ``algorithm`` is accepted for
-    signature compatibility and the search is always exhaustive.
+    ``'euclidean'``), Manhattan (``p=1``, ``'manhattan'``, ``'cityblock'``, ``'l1'``), Chebyshev
+    (``p=np.inf``, ``'chebyshev'``, ``'infinity'``) and weighted Hamming (``metric='hamming'``);
+    ``algorithm`` is accepted for signature compatibility and the search is always exhaustive.
     """
 
     DISTANCE_PRECISION_DECIMALS = 10
@@ -96,15 +97,21 @@ class RawKNNRegressor(DFIndexCrosswalkMixin, IndependentPredictorMixin, KNeighbo
         state.pop("_device_index", None)
         return state
 
+    # effective_metric_ -> search: scikit-learn maps minkowski p=1 / p=inf without weights to
+    # "manhattan" / "chebyshev", and its brute search runs the same distance for the aliases
+    _KINDS = {"euclidean": "euclidean", "manhattan": "manhattan", "cityblock": "manhattan",
+              "l1": "manhattan", "chebyshev": "chebyshev", "infinity": "chebyshev", "hamming": "hamming"}
+
     def _metric_kind(self) -> str:
         m = self.effective_metric_
-        if m == "euclidean":
-            return "euclidean"
-        if m == "hamming":
-            return "hamming"
-        raise NotImplementedError(
-            f"sknnr_b200 covers the brute Euclidean and Hamming searches; metric={self.metric!r} "
-            f"(effective {m!r}) has no CUDA path and there is no CPU fallback")
+        kind = self._KINDS.get(m) if isinstance(m, str) else None
+        if kind in ("manhattan", "chebyshev") and self.effective_metric_params_:
+            kind = None   # (a parametrised variant of the distance)
+        if kind is None:
+            raise NotImplementedError(
+                f"sknnr_b200 covers the brute Euclidean, Manhattan, Chebyshev and Hamming searches; "
+                f"metric={self.metric!r} (effective {m!r}) has no CUDA path and there is no CPU fallback")
+        return kind
 
     def _get_index(self):
         ix = self.__dict__.get("_device_index")
@@ -112,9 +119,10 @@ class RawKNNRegressor(DFIndexCrosswalkMixin, IndependentPredictorMixin, KNeighbo
             return ix
         y = self._y
         devices = devices_from_env()    # SKNNR_B200_DEVICES: the same fitted state on several GPUs
-        if self._metric_kind() == "euclidean":
+        kind = self._metric_kind()
+        if kind != "hamming":
             center, scale, proj = self.__dict__.get("_projection", (None, None, None))
-            make = lambda dev: KNNIndex(self._fit_X, center, scale, proj, y, device=dev)  # noqa: E731
+            make = lambda dev: KNNIndex(self._fit_X, center, scale, proj, y, device=dev, metric=kind)  # noqa: E731
             ix = MultiDeviceIndex(make, devices) if devices else make(None)
         else:
             ref_ids = np.asarray(self._fit_X)

@@ -1,7 +1,7 @@
 """Device-resident fitted state: thin Python owners of the C-ABI index handles.
 
-``KNNIndex`` serves the Euclidean-space estimators (Raw / Euclidean / Mahalanobis / MSN /
-GNN), ``HammingIndex`` serves RFNN.  Handles are caches: they are rebuilt from the NumPy
+``KNNIndex`` serves the float estimators (Raw / Euclidean / Mahalanobis / MSN / GNN) with a
+Euclidean, Manhattan or Chebyshev search, ``HammingIndex`` serves RFNN.  Handles are caches: they are rebuilt from the NumPy
 fitted attributes on demand and never pickled.
 """
 
@@ -212,11 +212,12 @@ def _raster_call(index, fn, handles, n_bands, bands, k, *, nodata=None, determin
 
 
 class KNNIndex(_IndexBase):
-    """Fitted state of one Euclidean-space estimator on the device.
+    """Fitted state of one float estimator on the device.
 
     ``fit_z``: transformed reference plots (``regressor_._fit_X``); ``center/scale/proj``:
     the affine projection ``Z = ((X - center) / scale) @ proj`` (any may be None);
-    ``y``: targets (``regressor_._y``).
+    ``y``: targets (``regressor_._y``); ``metric``: ``"euclidean"``, ``"manhattan"`` or
+    ``"chebyshev"``, the distance searched in the projected space.
     """
 
     _destroy = "sknnr_index_destroy"
@@ -229,8 +230,11 @@ class KNNIndex(_IndexBase):
         L.check(self._lib.sknnr_index_cascade_counts(self._h, out))
         return {"after_tensor": out[0], "to_fp32": out[1], "to_exact": out[2]}
 
-    def __init__(self, fit_z, center=None, scale=None, proj=None, y=None, device=None):
+    def __init__(self, fit_z, center=None, scale=None, proj=None, y=None, device=None, metric="euclidean"):
         super().__init__()
+        if metric not in L.METRICS:
+            raise ValueError(f"metric must be one of {sorted(L.METRICS)}, got {metric!r}")
+        self.metric = metric
         fit_z = _f64(fit_z)
         if fit_z.ndim != 2:
             raise ValueError("fit_z must be 2-D")
@@ -248,9 +252,9 @@ class KNNIndex(_IndexBase):
             self.d_in = self.d_out
         self.n_out = 0 if y is None else y.shape[1]
         self.device = default_device() if device is None else int(device)
-        L.check(self._lib.sknnr_index_create(
+        L.check(self._lib.sknnr_index_create_metric(
             _ptr(fit_z), self.n_ref, self.d_out, _ptr(center), _ptr(scale), _ptr(proj),
-            self.d_in, _ptr(y), self.n_out, self.device, C.byref(self._h)))
+            self.d_in, _ptr(y), self.n_out, L.METRICS[metric], self.device, C.byref(self._h)))
 
     # -- host-buffer query (the drop-in call) ------------------------------------------
     def query(self, X, k, *, exclude_self=False, deterministic=True, decimals=10,

@@ -18,6 +18,7 @@ F64, F32 = 0, 1
 EXCLUDE_SELF, DETERMINISTIC, TRANSFORMED, DEVICE_PTRS, CHECK_FINITE = 1, 2, 4, 8, 16
 W_NONE, W_UNIFORM, W_DISTANCE = 0, 1, 2
 ENGINE_AUTO, ENGINE_SIMT, ENGINE_TENSOR, ENGINE_EXACT = 0, 1, 2, 3
+METRICS = {"euclidean": 0, "manhattan": 1, "chebyshev": 2}   # SKNNR_METRIC_*
 MAX_CODE = 31743
 
 EXPORTS = [
@@ -30,6 +31,7 @@ EXPORTS = [
     "sknnr_forest_apply", "sknnr_hamming_kneighbors_forest", "sknnr_raster_kneighbors",
     "sknnr_hamming_raster_kneighbors_forest", "sknnr_device_alloc", "sknnr_device_free",
     "sknnr_ipc_export", "sknnr_ipc_open", "sknnr_ipc_close", "sknnr_device_copy", "sknnr_host_chunk_plan",
+    "sknnr_index_create_metric",
 ]
 
 
@@ -74,6 +76,7 @@ def load() -> C.CDLL:
     lib.sknnr_device_count.argtypes = [C.POINTER(C.c_int)]
     lib.sknnr_set_option.argtypes = [C.c_char_p, i64]
     lib.sknnr_index_create.argtypes = [vp, i64, i32, vp, vp, vp, i32, vp, i32, i32, C.POINTER(vp)]
+    lib.sknnr_index_create_metric.argtypes = [vp, i64, i32, vp, vp, vp, i32, vp, i32, i32, i32, C.POINTER(vp)]
     lib.sknnr_index_destroy.argtypes = [vp]
     lib.sknnr_kneighbors.argtypes = [vp, vp, i32, i64, i64, i64, i32, u32, i32, vp, vp, i32, vp, vp]
     lib.sknnr_transform.argtypes = [vp, vp, i32, i64, i64, vp]

@@ -575,9 +575,11 @@ struct sknnr_index : IndexBase {
     int d_in = 0, d_out = 0, dpad = 0;
     double *d_ref64 = nullptr, *d_center = nullptr, *d_scale = nullptr, *d_proj = nullptr,
            *d_mu = nullptr;
+    int metric = SKNNR_METRIC_EUCLIDEAN;
     float *d_rimg = nullptr;
     int n_rtiles = 0;
-    double r2max = 0.0;
+    double r2max = 0.0;            // max_j |ref_j - mu|^2; Manhattan / Chebyshev: max_j |ref_j - mu| in that norm
+    bool simt_ok = true;           // the FP32 image can serve as a filter (Manhattan / Chebyshev: no plot overflows it)
     __half *d_rimg_tc = nullptr;   // tensor-core engine reference image (FP16)
     int n_rtiles_tc = 0, kc_tot = 0, tc_nstage = 0;
     double tc_sigma = 1.0;         // power-of-two scale of both tensor-engine images
@@ -729,11 +731,25 @@ int sknnr_device_copy(int32_t device, void *dst, const void *src, int64_t bytes,
 }
 
 // -----------------------------------------------------------------------------------------
+// |x - mu| (Manhattan, Chebyshev) below this bound for the query and every plot: no score of the FP32
+// filter (twice the distance, plus rounding) can overflow, so every reference outside a candidate list
+// has a finite score and a list that is not full holds every reference
+constexpr double kLpNormLimit = 0x1p124;
+
 int sknnr_index_create(const double *fit_z, int64_t n_ref, int32_t d_out, const double *center,
                        const double *scale, const double *proj, int32_t d_in, const double *y,
                        int32_t n_out, int32_t device, sknnr_index **out) {
+    return sknnr_index_create_metric(fit_z, n_ref, d_out, center, scale, proj, d_in, y, n_out,
+                                     SKNNR_METRIC_EUCLIDEAN, device, out);
+}
+
+int sknnr_index_create_metric(const double *fit_z, int64_t n_ref, int32_t d_out, const double *center,
+                              const double *scale, const double *proj, int32_t d_in, const double *y,
+                              int32_t n_out, int32_t metric, int32_t device, sknnr_index **out) {
     if (!fit_z || !out || n_ref < 1 || d_out < 1 || d_in < 1)
         return fail(SKNNR_EINVAL, "bad arguments to sknnr_index_create");
+    if (metric != SKNNR_METRIC_EUCLIDEAN && metric != SKNNR_METRIC_MANHATTAN && metric != SKNNR_METRIC_CHEBYSHEV)
+        return fail(SKNNR_EINVAL, "unknown metric");
     if (!proj && d_in != d_out) return fail(SKNNR_EINVAL, "d_in != d_out without a projector");
     if (n_ref >= (1LL << 31) - 64) return fail(SKNNR_EUNSUP, "n_ref too large");
     if (y == nullptr) n_out = 0;
@@ -744,6 +760,7 @@ int sknnr_index_create(const double *fit_z, int64_t n_ref, int32_t d_out, const 
         delete ix;
         return rc;
     }
+    ix->metric = metric;
     ix->d_in = d_in;
     ix->d_out = d_out;
     ix->dpad = round_up(d_out, 8);
@@ -756,7 +773,10 @@ int sknnr_index_create(const double *fit_z, int64_t n_ref, int32_t d_out, const 
         for (int k = 0; k < d_out; ++k) mu[k] += fit_z[j * d_out + k];
     for (int k = 0; k < d_out; ++k) mu[k] /= (double)n_ref;
 
-    // reference tile images [(dpad+1)][64] f32, last row = |r|^2 (+inf for padding plots)
+    // reference tile images [(dpad+1)][64] f32, last row = |r|^2 (+inf for padding plots).
+    // Manhattan / Chebyshev: -2 (r - mu), the query image's own transform, and a last row of 0 (+inf
+    // for padding plots) that starts the sum / maximum.
+    const bool lp = metric != SKNNR_METRIC_EUCLIDEAN;
     const size_t tile_floats = (size_t)(ix->dpad + 1) * RTILE;
     std::vector<float> rimg((size_t)ix->n_rtiles * tile_floats, 0.0f);
     double r2max = 0.0;
@@ -771,6 +791,11 @@ int sknnr_index_create(const double *fit_z, int64_t n_ref, int32_t d_out, const 
             double n32 = 0.0, n64 = 0.0;
             for (int k = 0; k < d_out; ++k) {
                 const double v = fit_z[j * d_out + k] - mu[k];
+                if (lp) {
+                    img[(size_t)k * RTILE + jj] = (float)(-2.0 * v);
+                    n64 = metric == SKNNR_METRIC_MANHATTAN ? n64 + std::fabs(v) : std::max(n64, std::fabs(v));
+                    continue;
+                }
                 const float f = (float)v;
                 img[(size_t)k * RTILE + jj] = f;
                 n32 += (double)f * (double)f;
@@ -781,6 +806,7 @@ int sknnr_index_create(const double *fit_z, int64_t n_ref, int32_t d_out, const 
         }
     }
     ix->r2max = r2max;
+    if (lp) ix->simt_ok = r2max < kLpNormLimit;   // (false for NaN as well)
 
     auto up = [&](double **dst, const double *src, size_t n) -> cudaError_t {
         cudaError_t e = cudaMalloc(dst, n * sizeof(double));
@@ -807,7 +833,7 @@ int sknnr_index_create(const double *fit_z, int64_t n_ref, int32_t d_out, const 
     ix->n_rtiles_tc = (int)((n_ref + TC_N - 1) / TC_N);
     ix->tc_nstage = search_tc_pick_config(ix->kc_tot);
     // (below a thousand plots a tile pass is a handful of jobs: the FP32 engine is the better filter)
-    ix->tensor_ok = ix->tc_nstage != 0 && std::isfinite(r2max) && n_ref >= 1024;
+    ix->tensor_ok = !lp && ix->tc_nstage != 0 && std::isfinite(r2max) && n_ref >= 1024;
     if (e == cudaSuccess && ix->tensor_ok) {
         int ex = 0;
         if (r2max > 0.0) {
@@ -903,7 +929,8 @@ static int run_chunk(sknnr_index *ix, Slot &s, const void *dX, int x_f32, int64_
 
     int kc = pick_kc(kk, 1);   // 0: k (+1) is beyond the filtered engines' candidate lists -> exhaustive kernel
     if (kc != 0 && g_opt.kc > kc) kc = (int)g_opt.kc;
-    const bool simt_ok = kc != 0 && search_simt_pick_stages(ix->dpad, kc) != 0;
+    const bool lp = ix->metric != SKNNR_METRIC_EUCLIDEAN;   // Manhattan / Chebyshev: SIMT -> refine_lp -> exact
+    const bool simt_ok = kc != 0 && search_simt_pick_stages(ix->dpad, kc) != 0 && ix->simt_ok;
     const int ns_layout = g_opt.tc_streams == 1 ? 1 : (kk <= 7 ? 2 : 1);
     ix->ns_in_use = ns_layout;
     const bool tensor_ok = ix->tensor_ok && !ix->tensor_demoted[ns_layout] && kc != 0 && kc <= 16 && simt_ok;
@@ -946,7 +973,7 @@ static int run_chunk(sknnr_index *ix, Slot &s, const void *dX, int x_f32, int64_
     }
 
     ExactArgs ea{};
-    ea.metric = 0;
+    ea.metric = ix->metric == SKNNR_METRIC_MANHATTAN ? 2 : ix->metric == SKNNR_METRIC_CHEBYSHEV ? 3 : 0;
     ea.z64 = s.z64.p;
     ea.ref64 = ix->d_ref64;
     ea.d = ix->d_out;
@@ -1074,7 +1101,7 @@ static int run_chunk(sknnr_index *ix, Slot &s, const void *dX, int x_f32, int64_
     constexpr int kSimtMinRows = 256;
     const int bypass = stage2_count ? kSimtMinRows : 0;
     CK(launch_search_simt(s.qimg.p, ix->d_rimg, ix->dpad, ix->n_rtiles, rows, kc, s.cand_idx.p,
-                          s.cand_thr.p, stage2_count, ix->spread_tail ? ix->n_sm : 0, bypass, st));
+                          s.cand_thr.p, stage2_count, ix->spread_tail ? ix->n_sm : 0, bypass, st, ix->metric));
     if (g_opt.timing && !use_tc) CK(s.mark(st));
     FinishParams fp2 = fp;
     fp2.row_map = stage2_list;
@@ -1091,7 +1118,21 @@ static int run_chunk(sknnr_index *ix, Slot &s, const void *dX, int x_f32, int64_
     ra.bypass_rows = bypass;
     ra.n_rows_dev = stage2_count;
     ra.row_map = fp2.row_map;
-    CK(launch_refine(ra, fp2, st));
+    if (lp) {
+        // |score / 2 - distance| <= eps * (|q - mu| + max_j |r_j - mu|) in the metric's norm (DESIGN.md §2,
+        // "Manhattan and Chebyshev"): FP32 rounding of both images and of their difference, plus, for L1, dpad
+        // sequential FP32 additions; the 1 % covers the float64 terms (centring, the norms, the distances)
+        ra.eps_s = (ix->metric == SKNNR_METRIC_MANHATTAN ? ix->dpad + 2.0 : 2.0) * std::ldexp(1.0, -24) * 1.01;
+        ra.thr_scale = 0.5;
+        ra.qn_limit = kLpNormLimit;
+        // (+ 2^-120: the absolute error of image elements in FP32's subnormal range, at most 2^-150 each,
+        // which the relative bound does not cover)
+        ra.r2max = ix->r2max + 0x1p-120;
+        CK(launch_refine_lp(ra, ix->metric, fp2, st));
+        ix->n_simt_rows += rows;   // (the FP32 stage is the first one: every row of the chunk)
+    } else {
+        CK(launch_refine(ra, fp2, st));
+    }
     ix->stats.kernel_launches += 2;
 
     // stage 3: exhaustive float64 search of whatever is still uncertified (exact ties etc.)

@@ -29,11 +29,16 @@ cudaError_t launch_gather_rows(const double *z64, int d, const int *list, const 
                                long long max_rows, double *z64c, cudaStream_t st);
 
 // ---- search_simt.cu --------------------------------------------------------------------
+// distance of a float index (the values of SKNNR_METRIC_*)
+constexpr int METRIC_L2 = 0;     // Euclidean
+constexpr int METRIC_L1 = 1;     // Manhattan
+constexpr int METRIC_LINF = 2;   // Chebyshev
 size_t search_simt_smem_bytes(int dpad, int kc, int nstage);
 int search_simt_pick_stages(int dpad, int kc);
 cudaError_t launch_search_simt(const float *qimg, const float *rimg, int dpad, int n_rtiles,
                                long long n_q, int kc, int *cand_idx, float *cand_thr,
-                               const int *n_rows_dev, int spread_ctas, int bypass_rows, cudaStream_t st);
+                               const int *n_rows_dev, int spread_ctas, int bypass_rows, cudaStream_t st,
+                               int metric);
 // n_rows_dev != null: compacted launch, the row count is read on the device; spread_ctas > 0 then
 // deals the rows out over up to that many CTAs in units of one warp (0: one CTA per 384 rows); a compacted
 // launch with fewer than bypass_rows rows does nothing (refine then hands the rows on, RefineArgs.bypass_rows)
@@ -82,11 +87,16 @@ struct RefineArgs {
                             // goes to fb_list unexamined
 };
 cudaError_t launch_refine(const RefineArgs &a, const FinishParams &fp, cudaStream_t st);
+// The same stage for METRIC_L1 / METRIC_LINF: every candidate's float64 distance is recomputed in
+// scikit-learn's order (sequential sum / max of |z_k - r_k|), so the distances are bit-equal to its
+// own.  r2max holds max_j |ref_j - mu| in the metric's norm, qn_limit bounds |q - mu| the same way,
+// thr_scale = 0.5 (the images hold -2 (x - mu)); compacted launches are not supported.
+cudaError_t launch_refine_lp(const RefineArgs &a, int metric, const FinishParams &fp, cudaStream_t st);
 
 // Exhaustive float64 search for the rows in list[0..*count) (or all rows when list==null):
 // one CTA per row, all references, exact (distance, index) top-k, then finish_query.
 struct ExactArgs {
-    int metric;             // 0 = Euclidean (z64/ref64), 1 = weighted Hamming (codes + w)
+    int metric;             // 0 = Euclidean (z64/ref64), 1 = weighted Hamming (codes + w), 2 = Manhattan, 3 = Chebyshev
     const double *z64;
     const double *ref64;
     int d;

@@ -5,6 +5,7 @@
 //                    "certificate"), and finishes the row (self exclusion, sknnr's
 //                    deterministic ordering, outputs, weighted average); refine2_kernel is the
 //                    same for lists of <= 16 candidates with two queries per warp;
+//   refine_lp_kernel - the same for Manhattan / Chebyshev indexes, one lane per candidate;
 //   exact_kernel   - exhaustive float64 search for the rows whose certificate failed (and the
 //                    engine for shapes the fast kernels do not cover / unequal Hamming weights);
 //   weighted_average_kernel - seam S3 with caller-supplied weights.
@@ -301,12 +302,100 @@ cudaError_t launch_refine(const RefineArgs &a, const FinishParams &fp, cudaStrea
 }
 
 // ---------------------------------------------------------------------------------------
+// Manhattan / Chebyshev: scikit-learn's ManhattanDistance64 / ChebyshevDistance64
+// ($SP/sklearn/metrics/_dist_metrics.pyx.tp: d += fabs(x1[j] - x2[j]), resp. d = fmax(d, ...), j
+// ascending, and the identity as rdist_to_dist), written with explicit roundings so that neither the
+// order nor a contraction is the compiler's choice: the distances are bit-equal to the reference's.
+template <int M>
+__device__ __forceinline__ double dist_lp(const double *__restrict__ zq, const double *__restrict__ r, int d) {
+    double acc = 0.0;
+    for (int j = 0; j < d; ++j) {
+        const double t = fabs(__dsub_rn(zq[j], __ldg(r + j)));
+        acc = M == METRIC_L1 ? __dadd_rn(acc, t) : fmax(acc, t);
+    }
+    return acc;
+}
+
+// |q - mu| in the metric's norm, by the whole warp (lanes stride the features)
+template <int M>
+__device__ __forceinline__ double norm_lp_warp(const double *__restrict__ zq, const double *__restrict__ mu, int d,
+                                               int lane) {
+    double n = 0.0;
+    for (int k = lane; k < d; k += 32) {
+        const double t = fabs(zq[k] - mu[k]);
+        n = M == METRIC_L1 ? n + t : fmax(n, t);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const double other = __shfl_xor_sync(SK_FULL, n, o);
+        n = M == METRIC_L1 ? n + other : fmax(n, other);
+    }
+    return n;
+}
+
+// One warp per query, one lane per candidate (kc <= 32): lane l recomputes candidate l's distance in
+// scikit-learn's order, the warp sorts by (distance, index) and certifies the row when
+//     kth < thr * thr_scale - eps_s * (|q - mu| + max_j |r_j - mu|)      (DESIGN.md §2, "Manhattan and Chebyshev")
+// strictly, so that an exact tie with a reference outside the list goes to the exhaustive kernel.
+// Every score is finite while |q - mu| < qn_limit (and the index's plots are below the same limit):
+// thr = +inf then means that the list holds every reference.  A NaN norm never certifies.
+template <int M, int SORT>
+__global__ void __launch_bounds__(REFINE_WARPS * 32)
+refine_lp_kernel(RefineArgs a, FinishParams fp) {
+    const int warp = __shfl_sync(SK_FULL, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
+    const long long q = (long long)blockIdx.x * REFINE_WARPS + warp;
+    if (q >= a.n_q) return;
+    const double *zq = a.z64 + q * a.d;
+    const int c = lane < a.kc ? a.cand_idx[q * a.kc + lane] : -1;
+    SK_CHECK(c >= -1 && c < a.n_ref);
+    int id = 0x7fffffff;
+    double dist = SK_INF_D;
+    if (c >= 0 && c < a.n_ref) {
+        id = c;
+        dist = dist_lp<M>(zq, a.ref64 + (long long)c * a.d, a.d);
+    }
+    const double qn = norm_lp_warp<M>(zq, a.mu, a.d, lane);
+    warp_sort_pairs<double, SORT>(dist, id, lane);
+
+    const int kk = fp.k + (fp.exclude_self ? 1 : 0);
+    const double kth = __shfl_sync(SK_FULL, dist, kk - 1);
+    const float thr = a.cand_thr[q];
+    const bool ok = qn < a.qn_limit &&
+                    (thr == SK_INF_F || kth < (double)thr * a.thr_scale - a.eps_s * (qn + a.r2max));
+    if (!ok) {
+        if (lane == 0) a.fb_list[atomicAdd(a.fb_count, 1)] = (int)q;
+        return;
+    }
+    finish_query(fp, q, dist, id, lane);
+}
+
+cudaError_t launch_refine_lp(const RefineArgs &a, int metric, const FinishParams &fp, cudaStream_t st) {
+    if (a.n_q <= 0) return cudaSuccess;
+    if (a.kc > 32 || a.n_rows_dev || a.fb_thr || a.n_thr != 1) return cudaErrorInvalidValue;
+    const long long grid = (a.n_q + REFINE_WARPS - 1) / REFINE_WARPS;
+    // (lists of <= 16 sit in lanes 0..15: the sort network of 16 lanes suffices)
+    if (metric == METRIC_L1 && a.kc <= 16)
+        refine_lp_kernel<METRIC_L1, 16><<<(unsigned)grid, REFINE_WARPS * 32, 0, st>>>(a, fp);
+    else if (metric == METRIC_L1)
+        refine_lp_kernel<METRIC_L1, 32><<<(unsigned)grid, REFINE_WARPS * 32, 0, st>>>(a, fp);
+    else if (metric == METRIC_LINF && a.kc <= 16)
+        refine_lp_kernel<METRIC_LINF, 16><<<(unsigned)grid, REFINE_WARPS * 32, 0, st>>>(a, fp);
+    else if (metric == METRIC_LINF)
+        refine_lp_kernel<METRIC_LINF, 32><<<(unsigned)grid, REFINE_WARPS * 32, 0, st>>>(a, fp);
+    else
+        return cudaErrorInvalidValue;
+    return cudaGetLastError();
+}
+
+// ---------------------------------------------------------------------------------------
 constexpr int EXACT_THREADS = 256;
 
 __device__ __forceinline__ double exact_pair(const ExactArgs &a, long long q, int j) {
-    if (a.metric == 0) {
+    if (a.metric != 1) {
         const double *zq = a.z64 + q * a.d;
         const double *r = a.ref64 + (long long)j * a.d;
+        if (a.metric == 2) return dist_lp<METRIC_L1>(zq, r, a.d);
+        if (a.metric == 3) return dist_lp<METRIC_LINF>(zq, r, a.d);
         return dist2_serial(zq, r, a.d);
     }
     // weighted Hamming: left-to-right float64 sum of w_t over mismatching trees / sum(w)

@@ -29,7 +29,10 @@
 
 namespace sk {
 
-template <int KC>
+// M = METRIC_L2: Euclidean scores as above.  M = METRIC_L1 / METRIC_LINF (Manhattan / Chebyshev): both
+// images hold -2 (x - mu), the bias row holds 0 (+inf for padding plots), and a score is the FP32
+// sum (max) of |q_k - r_k| over the features, twice the approximate L1 (L-inf) distance.
+template <int KC, int M>
 __global__ void __launch_bounds__(SEARCH_THREADS, 1)
 search_simt_kernel(const float *__restrict__ qimg, const float *__restrict__ rimg, int dpad,
                    int n_rtiles, int nstage, long long n_q, int *__restrict__ cand_idx,
@@ -142,24 +145,56 @@ search_simt_kernel(const float *__restrict__ qimg, const float *__restrict__ rim
                 acc[i][3] = make_float2(n1.z, n1.w);
             }
         }
-        for (int k0 = 0; k0 < dpad; k0 += 8) {
+        if constexpr (M == METRIC_L2) {
+            for (int k0 = 0; k0 < dpad; k0 += 8) {
 #pragma unroll
-            for (int kk = 0; kk < 8; ++kk) {
-                const int k = k0 + kk;
-                const float4 qa = *reinterpret_cast<const float4 *>(qp + k * QTILE);
-                const float4 qb = *reinterpret_cast<const float4 *>(qp + k * QTILE + 16);
-                const float4 ra = *reinterpret_cast<const float4 *>(rp + k * RTILE);
-                const float4 rb = *reinterpret_cast<const float4 *>(rp + k * RTILE + 32);
-                const float2 r0 = make_float2(ra.x, ra.y), r1 = make_float2(ra.z, ra.w);
-                const float2 r2 = make_float2(rb.x, rb.y), r3 = make_float2(rb.z, rb.w);
-                const float qv[8] = {qa.x, qa.y, qa.z, qa.w, qb.x, qb.y, qb.z, qb.w};
+                for (int kk = 0; kk < 8; ++kk) {
+                    const int k = k0 + kk;
+                    const float4 qa = *reinterpret_cast<const float4 *>(qp + k * QTILE);
+                    const float4 qb = *reinterpret_cast<const float4 *>(qp + k * QTILE + 16);
+                    const float4 ra = *reinterpret_cast<const float4 *>(rp + k * RTILE);
+                    const float4 rb = *reinterpret_cast<const float4 *>(rp + k * RTILE + 32);
+                    const float2 r0 = make_float2(ra.x, ra.y), r1 = make_float2(ra.z, ra.w);
+                    const float2 r2 = make_float2(rb.x, rb.y), r3 = make_float2(rb.z, rb.w);
+                    const float qv[8] = {qa.x, qa.y, qa.z, qa.w, qb.x, qb.y, qb.z, qb.w};
 #pragma unroll
-                for (int i = 0; i < 8; ++i) {
-                    const float2 qd = make_float2(qv[i], qv[i]);
-                    acc[i][0] = __ffma2_rn(qd, r0, acc[i][0]);
-                    acc[i][1] = __ffma2_rn(qd, r1, acc[i][1]);
-                    acc[i][2] = __ffma2_rn(qd, r2, acc[i][2]);
-                    acc[i][3] = __ffma2_rn(qd, r3, acc[i][3]);
+                    for (int i = 0; i < 8; ++i) {
+                        const float2 qd = make_float2(qv[i], qv[i]);
+                        acc[i][0] = __ffma2_rn(qd, r0, acc[i][0]);
+                        acc[i][1] = __ffma2_rn(qd, r1, acc[i][1]);
+                        acc[i][2] = __ffma2_rn(qd, r2, acc[i][2]);
+                        acc[i][3] = __ffma2_rn(qd, r3, acc[i][3]);
+                    }
+                }
+            }
+        } else {
+            // one FADD2 forms the differences q_k - r_k of two references; L1 adds their magnitudes
+            // with a second FADD2 (|.| is an operand modifier), L-inf takes two FMNMX
+            for (int k0 = 0; k0 < dpad; k0 += 8) {
+#pragma unroll
+                for (int kk = 0; kk < 8; ++kk) {
+                    const int k = k0 + kk;
+                    const float4 qa = *reinterpret_cast<const float4 *>(qp + k * QTILE);
+                    const float4 qb = *reinterpret_cast<const float4 *>(qp + k * QTILE + 16);
+                    const float4 ra = *reinterpret_cast<const float4 *>(rp + k * RTILE);
+                    const float4 rb = *reinterpret_cast<const float4 *>(rp + k * RTILE + 32);
+                    const float2 nr[4] = {make_float2(-ra.x, -ra.y), make_float2(-ra.z, -ra.w),
+                                          make_float2(-rb.x, -rb.y), make_float2(-rb.z, -rb.w)};
+                    const float qv[8] = {qa.x, qa.y, qa.z, qa.w, qb.x, qb.y, qb.z, qb.w};
+#pragma unroll
+                    for (int i = 0; i < 8; ++i) {
+                        const float2 qd = make_float2(qv[i], qv[i]);
+#pragma unroll
+                        for (int c = 0; c < 4; ++c) {
+                            const float2 t = __fadd2_rn(qd, nr[c]);
+                            if constexpr (M == METRIC_L1) {
+                                acc[i][c] = __fadd2_rn(acc[i][c], make_float2(fabsf(t.x), fabsf(t.y)));
+                            } else {
+                                acc[i][c].x = fmaxf(acc[i][c].x, fabsf(t.x));
+                                acc[i][c].y = fmaxf(acc[i][c].y, fabsf(t.y));
+                            }
+                        }
+                    }
                 }
             }
         }
@@ -250,31 +285,44 @@ int search_simt_pick_stages(int dpad, int kc) {
     return 0;
 }
 
-template <int KC>
+template <int KC, int M>
 static cudaError_t launch_kc(const float *qimg, const float *rimg, int dpad, int n_rtiles,
                              long long n_q, int *cand_idx, float *cand_thr, const int *n_rows_dev,
                              int spread_ctas, int bypass_rows, cudaStream_t st) {
     const int nstage = search_simt_pick_stages(dpad, KC);
     if (nstage == 0) return cudaErrorInvalidValue;
     const size_t smem = search_simt_smem_bytes(dpad, KC, nstage);
-    cudaError_t e = cudaFuncSetAttribute(search_simt_kernel<KC>,
+    cudaError_t e = cudaFuncSetAttribute(search_simt_kernel<KC, M>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e != cudaSuccess) return e;
     const long long n_qtiles = (n_q + QTILE - 1) / QTILE;
     const long long grid = n_rows_dev && spread_ctas > n_qtiles ? spread_ctas : n_qtiles;
-    search_simt_kernel<KC><<<(unsigned)grid, SEARCH_THREADS, smem, st>>>(
+    search_simt_kernel<KC, M><<<(unsigned)grid, SEARCH_THREADS, smem, st>>>(
         qimg, rimg, dpad, n_rtiles, nstage, n_q, cand_idx, cand_thr, n_rows_dev, spread_ctas, bypass_rows);
     return cudaGetLastError();
 }
 
+template <int M>
+static cudaError_t launch_metric(const float *qimg, const float *rimg, int dpad, int n_rtiles, long long n_q,
+                                 int kc, int *cand_idx, float *cand_thr, const int *n_rows_dev, int spread_ctas,
+                                 int bypass_rows, cudaStream_t st) {
+    switch (kc) {
+        case 8: return launch_kc<8, M>(qimg, rimg, dpad, n_rtiles, n_q, cand_idx, cand_thr, n_rows_dev, spread_ctas, bypass_rows, st);
+        case 16: return launch_kc<16, M>(qimg, rimg, dpad, n_rtiles, n_q, cand_idx, cand_thr, n_rows_dev, spread_ctas, bypass_rows, st);
+        case 32: return launch_kc<32, M>(qimg, rimg, dpad, n_rtiles, n_q, cand_idx, cand_thr, n_rows_dev, spread_ctas, bypass_rows, st);
+        default: return cudaErrorInvalidValue;
+    }
+}
+
 cudaError_t launch_search_simt(const float *qimg, const float *rimg, int dpad, int n_rtiles,
                                long long n_q, int kc, int *cand_idx, float *cand_thr,
-                               const int *n_rows_dev, int spread_ctas, int bypass_rows, cudaStream_t st) {
+                               const int *n_rows_dev, int spread_ctas, int bypass_rows, cudaStream_t st,
+                               int metric) {
     if (n_q <= 0) return cudaSuccess;
-    switch (kc) {
-        case 8: return launch_kc<8>(qimg, rimg, dpad, n_rtiles, n_q, cand_idx, cand_thr, n_rows_dev, spread_ctas, bypass_rows, st);
-        case 16: return launch_kc<16>(qimg, rimg, dpad, n_rtiles, n_q, cand_idx, cand_thr, n_rows_dev, spread_ctas, bypass_rows, st);
-        case 32: return launch_kc<32>(qimg, rimg, dpad, n_rtiles, n_q, cand_idx, cand_thr, n_rows_dev, spread_ctas, bypass_rows, st);
+    switch (metric) {
+        case METRIC_L2: return launch_metric<METRIC_L2>(qimg, rimg, dpad, n_rtiles, n_q, kc, cand_idx, cand_thr, n_rows_dev, spread_ctas, bypass_rows, st);
+        case METRIC_L1: return launch_metric<METRIC_L1>(qimg, rimg, dpad, n_rtiles, n_q, kc, cand_idx, cand_thr, n_rows_dev, spread_ctas, bypass_rows, st);
+        case METRIC_LINF: return launch_metric<METRIC_LINF>(qimg, rimg, dpad, n_rtiles, n_q, kc, cand_idx, cand_thr, n_rows_dev, spread_ctas, bypass_rows, st);
         default: return cudaErrorInvalidValue;
     }
 }

@@ -32,7 +32,7 @@ def _regressor_and_image(est, image):
         raise ValueError(f"X has {image.shape[0]} features, but {type(est).__name__} is expecting "
                          f"{n_bands} features as input.")
     ix = reg._get_index()
-    if kind == "euclidean":
+    if kind != "hamming":
         if hasattr(est, "transformer_") and not est._fusable():
             raise NotImplementedError("the estimator's transformer is not an affine map")
         query = ix.query_raster
