@@ -38,9 +38,21 @@ extern "C" {
 #define SKNNR_EUNSUP (-5)   /* shape outside what the kernels cover                    */
 #define SKNNR_ENONFINITE (-6) /* SKNNR_CHECK_FINITE: a query value is NaN or +-inf      */
 
-/* dtype of a query matrix */
+/* dtype of a query matrix or raster block (x_dtype).  Every call that takes an x_dtype reads these
+ * element types as they are, from host or device memory: host buffers are copied to the device at
+ * their own element size, and the kernels convert each value to float64 as they load it
+ * (integers exactly below 2^53, int64 beyond rounded to nearest, as NumPy's cast to float64 does).
+ * Results therefore equal those of the same values passed as float64.  An integer input holds no
+ * NaN / inf: SKNNR_CHECK_FINITE has nothing to check, and a raster pixel of integer bands is masked
+ * only by `nodata`.  The forest walk rounds an integer to float32 through float64, as it rounds a
+ * float64 input.  Any other code: SKNNR_EINVAL. */
 #define SKNNR_F64 0
 #define SKNNR_F32 1
+#define SKNNR_U8 2
+#define SKNNR_I16 3
+#define SKNNR_U16 4
+#define SKNNR_I32 5
+#define SKNNR_I64 6
 
 /* flags for the query calls */
 #define SKNNR_EXCLUDE_SELF 1u   /* X=None semantics: search k+1, drop the query itself

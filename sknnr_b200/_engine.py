@@ -103,6 +103,30 @@ def _ptr(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
 
 
+def _native(X):
+    """``X`` as an array the library reads as it is (float64, float32, uint8, int16, uint16, int32,
+    int64) and its ``x_dtype`` code; any other dtype is converted to float64 (exact for every integer
+    below 2^53, so the results equal those of ``X.astype(np.float64)`` either way)."""
+    X = np.asarray(X)
+    code = L.x_dtype_code(X)
+    if code is None:
+        X = np.asarray(X, dtype=np.float64)
+        code = L.F64
+    return X, code
+
+
+def _raster_nodata(nodata, dtype):
+    """The float64 that the device compares every band value with.  A float band's nodata is first
+    rounded to the band's own type, as an ``image == nodata`` test on the host would do; an integer
+    band's stays the float64 given (``dtype.type(nodata)`` would truncate or overflow it), so a
+    nodata that is no value of the band type masks nothing."""
+    if nodata is None:
+        return None
+    if np.dtype(dtype).kind == "f":
+        return float(np.dtype(dtype).type(nodata))
+    return float(nodata)
+
+
 def _f64(a, ndim=None):
     if a is None:
         return None
@@ -176,9 +200,7 @@ def _raster_call(index, fn, handles, n_bands, bands, k, *, nodata=None, determin
                  weights=None, with_pred=False, return_distance=True, return_index=True, fill_dist=np.nan,
                  fill_idx=-1, fill_pred=np.nan, out_dist=None, out_idx=None, out_pred=None):
     """Shared body of the raster entry points (sknnr_raster_kneighbors and its Hamming + forest twin)."""
-    bands = np.asarray(bands)
-    if bands.dtype != np.float32:
-        bands = np.asarray(bands, dtype=np.float64)
+    bands, dt = _native(bands)
     if bands.ndim != 2 or bands.shape[0] != n_bands:
         raise ValueError(f"the image has {bands.shape[0] if bands.ndim == 2 else '?'} bands, "
                          f"but {n_bands} are expected")
@@ -200,11 +222,8 @@ def _raster_call(index, fn, handles, n_bands, bands, k, *, nodata=None, determin
     idx = _out(out_idx, (k, n_pix), np.int64) if return_index else None
     pred = _out(out_pred, (index.n_out, n_pix), np.float64) if mode != L.W_NONE else None
     n_valid = C.c_int64(0)
-    if nodata is not None:
-        # the comparison happens in float64 on the device: a nodata literal is first rounded to the
-        # bands' own type, as an `image == nodata` test on the host would do
-        nodata = float(bands.dtype.type(nodata))
-    L.check(fn(*handles, _ptr(bands), L.F32 if bands.dtype == np.float32 else L.F64, n_pix, stride,
+    nodata = _raster_nodata(nodata, bands.dtype)
+    L.check(fn(*handles, _ptr(bands), dt, n_pix, stride,
                0 if nodata is None else 1, 0.0 if nodata is None else float(nodata), int(k),
                index._flags(False, deterministic), int(decimals), _ptr(dist), _ptr(idx), mode, _ptr(pred),
                float(fill_dist), int(fill_idx), float(fill_pred), C.byref(n_valid)))
@@ -267,14 +286,12 @@ class KNNIndex(_IndexBase):
         if exclude_self:
             n_q, Xp, dt, ldx = self.n_ref, None, L.F64, 0
         else:
-            X = np.asarray(X)
-            if X.dtype != np.float32:
-                X = np.asarray(X, dtype=np.float64)
+            X, dt = _native(X)
             if X.ndim != 2:
                 raise ValueError("X must be 2-D")
             if X.strides[1] != X.itemsize or X.strides[0] % X.itemsize or X.strides[0] < X.shape[1] * X.itemsize:
                 X = np.ascontiguousarray(X)
-            n_q, dt = X.shape[0], (L.F32 if X.dtype == np.float32 else L.F64)
+            n_q = X.shape[0]
             ldx = X.strides[0] // X.itemsize if n_q > 1 else X.shape[1]
             want = self.d_out if transformed else self.d_in
             if X.shape[1] != want:
@@ -292,8 +309,9 @@ class KNNIndex(_IndexBase):
 
     # -- raster query: band-major image in, band-major layers out (scope row f4) -------
     def query_raster(self, bands, k, **kw):
-        """``bands``: ``[d_in, n_pix]`` float32/float64, pixels contiguous within a band (bands may
-        be strided).  A pixel with a NaN / inf band, or a band equal to ``nodata``, is masked and
+        """``bands``: ``[d_in, n_pix]`` float64, float32, uint8, int16, uint16, int32 or int64 (any other
+        dtype is converted to float64), pixels contiguous within a band (bands may be strided).  A pixel
+        with a NaN / inf band, or a band equal to ``nodata``, is masked and
         receives the fill values; the others are queried in pixel order.  Returns
         ``(dist [k, n_pix], idx [k, n_pix], pred [n_out, n_pix], n_valid)``; ``out_*`` are optional
         preallocated C-contiguous result arrays (e.g. from :func:`pinned_empty`)."""
@@ -302,25 +320,28 @@ class KNNIndex(_IndexBase):
     # -- device-pointer query (benchmarks, multi-GPU pipelines) -------------------------
     def query_device(self, x_ptr, x_is_f32, n_q, ldx, k, *, dist_ptr=0, idx_ptr=0, pred_ptr=0,
                      weights=None, deterministic=True, decimals=10, row_offset=0,
-                     transformed=False, stream=0):
+                     transformed=False, stream=0, x_dtype=None):
+        """``x_dtype``: NumPy dtype of the rows at ``x_ptr`` (one :func:`_lib.x_dtype_code` maps);
+        when given it takes the place of ``x_is_f32``."""
         mode = _weights_mode(weights, bool(pred_ptr))
         flags = self._flags(False, deterministic, transformed) | L.DEVICE_PTRS
+        if x_dtype is not None:
+            dt = L.x_dtype_code(np.dtype(x_dtype))
+            if dt is None:
+                raise ValueError(f"the device reads no {np.dtype(x_dtype)} rows")
+        else:
+            dt = L.F32 if x_is_f32 else L.F64
         L.check(self._lib.sknnr_kneighbors(
-            self._h, C.c_void_p(x_ptr), L.F32 if x_is_f32 else L.F64, int(n_q), int(ldx),
+            self._h, C.c_void_p(x_ptr), dt, int(n_q), int(ldx),
             int(row_offset), int(k), flags, int(decimals), C.c_void_p(dist_ptr or None),
             C.c_void_p(idx_ptr or None), mode, C.c_void_p(pred_ptr or None),
             C.c_void_p(stream or None)))
 
     def transform(self, X):
-        X = np.asarray(X)
-        if X.dtype != np.float32:
-            X = np.ascontiguousarray(X, dtype=np.float64)
-        else:
-            X = np.ascontiguousarray(X)
+        X, dt = _native(X)
+        X = np.ascontiguousarray(X)
         out = np.empty((X.shape[0], self.d_out), dtype=np.float64)
-        L.check(self._lib.sknnr_transform(
-            self._h, _ptr(X), L.F32 if X.dtype == np.float32 else L.F64, X.shape[0], X.shape[1],
-            _ptr(out)))
+        L.check(self._lib.sknnr_transform(self._h, _ptr(X), dt, X.shape[0], X.shape[1], _ptr(out)))
         return out
 
     def weighted_average(self, idx, w):
@@ -373,9 +394,7 @@ class HammingIndex(_IndexBase):
                      weights=None, with_pred=False, return_distance=True, return_index=True, out=None):
         """kneighbors (+ predict) on RAW feature rows: forest walk -> node codes -> Hamming
         search in one device call (sknnr_hamming_kneighbors_forest)."""
-        X = np.asarray(X)
-        if X.dtype != np.float32:
-            X = np.asarray(X, dtype=np.float64)
+        X, dt = _native(X)
         X = np.ascontiguousarray(X)
         if X.ndim != 2 or X.shape[1] != forest.n_features:
             raise ValueError(f"X has {X.shape[1] if X.ndim == 2 else '?'} features, but "
@@ -384,7 +403,7 @@ class HammingIndex(_IndexBase):
         mode = _weights_mode(weights, with_pred)
         dist, idx, pred = _outputs(out, n_q, k, self.n_out, return_distance, return_index, mode)
         L.check(self._lib.sknnr_hamming_kneighbors_forest(
-            self._h, forest._h, _ptr(X), L.F32 if X.dtype == np.float32 else L.F64, n_q, X.shape[1],
+            self._h, forest._h, _ptr(X), dt, n_q, X.shape[1],
             int(row_offset), int(k), self._flags(False, deterministic), int(decimals), _ptr(dist),
             _ptr(idx), mode, _ptr(pred), None))
         return dist, idx, pred
@@ -455,13 +474,10 @@ class ForestIndex:
 
     def apply(self, X) -> np.ndarray:
         """Node ID of every tree for every row, int64 ``[n, n_trees]`` (== hstack of est.apply)."""
-        X = np.asarray(X)
-        if X.dtype != np.float32:
-            X = np.asarray(X, dtype=np.float64)
+        X, dt = _native(X)
         X = np.ascontiguousarray(X)
         out = np.empty((X.shape[0], self.n_trees), dtype=np.int32)
-        L.check(self._lib.sknnr_forest_apply(self._h, _ptr(X), L.F32 if X.dtype == np.float32 else L.F64,
-                                             X.shape[0], X.shape[1], _ptr(out)))
+        L.check(self._lib.sknnr_forest_apply(self._h, _ptr(X), dt, X.shape[0], X.shape[1], _ptr(out)))
         return out.astype(np.int64)
 
     def close(self):

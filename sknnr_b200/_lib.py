@@ -10,16 +10,31 @@ from __future__ import annotations
 import ctypes as C
 import os
 
+import numpy as np
+
 from ._build import lib_path
 
 # mirrors include/sknnr_b200.h
 ABI_VERSION = 1
-F64, F32 = 0, 1
+F64, F32, U8, I16, U16, I32, I64 = 0, 1, 2, 3, 4, 5, 6
 EXCLUDE_SELF, DETERMINISTIC, TRANSFORMED, DEVICE_PTRS, CHECK_FINITE = 1, 2, 4, 8, 16
 W_NONE, W_UNIFORM, W_DISTANCE = 0, 1, 2
 ENGINE_AUTO, ENGINE_SIMT, ENGINE_TENSOR, ENGINE_EXACT = 0, 1, 2, 3
 METRICS = {"euclidean": 0, "manhattan": 1, "chebyshev": 2}   # SKNNR_METRIC_*
 MAX_CODE = 31743
+
+# integer element types the query calls read as they are (no float64 copy on the host)
+NATIVE_INT_DTYPES = (np.uint8, np.int16, np.uint16, np.int32, np.int64)
+_X_DTYPE_CODES = {np.dtype(t): c for t, c in ((np.float64, F64), (np.float32, F32), (np.uint8, U8),
+                                              (np.int16, I16), (np.uint16, U16), (np.int32, I32),
+                                              (np.int64, I64))}
+
+
+def x_dtype_code(arr):
+    """The ``x_dtype`` code under which the library reads ``arr`` (an array or a dtype) as it is:
+    float64, float32, uint8, int16, uint16, int32 or int64 in native byte order.  None for any
+    other dtype, which the caller converts to float64 first."""
+    return _X_DTYPE_CODES.get(np.dtype(getattr(arr, "dtype", arr)))
 
 EXPORTS = [
     "sknnr_last_error", "sknnr_abi_version", "sknnr_device_count", "sknnr_set_option",

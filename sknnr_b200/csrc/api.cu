@@ -918,7 +918,7 @@ int sknnr_index_cascade_counts(sknnr_index *ix, int64_t *out3) {
 //   2. SIMT   (FP32 FFMA2 scores, eps ~(2d+8) 2^-24) on the compacted rows of L1b -> refine -> L2
 //   3. exact  (float64, exhaustive) on L2
 // With engine = SIMT stage 1 is skipped (L1 = all rows); with engine = EXACT only stage 3 runs.
-static int run_chunk(sknnr_index *ix, Slot &s, const void *dX, int x_f32, int64_t ldx, bool transformed,
+static int run_chunk(sknnr_index *ix, Slot &s, const void *dX, int x_dtype, int64_t ldx, bool transformed,
                      int64_t rows, int64_t row0, int k, uint32_t flags, int decimals, int weights,
                      double *o_dist, long long *o_idx, double *o_pred, bool check_finite = false) {
     const bool excl = flags & SKNNR_EXCLUDE_SELF;
@@ -961,7 +961,7 @@ static int run_chunk(sknnr_index *ix, Slot &s, const void *dX, int x_f32, int64_
     CK(s.z64.reserve((size_t)rows * ix->d_out));
     if (engine != SKNNR_ENGINE_EXACT) CK(s.qimg.reserve((size_t)prow * ix->dpad));
     if (use_tc) CK(s.qimg_tc.reserve((size_t)prow * ix->kc_tot * 8));
-    CK(launch_project(dX, x_f32, ldx, rows, transformed ? ix->d_out : ix->d_in, ix->d_out, ix->dpad,
+    CK(launch_project(dX, x_dtype, ldx, rows, transformed ? ix->d_out : ix->d_in, ix->d_out, ix->dpad,
                       transformed ? nullptr : ix->d_center, transformed ? nullptr : ix->d_scale,
                       transformed ? nullptr : ix->d_proj, ix->d_mu, s.z64.p,
                       use_simt_first ? s.qimg.p : nullptr, use_tc ? s.qimg_tc.p : nullptr, ix->kc_tot,
@@ -1062,7 +1062,7 @@ static int run_chunk(sknnr_index *ix, Slot &s, const void *dX, int x_f32, int64_
             // dropped on the way, the pass costs a few CTAs, and the FP32 engine is left with the rows
             // that have more than 15 references inside the FP16 error margin of their k-th neighbour.
             CK(launch_gather_rows(s.z64.p, ix->d_out, list, count, rows, s.z64c.p, st));
-            CK(launch_project(s.z64c.p, 0, ix->d_out, rows, ix->d_out, ix->d_out, ix->dpad, nullptr, nullptr,
+            CK(launch_project(s.z64c.p, SKNNR_F64, ix->d_out, rows, ix->d_out, ix->d_out, ix->dpad, nullptr, nullptr,
                               nullptr, ix->d_mu, nullptr, nullptr, s.qimg_tc.p, ix->kc_tot, ix->tc_sigma, count,
                               nullptr, st));
             // (one stream of 16 whatever the first pass used: what the two-stream layout cannot certify
@@ -1087,7 +1087,7 @@ static int run_chunk(sknnr_index *ix, Slot &s, const void *dX, int x_f32, int64_
         }
         // stage 2 input: gather the uncertified rows and rebuild their FP32 query image
         CK(launch_gather_rows(s.z64.p, ix->d_out, list, count, rows, s.z64c.p, st));
-        CK(launch_project(s.z64c.p, 0, ix->d_out, rows, ix->d_out, ix->d_out, ix->dpad, nullptr, nullptr,
+        CK(launch_project(s.z64c.p, SKNNR_F64, ix->d_out, rows, ix->d_out, ix->d_out, ix->dpad, nullptr, nullptr,
                           nullptr, ix->d_mu, nullptr, s.qimg.p, nullptr, 0, 1.0, count, nullptr, st));
         ix->stats.kernel_launches += 4;
         stage2_count = count;
@@ -1161,7 +1161,7 @@ int sknnr_kneighbors(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_
     int kk = 0;
     int rc = check_query_args(ix->n_ref, ix->n_out, n_q, k, flags, weights, X, out_pred, kk);
     if (rc != SKNNR_OK) return rc;
-    if (x_dtype != SKNNR_F64 && x_dtype != SKNNR_F32) return fail(SKNNR_EINVAL, "bad x_dtype");
+    if (x_dtype_size(x_dtype) == 0) return fail(SKNNR_EINVAL, "bad x_dtype");
     std::lock_guard<std::mutex> g(ix->lock);
     CK(cudaSetDevice(ix->device));
 
@@ -1179,7 +1179,7 @@ int sknnr_kneighbors(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_
     }
     const int cols = transformed ? ix->d_out : ix->d_in;
     if (ldx < cols) return fail(SKNNR_EINVAL, "ldx smaller than the number of features");
-    const size_t esz = x_dtype == SKNNR_F32 ? 4 : 8;
+    const size_t esz = x_dtype_size(x_dtype);
     // A synchronous call takes any mix of host and device pointers (unified addressing): device
     // resident X is read in place, and results bound for device memory - this GPU's or a peer's
     // mapped through sknnr_ipc_open - leave each chunk as one copy-engine transfer on the D2H
@@ -1212,7 +1212,9 @@ int sknnr_kneighbors(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_
     const bool stage_idx = !dev_ptrs && out_idx && is_pageable(out_idx);
     const bool stage_pred = !dev_ptrs && weights != SKNNR_W_NONE && is_pageable(out_pred);
     const bool staged = stage_in || stage_dist || stage_idx || stage_pred;
-    const bool check_finite = (flags & SKNNR_CHECK_FINITE) && !dev_ptrs && !excl;
+    // (an integer matrix cannot hold NaN / inf: nothing to check)
+    const bool check_finite = (flags & SKNNR_CHECK_FINITE) && !dev_ptrs && !excl &&
+                              (x_dtype == SKNNR_F64 || x_dtype == SKNNR_F32);
     // device-resident queries have no copies to overlap: twice the chunk (fewer launches and cascade
     // tails; measured +1.8 %), while host buffers prefer the shorter pipeline ramp of the smaller one
     int64_t chunk = dev_ptrs ? 2 * g_opt.chunk_rows : (staged ? std::min(g_opt.stage_rows, g_opt.chunk_rows) : g_opt.chunk_rows);
@@ -1303,7 +1305,7 @@ int sknnr_kneighbors(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_
         // others keep to a few SMs, which costs the following chunk's tensor kernel less
         ix->spread_tail = r0 + rows >= n_q;
         CK(trace_mark(1, cin));
-        rc = run_chunk(ix, s, dX, x_dtype == SKNNR_F32, dld, transformed, rows, row_offset + r0, k,
+        rc = run_chunk(ix, s, dX, x_dtype, dld, transformed, rows, row_offset + r0, k,
                        flags, decimals, weights, o_dist, o_idx, o_pred, check_finite);
         if (rc != SKNNR_OK) return rc;
         if (!dev_ptrs) {
@@ -1387,11 +1389,11 @@ static int raster_impl(IX *ix, int d, const void *bands, int32_t x_dtype, int64_
     int kk = 0;
     int rc = check_query_args(ix->n_ref, ix->n_out, n_pix, k, flags, weights, bands, out_pred, kk);
     if (rc != SKNNR_OK) return rc;
-    if (x_dtype != SKNNR_F64 && x_dtype != SKNNR_F32) return fail(SKNNR_EINVAL, "bad x_dtype");
+    if (x_dtype_size(x_dtype) == 0) return fail(SKNNR_EINVAL, "bad x_dtype");
     if (band_stride < n_pix) return fail(SKNNR_EINVAL, "band_stride smaller than the number of pixels");
     std::lock_guard<std::mutex> g(ix->lock);
     CK(cudaSetDevice(ix->device));
-    const size_t esz = x_dtype == SKNNR_F32 ? 4 : 8;
+    const size_t esz = x_dtype_size(x_dtype);
     CallGuard guard(ix, nullptr);
     for (auto &s : ix->slots) CK(ix->finish_slot(s));
     for (auto &s : ix->slots) { s.ev_used = 0; s.fb_pending = false; s.flag_pending = false; }
@@ -1416,7 +1418,7 @@ static int raster_impl(IX *ix, int d, const void *bands, int32_t x_dtype, int64_
                              cudaMemcpyHostToDevice, s.stream));
         ix->stats.h2d_bytes += rows * d * (int64_t)esz;
         const int groups = (int)((rows + RASTER_GROUP - 1) / RASTER_GROUP);
-        CK(launch_raster_mask(s.x.p, x_dtype == SKNNR_F32, rows, d, use_nodata, nodata, s.r_pos.p,
+        CK(launch_raster_mask(s.x.p, x_dtype, rows, d, use_nodata, nodata, s.r_pos.p,
                               s.r_cnt.p, s.r_cnt.p + groups + 1, s.stream));
         CK(cudaMemcpyAsync(s.h_cnt, s.r_cnt.p + groups + 1, sizeof(int), cudaMemcpyDeviceToHost, s.stream));
         CK(cudaEventRecord(s.ev_cnt, s.stream));
@@ -1437,7 +1439,7 @@ static int raster_impl(IX *ix, int d, const void *bands, int32_t x_dtype, int64_
         long long *o_idx = nullptr;
         // (with nv == 0 the gather only turns the all-zero flags into "-1 = masked")
         CK(s.xc.reserve((size_t)std::max<int64_t>(nv, 1) * d * esz));
-        CK(launch_raster_gather(s.x.p, x_dtype == SKNNR_F32, rows, d, s.r_cnt.p, s.r_pos.p, s.xc.p, s.stream));
+        CK(launch_raster_gather(s.x.p, x_dtype, rows, d, s.r_cnt.p, s.r_pos.p, s.xc.p, s.stream));
         ix->stats.kernel_launches++;
         if (nv > 0) {
             if (out_dist) { CK(s.o_dist.reserve((size_t)nv * k)); o_dist = s.o_dist.p; }
@@ -1495,7 +1497,7 @@ int sknnr_raster_kneighbors(sknnr_index *ix, const void *bands, int32_t x_dtype,
                            if (ix->chunk_rows_seen >= 4096 && ix->chunk_fb_seen * 3 > ix->chunk_rows_seen)
                                ix->tensor_demoted[ix->ns_in_use] = true;
                            ix->spread_tail = false;
-                           return run_chunk(ix, s, xc, x_dtype == SKNNR_F32, ix->d_in, false, nv, row0, k, flags,
+                           return run_chunk(ix, s, xc, x_dtype, ix->d_in, false, nv, row0, k, flags,
                                             decimals, weights, o_dist, o_idx, o_pred);
                        });
 }
@@ -1504,9 +1506,10 @@ int sknnr_transform(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_q
                     double *out_z) {
     if (!ix || !X || !out_z || n_q < 0) return fail(SKNNR_EINVAL, "NULL argument");
     if (ldx < ix->d_in) return fail(SKNNR_EINVAL, "ldx smaller than the number of features");
+    if (x_dtype_size(x_dtype) == 0) return fail(SKNNR_EINVAL, "bad x_dtype");
     std::lock_guard<std::mutex> g(ix->lock);
     CK(cudaSetDevice(ix->device));
-    const size_t esz = x_dtype == SKNNR_F32 ? 4 : 8;
+    const size_t esz = x_dtype_size(x_dtype);
     Slot &s = ix->slots[0];
     const int64_t chunk = g_opt.chunk_rows;
     for (int64_t r0 = 0; r0 < n_q; r0 += chunk) {
@@ -1516,7 +1519,7 @@ int sknnr_transform(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_q
         CK(cudaMemcpy2DAsync(s.x.p, (size_t)ix->d_in * esz, (const unsigned char *)X + (size_t)r0 * ldx * esz,
                              (size_t)ldx * esz, (size_t)ix->d_in * esz, (size_t)rows,
                              cudaMemcpyHostToDevice, s.stream));
-        CK(launch_project(s.x.p, x_dtype == SKNNR_F32, ix->d_in, rows, ix->d_in, ix->d_out, ix->dpad,
+        CK(launch_project(s.x.p, x_dtype, ix->d_in, rows, ix->d_in, ix->d_out, ix->dpad,
                           ix->d_center, ix->d_scale, ix->d_proj, ix->d_mu, s.z64.p, nullptr, nullptr, 0, 1.0, nullptr, nullptr,
                           s.stream));
         CK(cudaMemcpyAsync(out_z + r0 * ix->d_out, s.z64.p, (size_t)rows * ix->d_out * 8,
@@ -1754,7 +1757,7 @@ static int hamming_kneighbors_impl(sknnr_hamming_index *ix, sknnr_forest *forest
     if (forest) {
         if (forest->n_trees != ix->n_trees) return fail(SKNNR_EINVAL, "forest and index disagree on the number of trees");
         if (forest->device != ix->device) return fail(SKNNR_EINVAL, "forest and index live on different devices");
-        if (x_dtype != SKNNR_F64 && x_dtype != SKNNR_F32) return fail(SKNNR_EINVAL, "bad x_dtype");
+        if (x_dtype_size(x_dtype) == 0) return fail(SKNNR_EINVAL, "bad x_dtype");
     }
     std::lock_guard<std::mutex> g(ix->lock);
     CK(cudaSetDevice(ix->device));
@@ -1770,7 +1773,7 @@ static int hamming_kneighbors_impl(sknnr_hamming_index *ix, sknnr_forest *forest
     }
     if (!forest && ldq < ix->n_trees) return fail(SKNNR_EINVAL, "ldq smaller than the number of trees");
     if (forest && ldq < forest->n_features) return fail(SKNNR_EINVAL, "ldx smaller than the number of features");
-    const size_t xesz = x_dtype == SKNNR_F32 ? 4 : 8;
+    const size_t xesz = x_dtype_size(x_dtype);
     cudaStream_t user_stream = dev_ptrs ? (cudaStream_t)stream : nullptr;
     CallGuard guard(ix, user_stream);
     if (dev_ptrs) {
@@ -1808,7 +1811,7 @@ static int hamming_kneighbors_impl(sknnr_hamming_index *ix, sknnr_forest *forest
                 dldx = cols;
             }
             CK(s.codes.reserve((size_t)rows * ix->n_trees));
-            CK(launch_forest_apply(dX, x_dtype == SKNNR_F32, dldx, rows, forest->n_features, forest->d_nodes,
+            CK(launch_forest_apply(dX, x_dtype, dldx, rows, forest->n_features, forest->d_nodes,
                                    forest->d_roots, forest->n_trees, s.codes.p, nullptr, ix->n_trees, s.stream));
             ix->stats.kernel_launches++;
             dq = s.codes.p;
@@ -1878,7 +1881,7 @@ int sknnr_hamming_raster_kneighbors_forest(sknnr_hamming_index *ix, sknnr_forest
                        [&](Slot &s, const void *xc, int64_t nv, int64_t row0, double *o_dist, long long *o_idx,
                            double *o_pred) -> int {
                            CK(s.codes.reserve((size_t)nv * ix->n_trees));
-                           CK(launch_forest_apply(xc, x_dtype == SKNNR_F32, forest->n_features, nv,
+                           CK(launch_forest_apply(xc, x_dtype, forest->n_features, nv,
                                                   forest->n_features, forest->d_nodes, forest->d_roots,
                                                   forest->n_trees, s.codes.p, nullptr, ix->n_trees, s.stream));
                            ix->stats.kernel_launches++;
@@ -1980,10 +1983,10 @@ int sknnr_forest_apply(sknnr_forest *f, const void *X, int32_t x_dtype, int64_t 
                        int32_t *out_ids) {
     if (!f || !X || !out_ids || n_q < 0) return fail(SKNNR_EINVAL, "NULL argument");
     if (ldx < f->n_features) return fail(SKNNR_EINVAL, "ldx smaller than the number of features");
-    if (x_dtype != SKNNR_F64 && x_dtype != SKNNR_F32) return fail(SKNNR_EINVAL, "bad x_dtype");
+    if (x_dtype_size(x_dtype) == 0) return fail(SKNNR_EINVAL, "bad x_dtype");
     std::lock_guard<std::mutex> g(f->lock);
     CK(cudaSetDevice(f->device));
-    const size_t esz = x_dtype == SKNNR_F32 ? 4 : 8;
+    const size_t esz = x_dtype_size(x_dtype);
     const int64_t chunk = g_opt.chunk_rows;
     for (int64_t r0 = 0; r0 < n_q; r0 += chunk) {
         const int64_t rows = std::min(chunk, n_q - r0);
@@ -1992,7 +1995,7 @@ int sknnr_forest_apply(sknnr_forest *f, const void *X, int32_t x_dtype, int64_t 
         CK(cudaMemcpy2DAsync(f->x.p, (size_t)f->n_features * esz, (const unsigned char *)X + (size_t)r0 * ldx * esz,
                              (size_t)ldx * esz, (size_t)f->n_features * esz, (size_t)rows, cudaMemcpyHostToDevice,
                              f->stream));
-        CK(launch_forest_apply(f->x.p, x_dtype == SKNNR_F32, f->n_features, rows, f->n_features, f->d_nodes,
+        CK(launch_forest_apply(f->x.p, x_dtype, f->n_features, rows, f->n_features, f->d_nodes,
                                f->d_roots, f->n_trees, nullptr, f->ids.p, f->n_trees, f->stream));
         CK(cudaMemcpyAsync(out_ids + r0 * f->n_trees, f->ids.p, (size_t)rows * f->n_trees * 4, cudaMemcpyDeviceToHost,
                            f->stream));

@@ -38,6 +38,17 @@ constexpr int MAXK = 32;        // entries handled by one warp-wide sort
 constexpr int TC_M = 128;
 constexpr int TC_N = 128;
 
+// A query value as float64, whatever the element type of the caller's matrix (kernels.h, with_x_type).
+// Every integer of these types below 2^53 converts exactly; int64 beyond rounds to nearest, as NumPy's
+// cast to float64 does - so the rest of a kernel sees the values the float64 path would.
+__device__ __forceinline__ double x_to_f64(double v) { return v; }
+__device__ __forceinline__ double x_to_f64(float v) { return (double)v; }
+__device__ __forceinline__ double x_to_f64(uint8_t v) { return __uint2double_rn(v); }
+__device__ __forceinline__ double x_to_f64(int16_t v) { return __int2double_rn(v); }
+__device__ __forceinline__ double x_to_f64(uint16_t v) { return __uint2double_rn(v); }
+__device__ __forceinline__ double x_to_f64(int32_t v) { return __int2double_rn(v); }
+__device__ __forceinline__ double x_to_f64(long long v) { return __ll2double_rn(v); }
+
 // ---------------------------------------------------------------------------------------
 // mbarrier + 1-D TMA bulk copy (cp.async.bulk -> SASS UBLKCP)
 // ---------------------------------------------------------------------------------------

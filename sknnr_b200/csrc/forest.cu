@@ -6,7 +6,8 @@
 // host between the forest and the neighbour search.
 //
 // Semantics replicated bit for bit from scikit-learn's Tree._apply_dense:
-//   * X is cast to float32 first (DTYPE), so float64 inputs are rounded to nearest even;
+//   * X is cast to float32 first (DTYPE), so float64 inputs are rounded to nearest even (integer
+//     inputs are read as they are and converted through float64, see walk_value);
 //   * at an internal node go left iff (double)x[feature] <= threshold (threshold is float64) - for
 //     a float32 x that is x <= (largest float32 <= threshold), which is what the 16-byte nodes hold;
 //     NaN follows the node's missing_go_to_left flag;
@@ -20,11 +21,25 @@
 #include "common.cuh"
 #include "kernels.h"
 
+#include <type_traits>
+
 namespace sk {
 
 constexpr int FOREST_THREADS = 256;  // queries per CTA
 constexpr int FOREST_TG = 32;        // trees per staging group
 constexpr int FOREST_ILP = 2;        // trees walked concurrently by one thread
+
+// The float32 a query value is walked with.  An integer goes through float64 first: that is the value
+// an integer array had on the float64 path (converted on the host, rounded to float32 here), so the
+// node IDs do not depend on the element type the caller hands over; below 2^53 it is also the single
+// rounding of scikit-learn's own cast.
+template <typename TX>
+__device__ __forceinline__ float walk_value(TX v) {
+    if constexpr (std::is_floating_point<TX>::value)
+        return (float)v;
+    else
+        return (float)x_to_f64(v);
+}
 
 template <typename TX>
 __global__ void __launch_bounds__(FOREST_THREADS)
@@ -39,7 +54,7 @@ forest_apply_kernel(const TX *__restrict__ X, long long ldx, long long n_q, int 
     const int rows = (int)min((long long)FOREST_THREADS, n_q - q0);
     for (int e = threadIdx.x; e < FOREST_THREADS * d; e += FOREST_THREADS) {
         const int r = e / d, c = e - r * d;
-        xs[r * xs_ld + c] = r < rows ? (float)X[(q0 + r) * ldx + c] : 0.0f;  // round to float32 like DTYPE
+        xs[r * xs_ld + c] = r < rows ? walk_value(X[(q0 + r) * ldx + c]) : 0.0f;  // round to float32 like DTYPE
     }
     __syncthreads();
     const float *xr = xs + threadIdx.x * xs_ld;
@@ -94,26 +109,22 @@ size_t forest_smem_bytes(int d) {
     return ((size_t)FOREST_THREADS * (d | 1) + (size_t)FOREST_THREADS * (FOREST_TG + 1)) * 4;
 }
 
-cudaError_t launch_forest_apply(const void *X, int x_is_f32, long long ldx, long long n_q, int d,
+cudaError_t launch_forest_apply(const void *X, int x_dtype, long long ldx, long long n_q, int d,
                                 const ForestNode *nodes, const int *roots, int n_trees,
                                 uint16_t *out_codes, int *out_ids, long long ld_out, cudaStream_t st) {
     if (n_q <= 0) return cudaSuccess;
     const size_t smem = forest_smem_bytes(d);
     if (smem > 227 * 1024) return cudaErrorInvalidValue;
     const long long grid = (n_q + FOREST_THREADS - 1) / FOREST_THREADS;
-    cudaError_t e;
-    if (x_is_f32) {
-        e = cudaFuncSetAttribute(forest_apply_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    return with_x_type(x_dtype, [&](auto zero) {
+        using TX = decltype(zero);
+        cudaError_t e = cudaFuncSetAttribute(forest_apply_kernel<TX>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             227 * 1024);
         if (e != cudaSuccess) return e;
-        forest_apply_kernel<float><<<(unsigned)grid, FOREST_THREADS, smem, st>>>(
-            (const float *)X, ldx, n_q, d, nodes, roots, n_trees, out_codes, out_ids, ld_out);
-    } else {
-        e = cudaFuncSetAttribute(forest_apply_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        if (e != cudaSuccess) return e;
-        forest_apply_kernel<double><<<(unsigned)grid, FOREST_THREADS, smem, st>>>(
-            (const double *)X, ldx, n_q, d, nodes, roots, n_trees, out_codes, out_ids, ld_out);
-    }
-    return cudaGetLastError();
+        forest_apply_kernel<TX><<<(unsigned)grid, FOREST_THREADS, smem, st>>>(
+            (const TX *)X, ldx, n_q, d, nodes, roots, n_trees, out_codes, out_ids, ld_out);
+        return cudaGetLastError();
+    });
 }
 
 }  // namespace sk

@@ -10,6 +10,34 @@ namespace sk {
 
 struct FinishParams;
 
+// ---- element types of a query matrix / raster block: the x_dtype codes of include/sknnr_b200.h
+// (SKNNR_F64 0, SKNNR_F32 1, SKNNR_U8 2, SKNNR_I16 3, SKNNR_U16 4, SKNNR_I32 5, SKNNR_I64 6) ------
+// Bytes per element; 0 for an unknown code.
+inline size_t x_dtype_size(int x_dtype) {
+    switch (x_dtype) {
+        case 0: case 6: return 8;
+        case 1: case 5: return 4;
+        case 3: case 4: return 2;
+        case 2: return 1;
+        default: return 0;
+    }
+}
+// f(TX{}) with TX the element type of x_dtype (the kernel instantiation a launcher picks);
+// cudaErrorInvalidValue for an unknown code
+template <class F>
+cudaError_t with_x_type(int x_dtype, F &&f) {
+    switch (x_dtype) {
+        case 0: return f(double{});
+        case 1: return f(float{});
+        case 2: return f(uint8_t{});
+        case 3: return f(int16_t{});
+        case 4: return f(uint16_t{});
+        case 5: return f(int32_t{});
+        case 6: return f(0LL);
+        default: return cudaErrorInvalidValue;
+    }
+}
+
 // ---- project.cu: Z = ((X - center) / scale) @ proj  (S2, a1-a4) -----------------------
 // Writes Z as float64 rows (exact re-rank operand) and as the search kernel's query tile
 // image [n_qtiles][dpad][256] f32 = -2 * (Z - mu).
@@ -19,7 +47,7 @@ struct FinishParams;
 // either engine - 256, 384, 512 - divides it).  n_rows_dev != null makes
 // the launch "compacted": only the first *n_rows_dev rows exist (device-side count).
 inline long long padded_rows(long long n) { return (n + 1535) / 1536 * 1536; }
-cudaError_t launch_project(const void *X, int x_is_f32, long long ldx, long long n_q, int d_in,
+cudaError_t launch_project(const void *X, int x_dtype, long long ldx, long long n_q, int d_in,
                            int d_out, int dpad, const double *center, const double *scale,
                            const double *proj, const double *mu, double *z64, float *qimg,
                            __half *qimg_tc, int tc_kc, double tc_sigma, const int *n_rows_dev,
@@ -167,17 +195,17 @@ struct __align__(16) ForestNode {
 size_t forest_smem_bytes(int d);
 // out_ids != null: node IDs relative to each tree's root (transform parity, int32 [n_q, ld_out]);
 // else out_codes: 16-bit node codes [n_q, ld_out]
-cudaError_t launch_forest_apply(const void *X, int x_is_f32, long long ldx, long long n_q, int d,
+cudaError_t launch_forest_apply(const void *X, int x_dtype, long long ldx, long long n_q, int d,
                                 const ForestNode *nodes, const int *roots, int n_trees,
                                 uint16_t *out_codes, int *out_ids, long long ld_out, cudaStream_t st);
 
 // ---- raster.cu (band-major raster blocks in, band-major result layers out) ------------------
 constexpr int RASTER_GROUP = 1024;   // pixels per CTA of the mask / gather kernels
 // pos [rows] <- valid flags, counts [groups + 1] <- exclusive group offsets (+ total), *total_out <- total
-cudaError_t launch_raster_mask(const void *bands, int x_is_f32, long long rows, int d, int use_nodata,
+cudaError_t launch_raster_mask(const void *bands, int x_dtype, long long rows, int d, int use_nodata,
                                double nodata, int *pos, int *counts, int *total_out, cudaStream_t st);
 // pos <- compacted row (or -1); xc [n_valid, d] <- the valid pixels' feature rows, pixel order kept
-cudaError_t launch_raster_gather(const void *bands, int x_is_f32, long long rows, int d, const int *offs,
+cudaError_t launch_raster_gather(const void *bands, int x_dtype, long long rows, int d, const int *offs,
                                  int *pos, void *xc, cudaStream_t st);
 cudaError_t launch_raster_scatter_f64(const int *pos, long long rows, const double *src, int width,
                                       double fill, double *out, long long ld_out, cudaStream_t st);

@@ -6,11 +6,14 @@
 //   CCorATransformer        ref:src/sknnr/transformers/_ccora_transformer.py:70
 //   CCATransformer          ref:src/sknnr/transformers/_cca_transformer.py:87
 // computed in float64 exactly as written (true division, centre first).  Raw map pixels are
-// read from HBM once; the kernel emits both operands the rest of the path needs:
+// read from HBM once, in the caller's element type (float64, float32 or an integer type, each
+// value converted to float64 on load); the kernel emits both operands the rest of the path needs:
 //   z64  [n_q, d_out] float64          - exact re-rank operand
 //   qimg [n_qtiles][dpad][256] float32 - search-kernel query tile image, -2 * (Z - mu)
 #include "common.cuh"
 #include "kernels.h"
+
+#include <type_traits>
 
 namespace sk {
 
@@ -58,7 +61,7 @@ project_kernel(const TX *__restrict__ X, long long ldx, long long n_q, int d_in,
                 rr[u] = r;
                 cc[u] = c;
                 const bool have = e0 + u < d_in && r < rows;
-                v[u] = have ? (double)X[(q0 + r) * ldx + c] : 0.0;
+                v[u] = have ? x_to_f64(X[(q0 + r) * ldx + c]) : 0.0;
                 r += dr;
                 c += dc;
                 if (c >= d_in) {
@@ -72,7 +75,9 @@ project_kernel(const TX *__restrict__ X, long long ldx, long long n_q, int d_in,
                 double w = v[u];
                 if (rr[u] < rows) {
                     // NaN / inf anywhere in the query block: the caller raises scikit-learn's ValueError
-                    if (nonfinite && !isfinite(w)) *nonfinite = 1;
+                    // (an integer matrix holds neither)
+                    if constexpr (std::is_floating_point<TX>::value)
+                        if (nonfinite && !isfinite(w)) *nonfinite = 1;
                     if (center) w -= center[cc[u]];
                     if (scale) w /= scale[cc[u]];
                     if (z_here) z64[(q0 + rr[u]) * d_out + cc[u]] = w;
@@ -94,8 +99,9 @@ project_kernel(const TX *__restrict__ X, long long ldx, long long n_q, int d_in,
         if (xs_in_smem) return xr[i];
         double v = 0.0;
         if (r < rows) {
-            v = (double)X[(q0 + r) * ldx + i];
-            if (nonfinite && !isfinite(v)) *nonfinite = 1;
+            v = x_to_f64(X[(q0 + r) * ldx + i]);
+            if constexpr (std::is_floating_point<TX>::value)
+                if (nonfinite && !isfinite(v)) *nonfinite = 1;
             if (center) v -= center[i];
             if (scale) v /= scale[i];
         }
@@ -162,7 +168,7 @@ project_kernel(const TX *__restrict__ X, long long ldx, long long n_q, int d_in,
     }
 }
 
-cudaError_t launch_project(const void *X, int x_is_f32, long long ldx, long long n_q, int d_in,
+cudaError_t launch_project(const void *X, int x_dtype, long long ldx, long long n_q, int d_in,
                            int d_out, int dpad, const double *center, const double *scale,
                            const double *proj, const double *mu, double *z64, float *qimg,
                            __half *qimg_tc, int tc_kc, double tc_sigma, const int *n_rows_dev,
@@ -179,23 +185,16 @@ cudaError_t launch_project(const void *X, int x_is_f32, long long ldx, long long
     // CTA tile size of the search engines divides padded_rows, a multiple of PROJ_THREADS)
     const long long padded = padded_rows(n_q);
     const long long grid = (padded + PROJ_THREADS - 1) / PROJ_THREADS;
-    cudaError_t e;
-    if (x_is_f32) {
-        e = cudaFuncSetAttribute(project_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 227 * 1024);
+    return with_x_type(x_dtype, [&](auto zero) {
+        using TX = decltype(zero);
+        cudaError_t e = cudaFuncSetAttribute(project_kernel<TX>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             227 * 1024);
         if (e != cudaSuccess) return e;
-        project_kernel<float><<<(unsigned)grid, PROJ_THREADS, smem, st>>>(
-            (const float *)X, ldx, n_q, d_in, d_out, dpad, center, scale, proj, mu, z64, qimg, qimg_tc,
+        project_kernel<TX><<<(unsigned)grid, PROJ_THREADS, smem, st>>>(
+            (const TX *)X, ldx, n_q, d_in, d_out, dpad, center, scale, proj, mu, z64, qimg, qimg_tc,
             tc_kc, tc_sigma, n_rows_dev, nonfinite, xs_in_smem, ps_in_smem);
-    } else {
-        e = cudaFuncSetAttribute(project_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 227 * 1024);
-        if (e != cudaSuccess) return e;
-        project_kernel<double><<<(unsigned)grid, PROJ_THREADS, smem, st>>>(
-            (const double *)X, ldx, n_q, d_in, d_out, dpad, center, scale, proj, mu, z64, qimg, qimg_tc,
-            tc_kc, tc_sigma, n_rows_dev, nonfinite, xs_in_smem, ps_in_smem);
-    }
-    return cudaGetLastError();
+        return cudaGetLastError();
+    });
 }
 
 }  // namespace sk

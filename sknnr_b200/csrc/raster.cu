@@ -11,9 +11,13 @@
 //   raster_gather_kernel  stable compaction + transpose: Xc[pos[p]][b] = band[b][p]
 //   (the usual chunk pipeline runs on Xc)
 //   raster_scatter_kernel band-major result layers, `fill` where the pixel was masked
-// All four are HBM-bound streaming kernels (8d bytes in, 8d out per pixel at f64).
+// All four are HBM-bound streaming kernels (8d bytes in, 8d out per pixel at f64).  The mask and
+// the gather read the bands in the caller's element type (float64, float32 or an integer type), and
+// the gather keeps it: the projection converts the compacted rows to float64 as it loads them.
 #include "common.cuh"
 #include "kernels.h"
+
+#include <type_traits>
 
 namespace sk {
 
@@ -31,9 +35,13 @@ raster_mask_kernel(const T *__restrict__ bands, long long rows, int d, int use_n
         bool ok = p < rows;
         if (ok) {
             for (int b = 0; b < d; ++b) {
-                const double v = (double)bands[(long long)b * rows + p];
-                // isfinite on the value the search will see; nodata compares in the input's type
-                ok = ok && isfinite(v) && !(use_nodata && v == nodata);
+                const double v = x_to_f64(bands[(long long)b * rows + p]);
+                // isfinite on the value the search will see; nodata compares in float64 (the caller
+                // rounds it to a float band's own type first; an integer band is never NaN / inf)
+                if constexpr (std::is_floating_point<T>::value)
+                    ok = ok && isfinite(v) && !(use_nodata && v == nodata);
+                else
+                    ok = ok && !(use_nodata && v == nodata);
             }
             pos[p] = ok ? 1 : 0;
         }
@@ -136,27 +144,29 @@ raster_scatter_kernel(const int *__restrict__ pos, long long rows, const T *__re
     for (int j = 0; j < width; ++j) out[(long long)j * ld_out + p] = r >= 0 ? src[(long long)r * width + j] : fill;
 }
 
-cudaError_t launch_raster_mask(const void *bands, int x_is_f32, long long rows, int d, int use_nodata,
+cudaError_t launch_raster_mask(const void *bands, int x_dtype, long long rows, int d, int use_nodata,
                                double nodata, int *pos, int *counts, int *total_out, cudaStream_t st) {
     if (rows <= 0) return cudaSuccess;
     const int groups = (int)((rows + RASTER_GROUP - 1) / RASTER_GROUP);
-    if (x_is_f32)
-        raster_mask_kernel<float><<<groups, RASTER_THREADS, 0, st>>>((const float *)bands, rows, d, use_nodata, nodata, pos, counts);
-    else
-        raster_mask_kernel<double><<<groups, RASTER_THREADS, 0, st>>>((const double *)bands, rows, d, use_nodata, nodata, pos, counts);
+    cudaError_t e = with_x_type(x_dtype, [&](auto zero) {
+        using T = decltype(zero);
+        raster_mask_kernel<T><<<groups, RASTER_THREADS, 0, st>>>((const T *)bands, rows, d, use_nodata, nodata, pos, counts);
+        return cudaGetLastError();
+    });
+    if (e != cudaSuccess) return e;
     raster_scan_kernel<<<1, 1024, 0, st>>>(counts, groups, total_out);
     return cudaGetLastError();
 }
 
-cudaError_t launch_raster_gather(const void *bands, int x_is_f32, long long rows, int d, const int *offs,
+cudaError_t launch_raster_gather(const void *bands, int x_dtype, long long rows, int d, const int *offs,
                                  int *pos, void *xc, cudaStream_t st) {
     if (rows <= 0) return cudaSuccess;
     const int groups = (int)((rows + RASTER_GROUP - 1) / RASTER_GROUP);
-    if (x_is_f32)
-        raster_gather_kernel<float><<<groups, RASTER_THREADS, 0, st>>>((const float *)bands, rows, d, offs, pos, (float *)xc);
-    else
-        raster_gather_kernel<double><<<groups, RASTER_THREADS, 0, st>>>((const double *)bands, rows, d, offs, pos, (double *)xc);
-    return cudaGetLastError();
+    return with_x_type(x_dtype, [&](auto zero) {
+        using T = decltype(zero);
+        raster_gather_kernel<T><<<groups, RASTER_THREADS, 0, st>>>((const T *)bands, rows, d, offs, pos, (T *)xc);
+        return cudaGetLastError();
+    });
 }
 
 cudaError_t launch_raster_scatter_f64(const int *pos, long long rows, const double *src, int width,

@@ -3,8 +3,9 @@ image - the loop a "sknnr-spatial"-style caller writes around ``est.kneighbors``
 (ref:src/sknnr/_base.py:285-352): flatten ``[bands, H, W]`` to ``[H*W, bands]``, drop the pixels
 with missing data, query, and put the results back as ``[k, H, W]`` / ``[n_targets, H, W]`` layers.
 
-Here the image goes to the device as it is; transpose, mask, compaction and the scatter back run
-there, next to the search (``sknnr_raster_kneighbors``), pipelined block by block.  The unmasked
+Here the image goes to the device as it is (float64, float32, or uint8 / int16 / uint16 / int32 /
+int64 without a float copy); transpose, mask, compaction and the scatter back run there, next to the
+search (``sknnr_raster_kneighbors``), pipelined block by block.  The unmasked
 pixels, in row-major pixel order, are numbered like the rows of one ``kneighbors(X[valid])`` call.
 """
 
@@ -12,6 +13,8 @@ from __future__ import annotations
 
 import numpy as np
 from sklearn.utils.validation import check_is_fitted
+
+from . import _lib as L
 
 __all__ = ["kneighbors_raster", "predict_raster"]
 
@@ -24,7 +27,7 @@ def _regressor_and_image(est, image):
     image = np.asarray(image)
     if image.ndim != 3:
         raise ValueError(f"expected an image of shape [bands, height, width], got {image.shape}")
-    if image.dtype != np.float32:
+    if L.x_dtype_code(image) is None:   # (uint8 / int16 / uint16 / int32 / int64 bands go as they are)
         image = np.asarray(image, dtype=np.float64)
     # (a transformed estimator's own n_features_in_ counts the transformed axes, as in the reference)
     n_bands = est.transformer_.n_features_in_ if hasattr(est, "transformer_") else reg.n_features_in_

@@ -8,6 +8,11 @@ from sklearn.preprocessing import StandardScaler
 from sklearn.utils.validation import FLOAT_DTYPES, check_is_fitted, validate_data
 
 from .. import _cache
+from .._lib import NATIVE_INT_DTYPES
+
+# dtypes a query keeps through validation: the floats scikit-learn keeps, plus the integer types the
+# device reads as they are (any other dtype becomes float64, the first entry, as before)
+QUERY_DTYPES = FLOAT_DTYPES + NATIVE_INT_DTYPES
 
 
 class DeviceProjectionMixin:
@@ -58,7 +63,7 @@ class StandardScalerWithDOF(DeviceProjectionMixin, StandardScaler):
     def _validate_query(self, X, finite=True):
         check_is_fitted(self)
         return validate_data(
-            self, X, reset=False, accept_sparse=False, copy=False, dtype=FLOAT_DTYPES,
+            self, X, reset=False, accept_sparse=False, copy=False, dtype=QUERY_DTYPES,
             force_writeable=False, ensure_all_finite="allow-nan" if finite else False,
         )
 

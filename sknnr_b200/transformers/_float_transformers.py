@@ -6,7 +6,7 @@ import numpy as np
 from sklearn.base import BaseEstimator, OneToOneFeatureMixin, TransformerMixin
 from sklearn.utils.validation import FLOAT_DTYPES, check_is_fitted, validate_data
 
-from ._base import ComponentReducerMixin, DeviceProjectionMixin, StandardScalerWithDOF
+from ._base import QUERY_DTYPES, ComponentReducerMixin, DeviceProjectionMixin, StandardScalerWithDOF
 from ._ordination import fit_cca, fit_ccora
 
 
@@ -48,8 +48,9 @@ class CCATransformer(DeviceProjectionMixin, ComponentReducerMixin, TransformerMi
     (mirrors ref:src/sknnr/transformers/_cca_transformer.py:21-97)."""
 
     def _checked(self, X, reset, finite=True):
-        return validate_data(self, X=X, reset=reset, dtype=FLOAT_DTYPES, ensure_all_finite=finite,
-                             ensure_min_features=2, ensure_min_samples=1)
+        # (a query keeps its integer dtype for the device; fit works in floats)
+        return validate_data(self, X=X, reset=reset, dtype=FLOAT_DTYPES if reset else QUERY_DTYPES,
+                             ensure_all_finite=finite, ensure_min_features=2, ensure_min_samples=1)
 
     def fit(self, X, y):
         self._drop_device_state()

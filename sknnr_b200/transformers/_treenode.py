@@ -16,6 +16,7 @@ from sklearn.base import BaseEstimator, TransformerMixin
 from sklearn.utils.validation import check_array, check_is_fitted, validate_data
 
 from .. import _cache
+from .._lib import x_dtype_code
 
 
 def _is_nan_like(v) -> bool:
@@ -156,6 +157,8 @@ class TreeNodeTransformer(TransformerMixin, BaseEstimator, ABC):
         float32 check of ``est.apply`` ($SP/sklearn/tree/_classes.py _validate_X_predict)."""
         check_is_fitted(self)
         X_arr = validate_data(self, X=X, reset=False, ensure_min_features=1, ensure_min_samples=1)
+        if X_arr.dtype.kind in "iu" and x_dtype_code(X_arr) is not None:
+            return X_arr   # uint8 ... int64: no NaN / inf to find, the device reads the array as it is
         with np.errstate(over="ignore"):
             X32 = np.asarray(X_arr, dtype=np.float32)
         check_array(X32, ensure_all_finite=True, estimator=self)
