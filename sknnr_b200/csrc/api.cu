@@ -14,6 +14,7 @@
 #include <deque>
 #include <functional>
 #include <mutex>
+#include <optional>
 #include <string>
 #include <thread>
 #include <chrono>
@@ -194,6 +195,12 @@ template <typename T>
 struct PinBuf {
     T *p = nullptr;
     size_t cap = 0;  // elements
+    PinBuf() = default;
+    PinBuf(const PinBuf &) = delete;
+    PinBuf &operator=(const PinBuf &) = delete;
+    ~PinBuf() {
+        if (p) cudaFreeHost(p);
+    }
     cudaError_t reserve(size_t n) {
         if (n <= cap) return cudaSuccess;
         if (p) cudaFreeHost(p);
@@ -202,11 +209,6 @@ struct PinBuf {
         cudaError_t e = cudaHostAlloc((void **)&p, n * sizeof(T), cudaHostAllocDefault);
         if (e == cudaSuccess) cap = n;
         return e;
-    }
-    void release() {
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
     }
 };
 
@@ -224,6 +226,12 @@ template <typename T>
 struct DevBuf {
     T *p = nullptr;
     size_t cap = 0;  // elements
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() {
+        if (p) cudaFree(p);
+    }
     cudaError_t reserve(size_t n) {
         if (n <= cap) return cudaSuccess;
         if (p) cudaFree(p);
@@ -233,12 +241,23 @@ struct DevBuf {
         if (e == cudaSuccess) cap = n;
         return e;
     }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
 };
+
+// cudaMalloc + copy of n elements of fitted state
+template <typename T>
+cudaError_t upload(T **dst, const T *src, size_t n) {
+    cudaError_t e = cudaMalloc(dst, n * sizeof(T));
+    if (e != cudaSuccess) return e;
+    return cudaMemcpy(*dst, src, n * sizeof(T), cudaMemcpyHostToDevice);
+}
+
+int check_device(int dev) {
+    int count = 0;
+    if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0)
+        return fail(SKNNR_ENODEV, "no CUDA device: sknnr_b200 has no CPU fallback");
+    if (dev < 0 || dev >= count) return fail(SKNNR_EINVAL, "bad device ordinal");
+    return SKNNR_OK;
+}
 
 // per-chunk device buffers + the stream the chunk runs on
 struct Slot {
@@ -257,7 +276,6 @@ struct Slot {
     DevBuf<int> fbm;               // failures of the tensor engine's second pass (stage 1b), same layout
     DevBuf<float> fb_thr;          // second-pass thresholds of the first-stage failures (order of fb's list)
     DevBuf<uint16_t> codes;        // node codes produced by the device forest walk
-    DevBuf<int> ids32;             // node IDs of sknnr_forest_apply
     DevBuf<uint32_t> qimg_h;       // Hamming query image
     DevBuf<int> cand_idx;
     DevBuf<float> cand_thr;
@@ -291,33 +309,15 @@ struct Slot {
     PinBuf<unsigned char> h_x, h_dist, h_idx, h_pred;
     struct CopyOut { void *dst; const void *src; size_t bytes; };
     std::vector<CopyOut> owed;
-    void release() {
-        x.release(); z64.release(); qimg.release(); qimg_tc.release(); z64c.release(); fb2.release(); fbm.release(); fb_thr.release();
-        codes.release(); ids32.release(); qimg_h.release(); cand_idx.release();
-        cand_thr.release(); cand_cnt.release(); fb.release(); o_dist.release();
-        o_idx.release(); o_pred.release();
-        xc.release(); r_pos.release(); r_cnt.release(); r_dist.release(); r_pred.release(); r_idx.release();
-        if (h_cnt) cudaFreeHost(h_cnt);
-        if (ev_cnt) cudaEventDestroy(ev_cnt);
-        h_cnt = nullptr; ev_cnt = nullptr;
-        for (auto e : evs) cudaEventDestroy(e);
-        evs.clear();
-        ev_used = 0;
-        if (h_fb) cudaFreeHost(h_fb);
-        nonfinite.release();
-        h_x.release(); h_dist.release(); h_idx.release(); h_pred.release();
-        owed.clear();
-        if (ev_last) cudaEventDestroy(ev_last);
-        ev_last = nullptr; last_pending = false; flag_pending = false;
-        if (ev_in) cudaEventDestroy(ev_in);
-        if (ev_out) cudaEventDestroy(ev_out);
-        ev_in = ev_out = nullptr;
-        if (stream) cudaStreamDestroy(stream);
-        if (tail_stream) cudaStreamDestroy(tail_stream);
-        if (ev_stage1) cudaEventDestroy(ev_stage1);
-        if (ev_tail) cudaEventDestroy(ev_tail);
-        tail_stream = nullptr; ev_stage1 = ev_tail = nullptr; tail_pending = false;
-        h_fb = nullptr; stream = nullptr;
+    // (the buffers free themselves after this body; the DevBuf members also make a Slot uncopyable)
+    ~Slot() {
+        for (cudaStream_t st : {stream, tail_stream})
+            if (st) cudaStreamDestroy(st);
+        for (cudaEvent_t e : {ev_stage1, ev_tail, ev_cnt, ev_last, ev_in, ev_out})
+            if (e) cudaEventDestroy(e);
+        for (cudaEvent_t e : evs) cudaEventDestroy(e);
+        for (int *h : {h_cnt, h_fb})
+            if (h) cudaFreeHost(h);
     }
     // record a timing event on `st` (pairs: even = start, odd = stop)
     cudaError_t mark(cudaStream_t st) {
@@ -359,10 +359,8 @@ struct IndexBase {
     cudaStream_t h2d_stream = nullptr, d2h_stream = nullptr, host_compute = nullptr;
 
     int init_common(int dev, const double *y, int64_t nref, int nout) {
-        int count = 0;
-        if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0)
-            return fail(SKNNR_ENODEV, "no CUDA device: sknnr_b200 has no CPU fallback");
-        if (dev < 0 || dev >= count) return fail(SKNNR_EINVAL, "bad device ordinal");
+        const int rc = check_device(dev);
+        if (rc != SKNNR_OK) return rc;
         device = dev;
         n_ref = nref;
         n_out = nout;
@@ -372,10 +370,7 @@ struct IndexBase {
         if (prop.major < 10)
             return fail(SKNNR_ENODEV, "sknnr_b200 kernels are built for sm_100a (B200) only");
         n_sm = prop.multiProcessorCount;
-        if (y && nout > 0) {
-            CK(cudaMalloc(&d_y, (size_t)nref * nout * sizeof(double)));
-            CK(cudaMemcpy(d_y, y, (size_t)nref * nout * sizeof(double), cudaMemcpyHostToDevice));
-        }
+        if (y && nout > 0) CK(upload(&d_y, y, (size_t)nref * nout));
         int prio_lo = 0, prio_hi = 0;
         CK(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
         CK(cudaStreamCreateWithFlags(&host_compute, cudaStreamNonBlocking));
@@ -399,18 +394,33 @@ struct IndexBase {
         }
         return SKNNR_OK;
     }
+    // frees what the index holds outside its slots and buffers, and makes its device current: the
+    // slots and buffers free themselves when the index is deleted, which follows at once
     void release_common() {
         cudaSetDevice(device);
-        for (auto &s : slots) s.release();
-        for (cudaStream_t *st : {&host_compute, &h2d_stream, &d2h_stream}) {
-            if (*st) cudaStreamDestroy(*st);
-            *st = nullptr;
-        }
-        exact_scr.release(); exact_big.release();
+        for (cudaStream_t st : {host_compute, h2d_stream, d2h_stream})
+            if (st) cudaStreamDestroy(st);
         if (ev_exact) cudaEventDestroy(ev_exact);
-        ev_exact = nullptr;
         if (d_y) cudaFree(d_y);
-        d_y = nullptr;
+    }
+    // Readies the index for a call (lock held, device current).  A synchronous call waits until every
+    // slot is free; a device-pointer call instead makes the caller's stream wait for whatever an earlier
+    // call (possibly a device-pointer call on another stream) left running on the first `dev_slots`
+    // slots, the ones it uses.  The call's counters then start from zero.
+    cudaError_t begin_call(bool dev_ptrs, cudaStream_t user, int dev_slots) {
+        for (int i = 0; i < kSlots; ++i) {
+            Slot &s = slots[i];
+            cudaError_t e = cudaSuccess;
+            if (!dev_ptrs) e = finish_slot(s);
+            else if (i < dev_slots && s.last_pending) e = cudaStreamWaitEvent(user, s.ev_last, 0);
+            if (e != cudaSuccess) return e;
+        }
+        for (auto &s : slots) { s.ev_used = 0; s.fb_pending = false; s.flag_pending = false; }
+        stats = sknnr_stats{};
+        n_simt_rows = n_exact_rows = 0;
+        chunk_rows_seen = chunk_fb_seen = chunk_fail_seen = 0;   // the demotion rule looks at this call's chunks only
+        saw_nonfinite = false;
+        return cudaSuccess;
     }
     // collect timing / fallback count of the chunk that last ran on this slot
     void harvest(Slot &s) {
@@ -508,14 +518,57 @@ struct IndexBase {
     }
 };
 
-// a device-pointer call lends the caller's stream to a slot for one chunk; the slot's own stream
-// comes back whatever way the scope is left
+// device buffers that take a chunk's results (null: not requested)
+struct ChunkOut {
+    double *dist = nullptr;
+    long long *idx = nullptr;
+    double *pred = nullptr;
+};
+
+// what the finishing kernels of one chunk need: its first row is row row0 of the query (row_offset
+// included), its results go to `o`
+FinishParams finish_params(const IndexBase *ix, int k, uint32_t flags, int decimals, int weights, int64_t row0,
+                           const ChunkOut &o) {
+    FinishParams fp{};
+    fp.k = k;
+    fp.exclude_self = (flags & SKNNR_EXCLUDE_SELF) ? 1 : 0;
+    fp.deterministic = (flags & SKNNR_DETERMINISTIC) ? 1 : 0;
+    fp.round_scale = std::pow(10.0, (double)decimals);
+    fp.row_offset = row0;
+    fp.out_dist = o.dist;
+    fp.out_idx = o.idx;
+    fp.weights = weights;
+    fp.y = ix->d_y;
+    fp.n_ref = (int)ix->n_ref;
+    fp.row_map = nullptr;
+    fp.n_out = ix->n_out;
+    fp.out_pred = o.pred;
+    return fp;
+}
+
+// A device-pointer call writes straight into the caller's arrays from row r0 on; any other call into
+// the slot's buffers, reserved here for `rows` rows.
+int chunk_outputs(const IndexBase *ix, Slot &s, bool dev_ptrs, int64_t r0, int64_t rows, int k, int weights,
+                  double *out_dist, int64_t *out_idx, double *out_pred, ChunkOut &o) {
+    o = ChunkOut{};
+    if (dev_ptrs) {
+        if (out_dist) o.dist = out_dist + r0 * k;
+        if (out_idx) o.idx = (long long *)out_idx + r0 * k;
+        if (weights != SKNNR_W_NONE) o.pred = out_pred + r0 * ix->n_out;
+        return SKNNR_OK;
+    }
+    if (out_dist) { CK(s.o_dist.reserve((size_t)rows * k)); o.dist = s.o_dist.p; }
+    if (out_idx) { CK(s.o_idx.reserve((size_t)rows * k)); o.idx = s.o_idx.p; }
+    if (weights != SKNNR_W_NONE) { CK(s.o_pred.reserve((size_t)rows * ix->n_out)); o.pred = s.o_pred.p; }
+    return SKNNR_OK;
+}
+
+// a call lends a stream (the caller's, or the host pipeline's compute stream) to a slot; the slot's
+// own stream comes back whatever way the scope is left
 struct StreamLoan {
     Slot &s;
     cudaStream_t saved;
-    StreamLoan(Slot &slot, cudaStream_t st, bool lend) : s(slot), saved(slot.stream) {
-        if (lend) s.stream = st;
-    }
+    StreamLoan(Slot &slot, cudaStream_t st) : s(slot), saved(slot.stream) { s.stream = st; }
     ~StreamLoan() { s.stream = saved; }
 };
 // leaves the handle quiescent when a call fails half way through its chunks
@@ -589,6 +642,12 @@ struct sknnr_index : IndexBase {
     // chunks of host-buffer calls with that layout only.
     bool tensor_demoted[3] = {false, false, false};
     int ns_in_use = 2;
+    // adaptive engine choice, applied before each chunk a host-buffer or raster call issues: if the FP16
+    // filter cannot certify > 5 % of the rows (ill-conditioned features: huge norms relative to neighbour
+    // distances) the FP32 engine is the better first stage for this index
+    void apply_demotion() {
+        if (chunk_rows_seen >= 4096 && chunk_fb_seen * 3 > chunk_rows_seen) tensor_demoted[ns_in_use] = true;
+    }
 };
 
 struct sknnr_hamming_index : IndexBase {
@@ -615,6 +674,12 @@ struct sknnr_forest {
     DevBuf<unsigned char> x;
     DevBuf<int> ids;
 };
+
+static int check_forest(const sknnr_hamming_index *ix, const sknnr_forest *f) {
+    if (f->n_trees != ix->n_trees) return fail(SKNNR_EINVAL, "forest and index disagree on the number of trees");
+    if (f->device != ix->device) return fail(SKNNR_EINVAL, "forest and index live on different devices");
+    return SKNNR_OK;
+}
 
 extern "C" {
 
@@ -808,19 +873,12 @@ int sknnr_index_create_metric(const double *fit_z, int64_t n_ref, int32_t d_out,
     ix->r2max = r2max;
     if (lp) ix->simt_ok = r2max < kLpNormLimit;   // (false for NaN as well)
 
-    auto up = [&](double **dst, const double *src, size_t n) -> cudaError_t {
-        cudaError_t e = cudaMalloc(dst, n * sizeof(double));
-        if (e != cudaSuccess) return e;
-        return cudaMemcpy(*dst, src, n * sizeof(double), cudaMemcpyHostToDevice);
-    };
-    cudaError_t e = up(&ix->d_ref64, fit_z, (size_t)n_ref * d_out);
-    if (e == cudaSuccess) e = up(&ix->d_mu, mu.data(), d_out);
-    if (e == cudaSuccess && center) e = up(&ix->d_center, center, d_in);
-    if (e == cudaSuccess && scale) e = up(&ix->d_scale, scale, d_in);
-    if (e == cudaSuccess && proj) e = up(&ix->d_proj, proj, (size_t)d_in * d_out);
-    if (e == cudaSuccess) e = cudaMalloc(&ix->d_rimg, rimg.size() * sizeof(float));
-    if (e == cudaSuccess)
-        e = cudaMemcpy(ix->d_rimg, rimg.data(), rimg.size() * sizeof(float), cudaMemcpyHostToDevice);
+    cudaError_t e = upload(&ix->d_ref64, fit_z, (size_t)n_ref * d_out);
+    if (e == cudaSuccess) e = upload(&ix->d_mu, mu.data(), d_out);
+    if (e == cudaSuccess && center) e = upload(&ix->d_center, center, d_in);
+    if (e == cudaSuccess && scale) e = upload(&ix->d_scale, scale, d_in);
+    if (e == cudaSuccess && proj) e = upload(&ix->d_proj, proj, (size_t)d_in * d_out);
+    if (e == cudaSuccess) e = upload(&ix->d_rimg, rimg.data(), rimg.size());
 
     // tensor-core engine image: tiles of 128 plots, [chunk][row][8] FP16 (round to nearest even) of
     // sigma * (r - mu), K = d' + 3 padded to a multiple of 16: elements d' .. d'+2 hold a 3-way FP16
@@ -868,9 +926,7 @@ int sknnr_index_create_metric(const double *fit_z, int64_t n_ref, int32_t d_out,
                 at(d_out + 2, jj) = __float2half_rn((float)lo);
             }
         }
-        e = cudaMalloc(&ix->d_rimg_tc, timg.size() * sizeof(__half));
-        if (e == cudaSuccess)
-            e = cudaMemcpy(ix->d_rimg_tc, timg.data(), timg.size() * sizeof(__half), cudaMemcpyHostToDevice);
+        e = upload(&ix->d_rimg_tc, timg.data(), timg.size());
     }
     if (e != cudaSuccess) {
         sknnr_index_destroy(ix);
@@ -889,7 +945,7 @@ int sknnr_index_destroy(sknnr_index *ix) {
     return SKNNR_OK;
 }
 
-int sknnr_index_stats(sknnr_index *ix, sknnr_stats *out) {
+static int stats_common(IndexBase *ix, sknnr_stats *out) {
     if (!ix || !out) return fail(SKNNR_EINVAL, "NULL argument");
     std::lock_guard<std::mutex> g(ix->lock);
     cudaSetDevice(ix->device);
@@ -897,6 +953,8 @@ int sknnr_index_stats(sknnr_index *ix, sknnr_stats *out) {
     *out = ix->stats;
     return SKNNR_OK;
 }
+
+int sknnr_index_stats(sknnr_index *ix, sknnr_stats *out) { return stats_common(ix, out); }
 
 int sknnr_index_cascade_counts(sknnr_index *ix, int64_t *out3) {
     if (!ix || !out3) return fail(SKNNR_EINVAL, "NULL argument");
@@ -920,7 +978,7 @@ int sknnr_index_cascade_counts(sknnr_index *ix, int64_t *out3) {
 // With engine = SIMT stage 1 is skipped (L1 = all rows); with engine = EXACT only stage 3 runs.
 static int run_chunk(sknnr_index *ix, Slot &s, const void *dX, int x_dtype, int64_t ldx, bool transformed,
                      int64_t rows, int64_t row0, int k, uint32_t flags, int decimals, int weights,
-                     double *o_dist, long long *o_idx, double *o_pred, bool check_finite = false) {
+                     const ChunkOut &o, bool check_finite = false) {
     const bool excl = flags & SKNNR_EXCLUDE_SELF;
     const int kk = k + (excl ? 1 : 0);
     cudaStream_t st = s.stream;
@@ -931,30 +989,19 @@ static int run_chunk(sknnr_index *ix, Slot &s, const void *dX, int x_dtype, int6
     if (kc != 0 && g_opt.kc > kc) kc = (int)g_opt.kc;
     const bool lp = ix->metric != SKNNR_METRIC_EUCLIDEAN;   // Manhattan / Chebyshev: SIMT -> refine_lp -> exact
     const bool simt_ok = kc != 0 && search_simt_pick_stages(ix->dpad, kc) != 0 && ix->simt_ok;
-    const int ns_layout = g_opt.tc_streams == 1 ? 1 : (kk <= 7 ? 2 : 1);
-    ix->ns_in_use = ns_layout;
-    const bool tensor_ok = ix->tensor_ok && !ix->tensor_demoted[ns_layout] && kc != 0 && kc <= 16 && simt_ok;
+    // tensor engine: two candidate streams per query while k (+1) <= 7 (twice the scanner warps), else
+    // one; a stream's list keeps at most 7 (ns = 2) / 15 (ns = 1) candidates
+    const int ns = g_opt.tc_streams == 1 ? 1 : (kk <= 7 ? 2 : 1);
+    ix->ns_in_use = ns;
+    const bool tensor_fits = ix->tensor_ok && kc != 0 && kc <= 16 && simt_ok;
     int engine = (int)g_opt.engine;
-    if (engine == SKNNR_ENGINE_AUTO) engine = tensor_ok ? SKNNR_ENGINE_TENSOR : SKNNR_ENGINE_SIMT;
-    if (engine == SKNNR_ENGINE_TENSOR && !(ix->tensor_ok && kc != 0 && kc <= 16 && simt_ok))
-        engine = SKNNR_ENGINE_SIMT;
+    if (engine == SKNNR_ENGINE_AUTO)
+        engine = tensor_fits && !ix->tensor_demoted[ns] ? SKNNR_ENGINE_TENSOR : SKNNR_ENGINE_SIMT;
+    if (engine == SKNNR_ENGINE_TENSOR && !tensor_fits) engine = SKNNR_ENGINE_SIMT;
     if (engine == SKNNR_ENGINE_SIMT && !simt_ok) engine = SKNNR_ENGINE_EXACT;
     ix->stats.engine = engine;
 
-    FinishParams fp{};
-    fp.k = k;
-    fp.exclude_self = excl ? 1 : 0;
-    fp.deterministic = (flags & SKNNR_DETERMINISTIC) ? 1 : 0;
-    fp.round_scale = std::pow(10.0, (double)decimals);
-    fp.row_offset = row0;
-    fp.out_dist = o_dist;
-    fp.out_idx = o_idx;
-    fp.weights = weights;
-    fp.y = ix->d_y;
-    fp.n_ref = (int)ix->n_ref;
-    fp.row_map = nullptr;
-    fp.n_out = ix->n_out;
-    fp.out_pred = o_pred;
+    const FinishParams fp = finish_params(ix, k, flags, decimals, weights, row0, o);
 
     const bool use_tc = engine == SKNNR_ENGINE_TENSOR;
     const bool use_simt_first = engine == SKNNR_ENGINE_SIMT;
@@ -1021,9 +1068,6 @@ static int run_chunk(sknnr_index *ix, Slot &s, const void *dX, int x_dtype, int6
     const int *stage2_list = nullptr;   // chunk rows of the compacted stage-2 rows
     if (use_tc) {
         if (g_opt.timing) CK(s.mark(st));
-        // two candidate streams per query while k (+1) <= 7 (twice the scanner warps), else one
-        int ns = kk <= 7 ? 2 : 1;   // a stream's list keeps at most 7 (ns = 2) / 15 (ns = 1) candidates
-        if (g_opt.tc_streams == 1) ns = 1;
         CK(launch_search_tc(s.qimg_tc.p, ix->d_rimg_tc, ix->kc_tot, ix->n_rtiles_tc, rows, ns, ix->tc_nstage,
                             (int)g_opt.tc_seed_stride, ix->tc_wide_joint, s.cand_idx.p,
                             s.cand_thr.p, nullptr, nullptr, st));
@@ -1188,22 +1232,8 @@ int sknnr_kneighbors(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_
 
     cudaStream_t user_stream = dev_ptrs ? (cudaStream_t)stream : nullptr;
     CallGuard guard(ix, user_stream);
-    // whatever an earlier call (possibly a device-pointer call on another stream) left running on
-    // the slots this call is going to use must be complete before their scratch is reused
-    if (dev_ptrs) {
-        for (int i = 0; i < 2; ++i) {
-            Slot &s = ix->slots[i];
-            if (s.last_pending) CK(cudaStreamWaitEvent(user_stream, s.ev_last, 0));
-        }
-    } else {
-        for (auto &s : ix->slots) CK(ix->finish_slot(s));
-    }
-    for (auto &s : ix->slots) { s.ev_used = 0; s.fb_pending = false; s.flag_pending = false; }
-    ix->stats = sknnr_stats{};
-    ix->n_simt_rows = ix->n_exact_rows = 0;
+    CK(ix->begin_call(dev_ptrs, user_stream, 2));
     ix->stats.n_queries = n_q;
-    ix->saw_nonfinite = false;
-    ix->chunk_rows_seen = ix->chunk_fb_seen = ix->chunk_fail_seen = 0;   // the demotion rule looks at this call's chunks only
     if (n_q == 0) { guard.ok = true; return SKNNR_OK; }
 
     // ordinary NumPy buffers are staged through page-locked slot buffers by the host pool
@@ -1249,14 +1279,10 @@ int sknnr_kneighbors(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_
         Slot &s = ix->slots[ci % n_slots];
         if (!dev_ptrs) {
             CK(ix->finish_slot(s));   // previous chunk on this slot is done, its results delivered
-            // adaptive engine choice: if the FP16 filter cannot certify > 5 % of the rows
-            // (ill-conditioned features: huge norms relative to neighbour distances) the FP32
-            // engine is the better first stage for this index
-            if (ix->chunk_rows_seen >= 4096 && ix->chunk_fb_seen * 3 > ix->chunk_rows_seen)
-                ix->tensor_demoted[ix->ns_in_use] = true;
+            ix->apply_demotion();
         }
         // (the chunk's kernels run on the caller's stream / the pipeline's compute stream, lent to the slot)
-        StreamLoan loan(s, dev_ptrs ? user_stream : ix->host_compute, true);
+        StreamLoan loan(s, dev_ptrs ? user_stream : ix->host_compute);
         if (dev_ptrs && s.tail_pending) {   // the slot's buffers are free once its previous tail is done
             CK(cudaStreamWaitEvent(user_stream, s.ev_tail, 0));
             s.tail_pending = false;
@@ -1290,23 +1316,15 @@ int sknnr_kneighbors(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_
             dX = s.x.p;
             dld = cols;
         }
-        double *o_dist = nullptr, *o_pred = nullptr;
-        long long *o_idx = nullptr;
-        if (dev_ptrs) {
-            if (out_dist) o_dist = out_dist + r0 * k;
-            if (out_idx) o_idx = (long long *)out_idx + r0 * k;
-            if (weights != SKNNR_W_NONE) o_pred = out_pred + r0 * ix->n_out;
-        } else {
-            if (out_dist) { CK(s.o_dist.reserve((size_t)rows * k)); o_dist = s.o_dist.p; }
-            if (out_idx) { CK(s.o_idx.reserve((size_t)rows * k)); o_idx = s.o_idx.p; }
-            if (weights != SKNNR_W_NONE) { CK(s.o_pred.reserve((size_t)rows * ix->n_out)); o_pred = s.o_pred.p; }
-        }
+        ChunkOut o;
+        rc = chunk_outputs(ix, s, dev_ptrs, r0, rows, k, weights, out_dist, out_idx, out_pred, o);
+        if (rc != SKNNR_OK) return rc;
         // the last chunk's second stage has nothing to hide under: it is dealt out over all SMs; the
         // others keep to a few SMs, which costs the following chunk's tensor kernel less
         ix->spread_tail = r0 + rows >= n_q;
         CK(trace_mark(1, cin));
         rc = run_chunk(ix, s, dX, x_dtype, dld, transformed, rows, row_offset + r0, k,
-                       flags, decimals, weights, o_dist, o_idx, o_pred, check_finite);
+                       flags, decimals, weights, o, check_finite);
         if (rc != SKNNR_OK) return rc;
         if (!dev_ptrs) {
             // the D2H stream picks the results up behind the first stage and the slot's tail
@@ -1327,9 +1345,9 @@ int sknnr_kneighbors(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_
                 ix->stats.d2h_bytes += (int64_t)bytes;
                 return cudaMemcpyAsync(to, src, bytes, cudaMemcpyDefault, cout);
             };
-            if (out_dist) CK(deliver(out_dist + r0 * k, o_dist, (size_t)rows * k * 8, stage_dist, s.h_dist));
-            if (out_idx) CK(deliver(out_idx + r0 * k, o_idx, (size_t)rows * k * 8, stage_idx, s.h_idx));
-            if (o_pred) CK(deliver(out_pred + r0 * ix->n_out, o_pred, (size_t)rows * ix->n_out * 8, stage_pred, s.h_pred));
+            if (out_dist) CK(deliver(out_dist + r0 * k, o.dist, (size_t)rows * k * 8, stage_dist, s.h_dist));
+            if (out_idx) CK(deliver(out_idx + r0 * k, o.idx, (size_t)rows * k * 8, stage_idx, s.h_idx));
+            if (o.pred) CK(deliver(out_pred + r0 * ix->n_out, o.pred, (size_t)rows * ix->n_out * 8, stage_pred, s.h_pred));
             CK(trace_mark(3, cout));
             CK(cudaEventRecord(s.ev_last, cout));
         } else {
@@ -1378,7 +1396,7 @@ int sknnr_kneighbors(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_
 //   B: gather (compaction + transpose) -> `run` (the index's chunk pipeline on the compacted rows)
 //      -> scatter to band-major layers -> D2H of the layers
 // The count is the only value the host waits for; everything else stays asynchronous.
-// run(slot, xc, n_valid, first_row, o_dist, o_idx, o_pred) enqueues the search of one block.
+// run(slot, xc, n_valid, first_row, out) enqueues the search of one block.
 template <class IX, class RUN>
 static int raster_impl(IX *ix, int d, const void *bands, int32_t x_dtype, int64_t n_pix, int64_t band_stride,
                        int32_t use_nodata, double nodata, int32_t k, uint32_t flags, int32_t weights,
@@ -1395,11 +1413,7 @@ static int raster_impl(IX *ix, int d, const void *bands, int32_t x_dtype, int64_
     CK(cudaSetDevice(ix->device));
     const size_t esz = x_dtype_size(x_dtype);
     CallGuard guard(ix, nullptr);
-    for (auto &s : ix->slots) CK(ix->finish_slot(s));
-    for (auto &s : ix->slots) { s.ev_used = 0; s.fb_pending = false; s.flag_pending = false; }
-    ix->stats = sknnr_stats{};
-    ix->n_simt_rows = ix->n_exact_rows = 0;
-    ix->chunk_rows_seen = ix->chunk_fb_seen = ix->chunk_fail_seen = 0;
+    CK(ix->begin_call(false, nullptr, 0));
     if (n_valid_out) *n_valid_out = 0;
     if (n_pix == 0) { guard.ok = true; return SKNNR_OK; }
 
@@ -1435,17 +1449,15 @@ static int raster_impl(IX *ix, int d, const void *bands, int32_t x_dtype, int64_
         const int64_t p0 = b * chunk, rows = std::min(chunk, n_pix - p0);
         CK(cudaEventSynchronize(s.ev_cnt));
         const int64_t nv = *s.h_cnt;
-        double *o_dist = nullptr, *o_pred = nullptr;
-        long long *o_idx = nullptr;
+        ChunkOut o;
         // (with nv == 0 the gather only turns the all-zero flags into "-1 = masked")
         CK(s.xc.reserve((size_t)std::max<int64_t>(nv, 1) * d * esz));
         CK(launch_raster_gather(s.x.p, x_dtype, rows, d, s.r_cnt.p, s.r_pos.p, s.xc.p, s.stream));
         ix->stats.kernel_launches++;
         if (nv > 0) {
-            if (out_dist) { CK(s.o_dist.reserve((size_t)nv * k)); o_dist = s.o_dist.p; }
-            if (out_idx) { CK(s.o_idx.reserve((size_t)nv * k)); o_idx = s.o_idx.p; }
-            if (weights != SKNNR_W_NONE) { CK(s.o_pred.reserve((size_t)nv * ix->n_out)); o_pred = s.o_pred.p; }
-            rc = run(s, (const void *)s.xc.p, nv, valid_before, o_dist, o_idx, o_pred);
+            rc = chunk_outputs(ix, s, false, 0, nv, k, weights, out_dist, out_idx, out_pred, o);
+            if (rc != SKNNR_OK) return rc;
+            rc = run(s, (const void *)s.xc.p, nv, valid_before, o);
             if (rc != SKNNR_OK) return rc;
             if (s.tail_pending) CK(cudaStreamWaitEvent(s.stream, s.ev_tail, 0));
         }
@@ -1453,7 +1465,7 @@ static int raster_impl(IX *ix, int d, const void *bands, int32_t x_dtype, int64_
         valid_before += nv;
         if (out_dist) {
             CK(s.r_dist.reserve((size_t)rows * k));
-            CK(launch_raster_scatter_f64(s.r_pos.p, rows, o_dist, k, fill_dist, s.r_dist.p, rows, s.stream));
+            CK(launch_raster_scatter_f64(s.r_pos.p, rows, o.dist, k, fill_dist, s.r_dist.p, rows, s.stream));
             CK(cudaMemcpy2DAsync(out_dist + p0, (size_t)n_pix * 8, s.r_dist.p, (size_t)rows * 8, (size_t)rows * 8,
                                  (size_t)k, cudaMemcpyDeviceToHost, s.stream));
             ix->stats.d2h_bytes += rows * k * 8;
@@ -1461,7 +1473,7 @@ static int raster_impl(IX *ix, int d, const void *bands, int32_t x_dtype, int64_
         }
         if (out_idx) {
             CK(s.r_idx.reserve((size_t)rows * k));
-            CK(launch_raster_scatter_i64(s.r_pos.p, rows, o_idx, k, (long long)fill_idx, s.r_idx.p, rows, s.stream));
+            CK(launch_raster_scatter_i64(s.r_pos.p, rows, o.idx, k, (long long)fill_idx, s.r_idx.p, rows, s.stream));
             CK(cudaMemcpy2DAsync(out_idx + p0, (size_t)n_pix * 8, s.r_idx.p, (size_t)rows * 8, (size_t)rows * 8,
                                  (size_t)k, cudaMemcpyDeviceToHost, s.stream));
             ix->stats.d2h_bytes += rows * k * 8;
@@ -1469,7 +1481,7 @@ static int raster_impl(IX *ix, int d, const void *bands, int32_t x_dtype, int64_
         }
         if (weights != SKNNR_W_NONE) {
             CK(s.r_pred.reserve((size_t)rows * ix->n_out));
-            CK(launch_raster_scatter_f64(s.r_pos.p, rows, o_pred, ix->n_out, fill_pred, s.r_pred.p, rows, s.stream));
+            CK(launch_raster_scatter_f64(s.r_pos.p, rows, o.pred, ix->n_out, fill_pred, s.r_pred.p, rows, s.stream));
             CK(cudaMemcpy2DAsync(out_pred + p0, (size_t)n_pix * 8, s.r_pred.p, (size_t)rows * 8, (size_t)rows * 8,
                                  (size_t)ix->n_out, cudaMemcpyDeviceToHost, s.stream));
             ix->stats.d2h_bytes += rows * ix->n_out * 8;
@@ -1492,13 +1504,11 @@ int sknnr_raster_kneighbors(sknnr_index *ix, const void *bands, int32_t x_dtype,
     if (!ix) return fail(SKNNR_EINVAL, "index is NULL");
     return raster_impl(ix, ix->d_in, bands, x_dtype, n_pix, band_stride, use_nodata, nodata, k, flags, weights,
                        out_dist, out_idx, out_pred, fill_dist, fill_idx, fill_pred, n_valid_out,
-                       [&](Slot &s, const void *xc, int64_t nv, int64_t row0, double *o_dist, long long *o_idx,
-                           double *o_pred) -> int {
-                           if (ix->chunk_rows_seen >= 4096 && ix->chunk_fb_seen * 3 > ix->chunk_rows_seen)
-                               ix->tensor_demoted[ix->ns_in_use] = true;
+                       [&](Slot &s, const void *xc, int64_t nv, int64_t row0, const ChunkOut &o) -> int {
+                           ix->apply_demotion();
                            ix->spread_tail = false;
                            return run_chunk(ix, s, xc, x_dtype, ix->d_in, false, nv, row0, k, flags,
-                                            decimals, weights, o_dist, o_idx, o_pred);
+                                            decimals, weights, o);
                        });
 }
 
@@ -1510,7 +1520,9 @@ int sknnr_transform(sknnr_index *ix, const void *X, int32_t x_dtype, int64_t n_q
     std::lock_guard<std::mutex> g(ix->lock);
     CK(cudaSetDevice(ix->device));
     const size_t esz = x_dtype_size(x_dtype);
+    // (an unsynchronised device-pointer call may still be using slot 0)
     Slot &s = ix->slots[0];
+    CK(ix->finish_slot(s));
     const int64_t chunk = g_opt.chunk_rows;
     for (int64_t r0 = 0; r0 < n_q; r0 += chunk) {
         const int64_t rows = std::min(chunk, n_q - r0);
@@ -1535,7 +1547,9 @@ static int weighted_average_common(IndexBase *ix, const int64_t *idx, const doub
     if (!ix->d_y) return fail(SKNNR_EINVAL, "index was built without targets");
     std::lock_guard<std::mutex> g(ix->lock);
     CK(cudaSetDevice(ix->device));
+    // (an unsynchronised device-pointer call may still be using slot 0)
     Slot &s = ix->slots[0];
+    CK(ix->finish_slot(s));
     CK(s.o_idx.reserve((size_t)n_q * k));
     CK(s.o_dist.reserve((size_t)n_q * k));
     CK(s.o_pred.reserve((size_t)n_q * ix->n_out));
@@ -1609,15 +1623,10 @@ int sknnr_hamming_index_create(const uint16_t *ref_codes, int64_t n_ref, int32_t
             ix->wq_err = err * (1.0 + 1e-9) + 4.0 * n_trees * std::ldexp(1.0, -53) * den;
         }
     }
-    cudaError_t e = cudaMalloc(&ix->d_rcodes, (size_t)n_ref * n_trees * 2);
-    if (e == cudaSuccess) e = cudaMalloc(&ix->d_wq, wq.size() * 4);
-    if (e == cudaSuccess) e = cudaMemcpy(ix->d_wq, wq.data(), wq.size() * 4, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess)
-        e = cudaMemcpy(ix->d_rcodes, ref_codes, (size_t)n_ref * n_trees * 2, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMalloc(&ix->d_w, (size_t)n_trees * 8);
-    if (e == cudaSuccess) e = cudaMemcpy(ix->d_w, w, (size_t)n_trees * 8, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMalloc(&ix->d_lut, lut.size() * 8);
-    if (e == cudaSuccess) e = cudaMemcpy(ix->d_lut, lut.data(), lut.size() * 8, cudaMemcpyHostToDevice);
+    cudaError_t e = upload(&ix->d_rcodes, ref_codes, (size_t)n_ref * n_trees);
+    if (e == cudaSuccess) e = upload(&ix->d_wq, wq.data(), wq.size());
+    if (e == cudaSuccess) e = upload(&ix->d_w, w, (size_t)n_trees);
+    if (e == cudaSuccess) e = upload(&ix->d_lut, lut.data(), lut.size());
     if (e == cudaSuccess)
         e = cudaMalloc(&ix->d_rimg, (size_t)ix->n_rtiles * ix->n_chunks * HAM_WC * RTILE * 4);
     if (e == cudaSuccess)
@@ -1641,34 +1650,15 @@ int sknnr_hamming_index_destroy(sknnr_hamming_index *ix) {
     return SKNNR_OK;
 }
 
-int sknnr_hamming_index_stats(sknnr_hamming_index *ix, sknnr_stats *out) {
-    if (!ix || !out) return fail(SKNNR_EINVAL, "NULL argument");
-    std::lock_guard<std::mutex> g(ix->lock);
-    cudaSetDevice(ix->device);
-    for (auto &s : ix->slots) ix->harvest(s);
-    *out = ix->stats;
-    return SKNNR_OK;
-}
+int sknnr_hamming_index_stats(sknnr_hamming_index *ix, sknnr_stats *out) { return stats_common(ix, out); }
 
 static int run_hamming_chunk(sknnr_hamming_index *ix, Slot &s, const uint16_t *dq, int64_t ldq,
                              int64_t rows, int64_t row0, int k, uint32_t flags, int decimals,
-                             int weights, double *o_dist, long long *o_idx, double *o_pred) {
+                             int weights, const ChunkOut &o) {
     const bool excl = flags & SKNNR_EXCLUDE_SELF;
     const int kk = k + (excl ? 1 : 0);
     cudaStream_t st = s.stream;
-    FinishParams fp{};
-    fp.k = k;
-    fp.exclude_self = excl ? 1 : 0;
-    fp.deterministic = (flags & SKNNR_DETERMINISTIC) ? 1 : 0;
-    fp.round_scale = std::pow(10.0, (double)decimals);
-    fp.row_offset = row0;
-    fp.out_dist = o_dist;
-    fp.out_idx = o_idx;
-    fp.weights = weights;
-    fp.y = ix->d_y;
-    fp.n_ref = (int)ix->n_ref;
-    fp.n_out = ix->n_out;
-    fp.out_pred = o_pred;
+    const FinishParams fp = finish_params(ix, k, flags, decimals, weights, row0, o);
 
     // equal weights: integer counts are exact, kc = k suffices.  Unequal weights: the fixed-point
     // filter keeps >= 8 spare candidates for the certificate of hamming_refine_kernel.
@@ -1755,8 +1745,7 @@ static int hamming_kneighbors_impl(sknnr_hamming_index *ix, sknnr_forest *forest
     int rc = check_query_args(ix->n_ref, ix->n_out, n_q, k, flags, weights, q, out_pred, kk);
     if (rc != SKNNR_OK) return rc;
     if (forest) {
-        if (forest->n_trees != ix->n_trees) return fail(SKNNR_EINVAL, "forest and index disagree on the number of trees");
-        if (forest->device != ix->device) return fail(SKNNR_EINVAL, "forest and index live on different devices");
+        if ((rc = check_forest(ix, forest)) != SKNNR_OK) return rc;
         if (x_dtype_size(x_dtype) == 0) return fail(SKNNR_EINVAL, "bad x_dtype");
     }
     std::lock_guard<std::mutex> g(ix->lock);
@@ -1776,21 +1765,17 @@ static int hamming_kneighbors_impl(sknnr_hamming_index *ix, sknnr_forest *forest
     const size_t xesz = x_dtype_size(x_dtype);
     cudaStream_t user_stream = dev_ptrs ? (cudaStream_t)stream : nullptr;
     CallGuard guard(ix, user_stream);
-    if (dev_ptrs) {
-        if (ix->slots[0].last_pending) CK(cudaStreamWaitEvent(user_stream, ix->slots[0].ev_last, 0));
-    } else {
-        for (auto &s : ix->slots) CK(ix->finish_slot(s));
-    }
-    for (auto &s : ix->slots) { s.ev_used = 0; s.fb_pending = false; s.flag_pending = false; }
-    ix->stats = sknnr_stats{};
+    CK(ix->begin_call(dev_ptrs, user_stream, 1));
     ix->stats.n_queries = n_q;
     if (n_q == 0) { guard.ok = true; return SKNNR_OK; }
+    // a device-pointer call runs every chunk on slot 0, on the caller's stream
+    std::optional<StreamLoan> loan;
+    if (dev_ptrs) loan.emplace(ix->slots[0], user_stream);
     const int64_t chunk = std::min<int64_t>(g_opt.chunk_rows, (n_q + 255) / 256 * 256);
     int ci = 0;
     for (int64_t r0 = 0; r0 < n_q; r0 += chunk, ++ci) {
         const int64_t rows = std::min(chunk, n_q - r0);
         Slot &s = dev_ptrs ? ix->slots[0] : ix->slots[ci % IndexBase::kSlots];
-        StreamLoan loan(s, user_stream, dev_ptrs);
         if (!dev_ptrs) CK(ix->finish_slot(s));
         const uint16_t *dq;
         int64_t dld = ldq;
@@ -1827,31 +1812,22 @@ static int hamming_kneighbors_impl(sknnr_hamming_index *ix, sknnr_forest *forest
             dq = (const uint16_t *)s.x.p;
             dld = ix->n_trees;
         }
-        double *o_dist = nullptr, *o_pred = nullptr;
-        long long *o_idx = nullptr;
-        if (dev_ptrs) {
-            if (out_dist) o_dist = out_dist + r0 * k;
-            if (out_idx) o_idx = (long long *)out_idx + r0 * k;
-            if (weights != SKNNR_W_NONE) o_pred = out_pred + r0 * ix->n_out;
-        } else {
-            if (out_dist) { CK(s.o_dist.reserve((size_t)rows * k)); o_dist = s.o_dist.p; }
-            if (out_idx) { CK(s.o_idx.reserve((size_t)rows * k)); o_idx = s.o_idx.p; }
-            if (weights != SKNNR_W_NONE) { CK(s.o_pred.reserve((size_t)rows * ix->n_out)); o_pred = s.o_pred.p; }
-        }
-        rc = run_hamming_chunk(ix, s, dq, dld, rows, row_offset + r0, k, flags, decimals, weights,
-                               o_dist, o_idx, o_pred);
+        ChunkOut o;
+        rc = chunk_outputs(ix, s, dev_ptrs, r0, rows, k, weights, out_dist, out_idx, out_pred, o);
+        if (rc != SKNNR_OK) return rc;
+        rc = run_hamming_chunk(ix, s, dq, dld, rows, row_offset + r0, k, flags, decimals, weights, o);
         if (rc != SKNNR_OK) return rc;
         if (!dev_ptrs) {
             if (out_dist) {
-                CK(cudaMemcpyAsync(out_dist + r0 * k, o_dist, (size_t)rows * k * 8, cudaMemcpyDeviceToHost, s.stream));
+                CK(cudaMemcpyAsync(out_dist + r0 * k, o.dist, (size_t)rows * k * 8, cudaMemcpyDeviceToHost, s.stream));
                 ix->stats.d2h_bytes += rows * k * 8;
             }
             if (out_idx) {
-                CK(cudaMemcpyAsync(out_idx + r0 * k, o_idx, (size_t)rows * k * 8, cudaMemcpyDeviceToHost, s.stream));
+                CK(cudaMemcpyAsync(out_idx + r0 * k, o.idx, (size_t)rows * k * 8, cudaMemcpyDeviceToHost, s.stream));
                 ix->stats.d2h_bytes += rows * k * 8;
             }
-            if (o_pred) {
-                CK(cudaMemcpyAsync(out_pred + r0 * ix->n_out, o_pred, (size_t)rows * ix->n_out * 8, cudaMemcpyDeviceToHost, s.stream));
+            if (o.pred) {
+                CK(cudaMemcpyAsync(out_pred + r0 * ix->n_out, o.pred, (size_t)rows * ix->n_out * 8, cudaMemcpyDeviceToHost, s.stream));
                 ix->stats.d2h_bytes += rows * ix->n_out * 8;
             }
         } else {
@@ -1874,19 +1850,18 @@ int sknnr_hamming_raster_kneighbors_forest(sknnr_hamming_index *ix, sknnr_forest
                                            int32_t weights, double *out_pred, double fill_dist,
                                            int64_t fill_idx, double fill_pred, int64_t *n_valid_out) {
     if (!ix || !forest) return fail(SKNNR_EINVAL, "index or forest is NULL");
-    if (forest->n_trees != ix->n_trees) return fail(SKNNR_EINVAL, "forest and index disagree on the number of trees");
-    if (forest->device != ix->device) return fail(SKNNR_EINVAL, "forest and index live on different devices");
+    const int rc = check_forest(ix, forest);
+    if (rc != SKNNR_OK) return rc;
     return raster_impl(ix, forest->n_features, bands, x_dtype, n_pix, band_stride, use_nodata, nodata, k, flags,
                        weights, out_dist, out_idx, out_pred, fill_dist, fill_idx, fill_pred, n_valid_out,
-                       [&](Slot &s, const void *xc, int64_t nv, int64_t row0, double *o_dist, long long *o_idx,
-                           double *o_pred) -> int {
+                       [&](Slot &s, const void *xc, int64_t nv, int64_t row0, const ChunkOut &o) -> int {
                            CK(s.codes.reserve((size_t)nv * ix->n_trees));
                            CK(launch_forest_apply(xc, x_dtype, forest->n_features, nv,
                                                   forest->n_features, forest->d_nodes, forest->d_roots,
                                                   forest->n_trees, s.codes.p, nullptr, ix->n_trees, s.stream));
                            ix->stats.kernel_launches++;
                            return run_hamming_chunk(ix, s, s.codes.p, ix->n_trees, nv, row0, k, flags, decimals,
-                                                    weights, o_dist, o_idx, o_pred);
+                                                    weights, o);
                        });
 }
 
@@ -1915,10 +1890,8 @@ int sknnr_forest_create(const int32_t *tree_offsets, const int32_t *children_lef
     if (!tree_offsets || !children_left || !children_right || !feature || !threshold || !out || n_trees < 1 ||
         n_features < 1)
         return fail(SKNNR_EINVAL, "bad arguments to sknnr_forest_create");
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0)
-        return fail(SKNNR_ENODEV, "no CUDA device: sknnr_b200 has no CPU fallback");
-    if (device < 0 || device >= count) return fail(SKNNR_EINVAL, "bad device ordinal");
+    const int rc = check_device(device);
+    if (rc != SKNNR_OK) return rc;
     if (forest_smem_bytes(n_features) > 227 * 1024) return fail(SKNNR_EUNSUP, "too many features for the forest kernel");
     const long long n_nodes = tree_offsets[n_trees];
     if (n_nodes < n_trees) return fail(SKNNR_EINVAL, "bad tree offsets");
@@ -1954,10 +1927,8 @@ int sknnr_forest_create(const int32_t *tree_offsets, const int32_t *children_lef
     f->n_features = n_features;
     f->n_nodes = n_nodes;
     cudaError_t e = cudaSetDevice(device);
-    if (e == cudaSuccess) e = cudaMalloc(&f->d_nodes, nodes.size() * sizeof(ForestNode));
-    if (e == cudaSuccess) e = cudaMemcpy(f->d_nodes, nodes.data(), nodes.size() * sizeof(ForestNode), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMalloc(&f->d_roots, roots.size() * sizeof(int));
-    if (e == cudaSuccess) e = cudaMemcpy(f->d_roots, roots.data(), roots.size() * sizeof(int), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = upload(&f->d_nodes, nodes.data(), nodes.size());
+    if (e == cudaSuccess) e = upload(&f->d_roots, roots.data(), roots.size());
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&f->stream, cudaStreamNonBlocking);
     if (e != cudaSuccess) {
         sknnr_forest_destroy(f);
@@ -1973,8 +1944,6 @@ int sknnr_forest_destroy(sknnr_forest *f) {
     if (f->stream) cudaStreamDestroy(f->stream);
     cudaFree(f->d_nodes);
     cudaFree(f->d_roots);
-    f->x.release();
-    f->ids.release();
     delete f;
     return SKNNR_OK;
 }
