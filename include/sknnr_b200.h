@@ -233,6 +233,29 @@ int sknnr_hamming_weighted_average(sknnr_hamming_index *index, const int64_t *id
                                    const double *w, int64_t n_q, int32_t k,
                                    double *out_pred);
 int sknnr_hamming_index_stats(sknnr_hamming_index *index, sknnr_stats *out);
+/* out3[0] rows of the last call the filter's certificate left uncertified (= stats.n_fallback),
+ * out3[1] 0 (no FP32 stage), out3[2] rows that reached the exhaustive float64 kernel.        */
+int sknnr_hamming_index_cascade_counts(sknnr_hamming_index *index, int64_t *out3);
+
+/* ---- Wide mode: trees with more than 31743 distinct node IDs ---------------------------------
+ * 16-bit codes run out at 31743 per tree.  A wide index keeps exact u32 codes per tree
+ * (0xFFFFFFFF = "matches nothing", allowed in queries only) and runs the 16-bit search as a filter on
+ * their hashed image (code mod 31743).  Hashing only merges distinct codes, so a hashed count never
+ * exceeds the true one; a float64 re-rank of the candidates on the exact codes certifies the top k,
+ * and the rows it cannot certify go to the exhaustive kernel on the exact codes.  Results are the
+ * same as those of a 16-bit index over the same IDs would be: bit-equal to SciPy.
+ *   ref_codes [n_ref, n_trees] u32 C-order; every other argument as in sknnr_hamming_index_create.
+ * A wide index answers sknnr_hamming_kneighbors_wide (q_codes [n_q, ldq] u32), and the forest entry
+ * points with any forest (the walk's node IDs are the exact codes); sknnr_hamming_kneighbors
+ * refuses it.                                                                                  */
+int sknnr_hamming_index_create_wide(const uint32_t *ref_codes, int64_t n_ref, int32_t n_trees,
+                                    const double *w, const double *y, int32_t n_out,
+                                    int32_t device, sknnr_hamming_index **out);
+int sknnr_hamming_kneighbors_wide(sknnr_hamming_index *index, const uint32_t *q_codes,
+                                  int64_t n_q, int64_t ldq, int64_t row_offset, int32_t k,
+                                  uint32_t flags, int32_t decimals, double *out_dist,
+                                  int64_t *out_idx, int32_t weights, double *out_pred,
+                                  void *stream);
 
 /* ---- Forests: RFNodeTransformer.transform on the device (scope row f1) -------------------
  * Replaces ref:src/sknnr/transformers/_tree_node_transformer.py:177-201 (est.apply per forest,
@@ -246,7 +269,8 @@ int sknnr_hamming_index_stats(sknnr_hamming_index *index, sknnr_stats *out);
  *             scikit-learn's tree_ arrays (child indices local to their tree, -1 = leaf;
  *             missing_go_to_left may be NULL)
  *   node_code [n_nodes] u16 or NULL: the node code the Hamming index uses for each (leaf)
- *             node, 31743 = "matches nothing"; NULL = the node ID itself                    */
+ *             node, 31743 = "matches nothing"; NULL = the node ID itself.  A wide Hamming
+ *             index reads the node IDs themselves and ignores node_code.                       */
 int sknnr_forest_create(const int32_t *tree_offsets, const int32_t *children_left,
                         const int32_t *children_right, const int32_t *feature,
                         const double *threshold, const uint8_t *missing_go_to_left,

@@ -47,21 +47,41 @@ class IndependentPredictorMixin:
         self.independent_score_ = float(r2_score(y, self.independent_prediction_))
 
 
-def _node_code_tables(ref_ids: np.ndarray):
-    """Map each tree's node IDs to dense 16-bit codes (only equality matters)."""
+class WideCodes:
+    """Code tables of a wide Hamming index (a tree with more than ``L.MAX_CODE`` distinct node IDs):
+    exact 32-bit codes, ``L.WIDE_NONE`` for a value that matches nothing.  ``tables`` None: every
+    node ID is its own code (a forest's node IDs, which the device walk emits as they are); else,
+    per tree, the sorted node IDs that map to codes 0, 1, ..."""
+
+    def __init__(self, tables):
+        self.tables = tables
+
+
+def _node_code_tables(ref_ids: np.ndarray, ids_are_codes: bool = False):
+    """Map each tree's node IDs to dense 16-bit codes (only equality matters): None when the IDs
+    already fit, else the per-tree tables of sorted IDs.  When a tree has more distinct IDs than
+    16-bit codes reach, a :class:`WideCodes` (``ids_are_codes``: the IDs are a forest's node IDs
+    and serve as their own codes)."""
     if ref_ids.min() >= 0 and ref_ids.max() < L.MAX_CODE:
         return None  # IDs already fit: identity mapping
-    tables = []
-    for t in range(ref_ids.shape[1]):
-        u = np.unique(ref_ids[:, t])
-        if len(u) > L.MAX_CODE:
-            raise NotImplementedError("more than 31743 distinct node IDs in one tree")
-        tables.append(u)
-    return tables
+    tables = [np.unique(ref_ids[:, t]) for t in range(ref_ids.shape[1])]
+    if max(len(u) for u in tables) <= L.MAX_CODE:
+        return tables
+    if ids_are_codes and ref_ids.min() >= 0 and ref_ids.max() < L.WIDE_NONE:
+        return WideCodes(None)
+    return WideCodes(tables)
+
+
+def _forest_tables(tables):
+    """The code tables a device forest needs for an index coded by ``tables``: none for a wide
+    index, whose forest queries carry the node IDs themselves."""
+    return None if isinstance(tables, WideCodes) else tables
 
 
 def _encode_nodes(ids: np.ndarray, tables) -> np.ndarray:
     ids = np.asarray(ids)
+    if isinstance(tables, WideCodes):
+        return _encode_wide(ids, tables.tables)
     if tables is None:
         bad = (ids < 0) | (ids >= L.MAX_CODE)
         out = ids.astype(np.uint16)
@@ -73,6 +93,22 @@ def _encode_nodes(ids: np.ndarray, tables) -> np.ndarray:
         pos_c = np.minimum(pos, len(u) - 1)
         hit = u[pos_c] == ids[:, t]
         out[:, t] = np.where(hit, pos_c, L.MAX_CODE)
+    return out
+
+
+def _encode_wide(ids: np.ndarray, tables) -> np.ndarray:
+    """Exact u32 codes of a wide index (``WideCodes.tables``); unseen values match nothing."""
+    if tables is None:
+        out = np.full(ids.shape, L.WIDE_NONE, dtype=np.uint32)
+        ok = (ids >= 0) & (ids < L.WIDE_NONE)
+        out[ok] = ids[ok]
+        return out
+    out = np.empty(ids.shape, dtype=np.uint32)
+    for t, u in enumerate(tables):
+        pos = np.searchsorted(u, ids[:, t])
+        pos_c = np.minimum(pos, len(u) - 1)
+        hit = u[pos_c] == ids[:, t]
+        out[:, t] = np.where(hit, pos_c, L.WIDE_NONE)
     return out
 
 
@@ -129,7 +165,7 @@ class RawKNNRegressor(DFIndexCrosswalkMixin, IndependentPredictorMixin, KNeighbo
             if not np.all(ref_ids == np.floor(ref_ids)):
                 raise NotImplementedError("the Hamming path expects integer node IDs")
             ref_ids = ref_ids.astype(np.int64)
-            tables = _node_code_tables(ref_ids)
+            tables = _node_code_tables(ref_ids, ids_are_codes=self.__dict__.get("_forest_node_ids", False))
             self.__dict__["_node_tables"] = tables
             w = (self.effective_metric_params_ or {}).get("w")
             if w is None:
@@ -183,7 +219,8 @@ class RawKNNRegressor(DFIndexCrosswalkMixin, IndependentPredictorMixin, KNeighbo
             return ix.query(None, k, exclude_self=True, **kw)
         if forest is not None:
             k = self._check_k(n_neighbors, False, X.shape[0])
-            fx = forest._forest_index(self.__dict__.get("_node_tables"), devices=getattr(ix, "devices", None))
+            fx = forest._forest_index(_forest_tables(self.__dict__.get("_node_tables")),
+                                      devices=getattr(ix, "devices", None))
             return ix.query_forest(fx, X, k, **kw)
         hamming = hasattr(ix, "n_trees")
         if not raw:
@@ -196,7 +233,7 @@ class RawKNNRegressor(DFIndexCrosswalkMixin, IndependentPredictorMixin, KNeighbo
             if Xa.dtype.kind == "f":
                 # scipy's hamming compares values, not truncated integers: a non-integer query
                 # value equals no node ID ($SP/scipy/spatial/distance.py:1718-1723)
-                codes[Xa != np.floor(Xa)] = L.MAX_CODE
+                codes[Xa != np.floor(Xa)] = L.WIDE_NONE if codes.dtype == np.uint32 else L.MAX_CODE
             return ix.query(codes, k, **kw)
         # The reference rejects non-finite values when the regressor validates the (transformed)
         # array ($SP/sklearn/neighbors/_base.py:831-838).  The projection kernel reads every query
@@ -299,6 +336,9 @@ class TransformedKNeighborsRegressor(BaseEstimator, ABC):
         if self._fusable():
             center, scale, proj, _ = self.transformer_._affine()
             self.regressor_._projection = (center, scale, proj)
+        if hasattr(self.transformer_, "_forest_index"):
+            # (node IDs the device forest walk reproduces: a wide index keeps them as its codes)
+            self.regressor_._forest_node_ids = True
         self.regressor_.fit(X_transformed, y)
         self.regressor_._set_dataframe_index_in(X)
 

@@ -354,22 +354,34 @@ class KNNIndex(_IndexBase):
 
 
 class HammingIndex(_IndexBase):
-    """Fitted state of an RFNN-style estimator: 16-bit node codes + Hamming weights."""
+    """Fitted state of an RFNN-style estimator: node codes + Hamming weights.  ``ref_codes`` of
+    dtype uint32 make a wide index (exact 32-bit codes, ``L.WIDE_NONE`` matches nothing, for trees
+    with more than ``L.MAX_CODE`` distinct node IDs); any other dtype holds 16-bit codes."""
 
     _destroy = "sknnr_hamming_index_destroy"
     _stats = "sknnr_hamming_index_stats"
 
     def __init__(self, ref_codes, w, y=None, device=None):
         super().__init__()
-        ref_codes = np.ascontiguousarray(ref_codes, dtype=np.uint16)
+        self.wide = np.asarray(ref_codes).dtype == np.uint32
+        self._code_dtype = np.uint32 if self.wide else np.uint16
+        ref_codes = np.ascontiguousarray(ref_codes, dtype=self._code_dtype)
         self.n_ref, self.n_trees = ref_codes.shape
         w = _f64(w)
         y = _f64(y, 2)
         self.n_out = 0 if y is None else y.shape[1]
         self.device = default_device() if device is None else int(device)
-        L.check(self._lib.sknnr_hamming_index_create(
-            _ptr(ref_codes), self.n_ref, self.n_trees, _ptr(w), _ptr(y), self.n_out, self.device,
-            C.byref(self._h)))
+        create = self._lib.sknnr_hamming_index_create_wide if self.wide else self._lib.sknnr_hamming_index_create
+        L.check(create(_ptr(ref_codes), self.n_ref, self.n_trees, _ptr(w), _ptr(y), self.n_out, self.device,
+                       C.byref(self._h)))
+        self._kneighbors = self._lib.sknnr_hamming_kneighbors_wide if self.wide else self._lib.sknnr_hamming_kneighbors
+
+    def cascade_counts(self) -> dict:
+        """Rows of the last call the filter left uncertified, and rows that reached the exhaustive
+        float64 kernel (those, plus every row of a call the filter does not serve)."""
+        out = (C.c_int64 * 3)()
+        L.check(self._lib.sknnr_hamming_index_cascade_counts(self._h, out))
+        return {"uncertified": out[0], "to_exact": out[2]}
 
     def query(self, codes, k, *, exclude_self=False, deterministic=True, decimals=10,
               row_offset=0, weights=None, with_pred=False, return_distance=True,
@@ -377,14 +389,14 @@ class HammingIndex(_IndexBase):
         if exclude_self:
             n_q, cp, ldq = self.n_ref, None, 0
         else:
-            codes = np.ascontiguousarray(codes, dtype=np.uint16)
+            codes = np.ascontiguousarray(codes, dtype=self._code_dtype)
             n_q, ldq = codes.shape[0], codes.shape[1]
             if ldq != self.n_trees:
                 raise ValueError(f"X has {ldq} features, but {self.n_trees} are expected")
             cp = _ptr(codes)
         mode = _weights_mode(weights, with_pred)
         dist, idx, pred = _outputs(out, n_q, k, self.n_out, return_distance, return_index, mode)
-        L.check(self._lib.sknnr_hamming_kneighbors(
+        L.check(self._kneighbors(
             self._h, cp, n_q, ldq, int(row_offset), int(k),
             self._flags(exclude_self, deterministic), int(decimals), _ptr(dist), _ptr(idx), mode,
             _ptr(pred), None))
@@ -418,7 +430,7 @@ class HammingIndex(_IndexBase):
                      deterministic=True, decimals=10, row_offset=0, stream=0):
         mode = _weights_mode(weights, bool(pred_ptr))
         flags = self._flags(False, deterministic) | L.DEVICE_PTRS
-        L.check(self._lib.sknnr_hamming_kneighbors(
+        L.check(self._kneighbors(
             self._h, C.c_void_p(q_ptr), int(n_q), int(ldq), int(row_offset), int(k), flags,
             int(decimals), C.c_void_p(dist_ptr or None), C.c_void_p(idx_ptr or None), mode,
             C.c_void_p(pred_ptr or None), C.c_void_p(stream or None)))

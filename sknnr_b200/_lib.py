@@ -22,6 +22,7 @@ W_NONE, W_UNIFORM, W_DISTANCE = 0, 1, 2
 ENGINE_AUTO, ENGINE_SIMT, ENGINE_TENSOR, ENGINE_EXACT = 0, 1, 2, 3
 METRICS = {"euclidean": 0, "manhattan": 1, "chebyshev": 2}   # SKNNR_METRIC_*
 MAX_CODE = 31743
+WIDE_NONE = 0xFFFFFFFF   # wide mode: the u32 code that matches nothing
 
 # integer element types the query calls read as they are (no float64 copy on the host)
 NATIVE_INT_DTYPES = (np.uint8, np.int16, np.uint16, np.int32, np.int64)
@@ -46,7 +47,8 @@ EXPORTS = [
     "sknnr_forest_apply", "sknnr_hamming_kneighbors_forest", "sknnr_raster_kneighbors",
     "sknnr_hamming_raster_kneighbors_forest", "sknnr_device_alloc", "sknnr_device_free",
     "sknnr_ipc_export", "sknnr_ipc_open", "sknnr_ipc_close", "sknnr_device_copy", "sknnr_host_chunk_plan",
-    "sknnr_index_create_metric",
+    "sknnr_index_create_metric", "sknnr_hamming_index_create_wide", "sknnr_hamming_kneighbors_wide",
+    "sknnr_hamming_index_cascade_counts",
 ]
 
 
@@ -103,6 +105,9 @@ def load() -> C.CDLL:
     lib.sknnr_hamming_kneighbors.argtypes = [vp, vp, i64, i64, i64, i32, u32, i32, vp, vp, i32, vp, vp]
     lib.sknnr_hamming_weighted_average.argtypes = [vp, vp, vp, i64, i32, vp]
     lib.sknnr_hamming_index_stats.argtypes = [vp, C.POINTER(Stats)]
+    lib.sknnr_hamming_index_cascade_counts.argtypes = [vp, C.POINTER(C.c_int64)]
+    lib.sknnr_hamming_index_create_wide.argtypes = lib.sknnr_hamming_index_create.argtypes
+    lib.sknnr_hamming_kneighbors_wide.argtypes = lib.sknnr_hamming_kneighbors.argtypes
     lib.sknnr_host_alloc.argtypes = [C.POINTER(vp), i64]
     lib.sknnr_host_free.argtypes = [vp]
     lib.sknnr_measure_fp32_peak.argtypes = [i32, C.POINTER(C.c_double)]

@@ -276,6 +276,7 @@ struct Slot {
     DevBuf<int> fbm;               // failures of the tensor engine's second pass (stage 1b), same layout
     DevBuf<float> fb_thr;          // second-pass thresholds of the first-stage failures (order of fb's list)
     DevBuf<uint16_t> codes;        // node codes produced by the device forest walk
+    DevBuf<uint32_t> wide;         // wide mode: exact query codes (forest walk node IDs or the caller's)
     DevBuf<uint32_t> qimg_h;       // Hamming query image
     DevBuf<int> cand_idx;
     DevBuf<float> cand_thr;
@@ -652,7 +653,8 @@ struct sknnr_index : IndexBase {
 
 struct sknnr_hamming_index : IndexBase {
     int n_trees = 0, n_chunks = 0, n_rtiles = 0;
-    uint16_t *d_rcodes = nullptr;
+    uint16_t *d_rcodes = nullptr;  // wide mode: the filter codes of d_rwide
+    uint32_t *d_rwide = nullptr;   // wide mode only: exact u32 codes
     uint32_t *d_rimg = nullptr;
     double *d_w = nullptr, *d_lut = nullptr;
     double wsum = 0.0;
@@ -1567,14 +1569,11 @@ int sknnr_weighted_average(sknnr_index *ix, const int64_t *idx, const double *w,
 }
 
 // -----------------------------------------------------------------------------------------
-int sknnr_hamming_index_create(const uint16_t *ref_codes, int64_t n_ref, int32_t n_trees,
-                               const double *w, const double *y, int32_t n_out, int32_t device,
-                               sknnr_hamming_index **out) {
-    if (!ref_codes || !w || !out || n_ref < 1 || n_trees < 1)
-        return fail(SKNNR_EINVAL, "bad arguments to sknnr_hamming_index_create");
-    if (n_ref >= (1LL << 31) - 64) return fail(SKNNR_EUNSUP, "n_ref too large");
-    for (int64_t e = 0; e < n_ref * (int64_t)n_trees; ++e)
-        if (ref_codes[e] > 31743) return fail(SKNNR_EINVAL, "node codes must be <= 31743");
+// Shared body of sknnr_hamming_index_create (ref_wide == NULL) and sknnr_hamming_index_create_wide
+// (ref_codes: the filter codes of ref_wide)
+static int hamming_index_create(const uint16_t *ref_codes, const uint32_t *ref_wide, int64_t n_ref,
+                                int32_t n_trees, const double *w, const double *y, int32_t n_out,
+                                int32_t device, sknnr_hamming_index **out) {
     if (y == nullptr) n_out = 0;
     sknnr_hamming_index *ix = new sknnr_hamming_index();
     int rc = ix->init_common(device, y, n_ref, n_out);
@@ -1624,6 +1623,7 @@ int sknnr_hamming_index_create(const uint16_t *ref_codes, int64_t n_ref, int32_t
         }
     }
     cudaError_t e = upload(&ix->d_rcodes, ref_codes, (size_t)n_ref * n_trees);
+    if (e == cudaSuccess && ref_wide) e = upload(&ix->d_rwide, ref_wide, (size_t)n_ref * n_trees);
     if (e == cudaSuccess) e = upload(&ix->d_wq, wq.data(), wq.size());
     if (e == cudaSuccess) e = upload(&ix->d_w, w, (size_t)n_trees);
     if (e == cudaSuccess) e = upload(&ix->d_lut, lut.data(), lut.size());
@@ -1641,16 +1641,52 @@ int sknnr_hamming_index_create(const uint16_t *ref_codes, int64_t n_ref, int32_t
     return SKNNR_OK;
 }
 
+int sknnr_hamming_index_create(const uint16_t *ref_codes, int64_t n_ref, int32_t n_trees,
+                               const double *w, const double *y, int32_t n_out, int32_t device,
+                               sknnr_hamming_index **out) {
+    if (!ref_codes || !w || !out || n_ref < 1 || n_trees < 1)
+        return fail(SKNNR_EINVAL, "bad arguments to sknnr_hamming_index_create");
+    if (n_ref >= (1LL << 31) - 64) return fail(SKNNR_EUNSUP, "n_ref too large");
+    for (int64_t e = 0; e < n_ref * (int64_t)n_trees; ++e)
+        if (ref_codes[e] > 31743) return fail(SKNNR_EINVAL, "node codes must be <= 31743");
+    return hamming_index_create(ref_codes, nullptr, n_ref, n_trees, w, y, n_out, device, out);
+}
+
+int sknnr_hamming_index_create_wide(const uint32_t *ref_codes, int64_t n_ref, int32_t n_trees,
+                                    const double *w, const double *y, int32_t n_out, int32_t device,
+                                    sknnr_hamming_index **out) {
+    if (!ref_codes || !w || !out || n_ref < 1 || n_trees < 1)
+        return fail(SKNNR_EINVAL, "bad arguments to sknnr_hamming_index_create_wide");
+    if (n_ref >= (1LL << 31) - 64) return fail(SKNNR_EUNSUP, "n_ref too large");
+    std::vector<uint16_t> filt((size_t)n_ref * n_trees);
+    for (size_t e = 0; e < filt.size(); ++e) {
+        if (ref_codes[e] == WIDE_NONE) return fail(SKNNR_EINVAL, "reference codes must be < 0xFFFFFFFF");
+        filt[e] = hamming_filter_code(ref_codes[e]);
+    }
+    return hamming_index_create(filt.data(), ref_codes, n_ref, n_trees, w, y, n_out, device, out);
+}
+
 int sknnr_hamming_index_destroy(sknnr_hamming_index *ix) {
     if (!ix) return SKNNR_OK;
     ix->release_common();
-    cudaFree(ix->d_rcodes); cudaFree(ix->d_rimg); cudaFree(ix->d_w); cudaFree(ix->d_lut);
+    cudaFree(ix->d_rcodes); cudaFree(ix->d_rwide); cudaFree(ix->d_rimg); cudaFree(ix->d_w); cudaFree(ix->d_lut);
     cudaFree(ix->d_wq);
     delete ix;
     return SKNNR_OK;
 }
 
 int sknnr_hamming_index_stats(sknnr_hamming_index *ix, sknnr_stats *out) { return stats_common(ix, out); }
+
+int sknnr_hamming_index_cascade_counts(sknnr_hamming_index *ix, int64_t *out3) {
+    if (!ix || !out3) return fail(SKNNR_EINVAL, "NULL argument");
+    std::lock_guard<std::mutex> g(ix->lock);
+    cudaSetDevice(ix->device);
+    for (auto &s : ix->slots) ix->harvest(s);
+    out3[0] = ix->stats.n_fallback;
+    out3[1] = 0;
+    out3[2] = ix->stats.n_fallback + ix->n_exact_rows;
+    return SKNNR_OK;
+}
 
 static int run_hamming_chunk(sknnr_hamming_index *ix, Slot &s, const uint16_t *dq, int64_t ldq,
                              int64_t rows, int64_t row0, int k, uint32_t flags, int decimals,
@@ -1685,6 +1721,7 @@ static int run_hamming_chunk(sknnr_hamming_index *ix, Slot &s, const uint16_t *d
         CK(ix->launch_exact_chained(ea, fp, kk, st));
         if (g_opt.timing) CK(s.mark(st));
         ix->stats.kernel_launches++;
+        ix->n_exact_rows += rows;
         return SKNNR_OK;
     }
     const int kc = fast_u ? kc_u : kc_w;
@@ -1732,15 +1769,125 @@ static int run_hamming_chunk(sknnr_hamming_index *ix, Slot &s, const uint16_t *d
     return SKNNR_OK;
 }
 
-// Shared body of sknnr_hamming_kneighbors (forest == NULL: `q` holds u16 node codes, row stride
-// ldq elements) and sknnr_hamming_kneighbors_forest (`q` holds raw feature rows of x_dtype, row
-// stride ldq elements; every chunk is walked through the forest on the device first).
+// Wide mode: the 16-bit search runs on the filter codes dq; hamming_wide_refine_kernel re-ranks its
+// candidates on the exact codes dw and certifies them; the rows it cannot certify (and every row when
+// k (+1) > 24) go to the exhaustive kernel on the exact codes.
+static int run_hamming_wide_chunk(sknnr_hamming_index *ix, Slot &s, const uint16_t *dq, int64_t ldq,
+                                  const uint32_t *dw, int64_t ldw, int64_t rows, int64_t row0, int k,
+                                  uint32_t flags, int decimals, int weights, const ChunkOut &o) {
+    const bool excl = flags & SKNNR_EXCLUDE_SELF;
+    const int kk = k + (excl ? 1 : 0);
+    cudaStream_t st = s.stream;
+    const FinishParams fp = finish_params(ix, k, flags, decimals, weights, row0, o);
+
+    // both certificates need spare candidates: lists of >= k (+1) + 8
+    const bool exact_only = g_opt.engine == SKNNR_ENGINE_EXACT;
+    const int kc8 = pick_kc(kk, 8);
+    const bool fast_u = ix->uniform && kc8 != 0 && ix->n_chunks * HAM_WC <= 2048 && !exact_only;
+    const bool fast_w = !fast_u && !ix->uniform && ix->wq_ok && kc8 != 0 && !exact_only;
+    ix->stats.engine = (fast_u || fast_w) ? SKNNR_ENGINE_SIMT : SKNNR_ENGINE_EXACT;
+
+    ExactArgs ea{};
+    ea.metric = 4;
+    ea.qwide = dw;
+    ea.ldq = ldw;
+    ea.rwide = ix->d_rwide;
+    ea.n_trees = ix->n_trees;
+    ea.w = ix->d_w;
+    ea.wsum = ix->wsum;
+    ea.n_q = rows;
+    ea.n_ref = (int)ix->n_ref;
+    ea.grid = ix->exact_ctas(rows);
+    if (!fast_u && !fast_w) {
+        if (g_opt.timing) CK(s.mark(st));
+        CK(ix->launch_exact_chained(ea, fp, kk, st));
+        if (g_opt.timing) CK(s.mark(st));
+        ix->stats.kernel_launches++;
+        ix->n_exact_rows += rows;
+        return SKNNR_OK;
+    }
+    const int kc = fast_u ? kc8 : std::max(16, kc8);
+    const int64_t n_qtiles = (rows + QTILE - 1) / QTILE;
+    CK(s.qimg_h.reserve((size_t)n_qtiles * ix->n_chunks * HAM_WC * QTILE));
+    CK(s.cand_idx.reserve((size_t)rows * kc));
+    CK(s.cand_cnt.reserve((size_t)rows * kc));
+    CK(launch_hamming_pack(dq, rows, ldq, ix->n_trees, ix->n_chunks, QTILE, 31743, s.qimg_h.p, st));
+    if (g_opt.timing) CK(s.mark(st));
+    CK(launch_hamming_search(s.qimg_h.p, ix->d_rimg, fast_w ? ix->d_wq : nullptr, ix->n_chunks, ix->n_rtiles,
+                             rows, (int)ix->n_ref, kc, s.cand_idx.p, s.cand_cnt.p, st));
+    if (g_opt.timing) CK(s.mark(st));
+    CK(s.fb.reserve((size_t)rows + 1));
+    CK(cudaMemsetAsync(s.fb.p, 0, sizeof(int), st));
+    HammingWideRefineArgs ha{};
+    ha.cand_idx = s.cand_idx.p;
+    ha.cand_cnt = s.cand_cnt.p;
+    ha.kc = kc;
+    ha.qcodes = dw;
+    ha.ldq = ldw;
+    ha.rcodes = ix->d_rwide;
+    ha.n_trees = ix->n_trees;
+    ha.lut = fast_u ? ix->d_lut : nullptr;
+    ha.w = ix->d_w;
+    ha.wsum = ix->wsum;
+    ha.scale = ix->wq_scale;
+    ha.err = ix->wq_err;
+    ha.n_q = rows;
+    ha.fb_count = s.fb.p;
+    ha.fb_list = s.fb.p + 1;
+    CK(launch_hamming_wide_refine(ha, fp, st));
+    ea.list = s.fb.p + 1;
+    ea.count = s.fb.p;
+    CK(ix->launch_exact_chained(ea, fp, kk, st));
+    CK(cudaMemcpyAsync(&s.h_fb[0], s.fb.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+    s.h_fb[1] = 0;
+    s.fb_pending = true;
+    s.rows_in_flight = 0;
+    ix->stats.kernel_launches += 4;
+    return SKNNR_OK;
+}
+
+// The search of one chunk of query codes: dq the 16-bit codes (row stride ldq); in wide mode dw the
+// exact codes (row stride ldw) and dq their filter codes
+static int run_codes_chunk(sknnr_hamming_index *ix, Slot &s, const uint16_t *dq, int64_t ldq,
+                           const uint32_t *dw, int64_t ldw, int64_t rows, int64_t row0, int k,
+                           uint32_t flags, int decimals, int weights, const ChunkOut &o) {
+    if (ix->d_rwide)
+        return run_hamming_wide_chunk(ix, s, dq, ldq, dw, ldw, rows, row0, k, flags, decimals, weights, o);
+    return run_hamming_chunk(ix, s, dq, ldq, rows, row0, k, flags, decimals, weights, o);
+}
+
+// Forest walk of `rows` feature rows x (row stride ldx) to the index's query codes, on s.stream:
+// s.codes holds the 16-bit codes; in wide mode s.wide holds the node IDs (the exact codes) and
+// s.codes their filter codes
+static int walk_forest(sknnr_hamming_index *ix, sknnr_forest *forest, Slot &s, const void *x,
+                       int32_t x_dtype, int64_t ldx, int64_t rows) {
+    CK(s.codes.reserve((size_t)rows * ix->n_trees));
+    if (!ix->d_rwide) {
+        CK(launch_forest_apply(x, x_dtype, ldx, rows, forest->n_features, forest->d_nodes, forest->d_roots,
+                               forest->n_trees, s.codes.p, nullptr, ix->n_trees, s.stream));
+        ix->stats.kernel_launches++;
+        return SKNNR_OK;
+    }
+    CK(s.wide.reserve((size_t)rows * ix->n_trees));
+    CK(launch_forest_apply(x, x_dtype, ldx, rows, forest->n_features, forest->d_nodes, forest->d_roots,
+                           forest->n_trees, nullptr, (int *)s.wide.p, ix->n_trees, s.stream));
+    CK(launch_hamming_hash(s.wide.p, rows, ix->n_trees, ix->n_trees, s.codes.p, s.stream));
+    ix->stats.kernel_launches += 2;
+    return SKNNR_OK;
+}
+
+// Shared body of sknnr_hamming_kneighbors / sknnr_hamming_kneighbors_wide (forest == NULL: `q` holds
+// the index's node codes, u16, or u32 in wide mode, row stride ldq elements) and
+// sknnr_hamming_kneighbors_forest (`q` holds raw feature rows of x_dtype, row stride ldq elements;
+// every chunk is walked through the forest on the device first).
 static int hamming_kneighbors_impl(sknnr_hamming_index *ix, sknnr_forest *forest, const void *q,
                                    int32_t x_dtype, int64_t n_q, int64_t ldq, int64_t row_offset,
                                    int32_t k, uint32_t flags, int32_t decimals, double *out_dist,
                                    int64_t *out_idx, int32_t weights, double *out_pred, void *stream) {
     if (!ix) return fail(SKNNR_EINVAL, "index is NULL");
-    const uint16_t *q_codes = forest ? nullptr : (const uint16_t *)q;
+    const void *q_codes = forest ? nullptr : q;
+    const bool wide = ix->d_rwide != nullptr;
+    const size_t code_bytes = wide ? 4 : 2;
     int kk = 0;
     int rc = check_query_args(ix->n_ref, ix->n_out, n_q, k, flags, weights, q, out_pred, kk);
     if (rc != SKNNR_OK) return rc;
@@ -1755,7 +1902,7 @@ static int hamming_kneighbors_impl(sknnr_hamming_index *ix, sknnr_forest *forest
     bool q_on_device = dev_ptrs;
     if (excl) {
         forest = nullptr;   // X=None: the reference plots' own codes
-        q_codes = ix->d_rcodes;
+        q_codes = wide ? (const void *)ix->d_rwide : (const void *)ix->d_rcodes;
         n_q = ix->n_ref;
         ldq = ix->n_trees;
         q_on_device = true;
@@ -1779,6 +1926,8 @@ static int hamming_kneighbors_impl(sknnr_hamming_index *ix, sknnr_forest *forest
         if (!dev_ptrs) CK(ix->finish_slot(s));
         const uint16_t *dq;
         int64_t dld = ldq;
+        const uint32_t *dw = nullptr;    // wide mode: exact codes
+        int64_t dldw = ldq;
         if (forest) {
             // raw feature rows -> device -> forest walk -> 16-bit node codes, all on s.stream
             const void *dX;
@@ -1795,27 +1944,44 @@ static int hamming_kneighbors_impl(sknnr_hamming_index *ix, sknnr_forest *forest
                 dX = s.x.p;
                 dldx = cols;
             }
-            CK(s.codes.reserve((size_t)rows * ix->n_trees));
-            CK(launch_forest_apply(dX, x_dtype, dldx, rows, forest->n_features, forest->d_nodes,
-                                   forest->d_roots, forest->n_trees, s.codes.p, nullptr, ix->n_trees, s.stream));
-            ix->stats.kernel_launches++;
+            if ((rc = walk_forest(ix, forest, s, dX, x_dtype, dldx, rows)) != SKNNR_OK) return rc;
             dq = s.codes.p;
             dld = ix->n_trees;
-        } else if (q_on_device) {
-            dq = q_codes + (size_t)r0 * ldq;
+            dw = s.wide.p;
+            dldw = ix->n_trees;
         } else {
-            CK(s.x.reserve((size_t)rows * ix->n_trees * 2));
-            CK(cudaMemcpy2DAsync(s.x.p, (size_t)ix->n_trees * 2, q_codes + (size_t)r0 * ldq,
-                                 (size_t)ldq * 2, (size_t)ix->n_trees * 2, (size_t)rows,
-                                 cudaMemcpyHostToDevice, s.stream));
-            ix->stats.h2d_bytes += rows * ix->n_trees * 2;
-            dq = (const uint16_t *)s.x.p;
-            dld = ix->n_trees;
+            const void *dcodes;
+            if (q_on_device) {
+                dcodes = (const unsigned char *)q_codes + (size_t)r0 * ldq * code_bytes;
+            } else {
+                CK(s.x.reserve((size_t)rows * ix->n_trees * code_bytes));
+                CK(cudaMemcpy2DAsync(s.x.p, (size_t)ix->n_trees * code_bytes,
+                                     (const unsigned char *)q_codes + (size_t)r0 * ldq * code_bytes,
+                                     (size_t)ldq * code_bytes, (size_t)ix->n_trees * code_bytes, (size_t)rows,
+                                     cudaMemcpyHostToDevice, s.stream));
+                ix->stats.h2d_bytes += rows * ix->n_trees * (int64_t)code_bytes;
+                dcodes = s.x.p;
+                dld = ix->n_trees;
+            }
+            if (!wide) {
+                dq = (const uint16_t *)dcodes;
+            } else if (excl) {
+                dq = ix->d_rcodes + (size_t)r0 * ldq;   // (the reference's filter codes exist already)
+                dw = (const uint32_t *)dcodes;
+            } else {
+                dw = (const uint32_t *)dcodes;
+                dldw = dld;
+                CK(s.codes.reserve((size_t)rows * ix->n_trees));
+                CK(launch_hamming_hash(dw, rows, dldw, ix->n_trees, s.codes.p, s.stream));
+                ix->stats.kernel_launches++;
+                dq = s.codes.p;
+                dld = ix->n_trees;
+            }
         }
         ChunkOut o;
         rc = chunk_outputs(ix, s, dev_ptrs, r0, rows, k, weights, out_dist, out_idx, out_pred, o);
         if (rc != SKNNR_OK) return rc;
-        rc = run_hamming_chunk(ix, s, dq, dld, rows, row_offset + r0, k, flags, decimals, weights, o);
+        rc = run_codes_chunk(ix, s, dq, dld, dw, dldw, rows, row_offset + r0, k, flags, decimals, weights, o);
         if (rc != SKNNR_OK) return rc;
         if (!dev_ptrs) {
             if (out_dist) {
@@ -1855,13 +2021,10 @@ int sknnr_hamming_raster_kneighbors_forest(sknnr_hamming_index *ix, sknnr_forest
     return raster_impl(ix, forest->n_features, bands, x_dtype, n_pix, band_stride, use_nodata, nodata, k, flags,
                        weights, out_dist, out_idx, out_pred, fill_dist, fill_idx, fill_pred, n_valid_out,
                        [&](Slot &s, const void *xc, int64_t nv, int64_t row0, const ChunkOut &o) -> int {
-                           CK(s.codes.reserve((size_t)nv * ix->n_trees));
-                           CK(launch_forest_apply(xc, x_dtype, forest->n_features, nv,
-                                                  forest->n_features, forest->d_nodes, forest->d_roots,
-                                                  forest->n_trees, s.codes.p, nullptr, ix->n_trees, s.stream));
-                           ix->stats.kernel_launches++;
-                           return run_hamming_chunk(ix, s, s.codes.p, ix->n_trees, nv, row0, k, flags, decimals,
-                                                    weights, o);
+                           const int r = walk_forest(ix, forest, s, xc, x_dtype, forest->n_features, nv);
+                           if (r != SKNNR_OK) return r;
+                           return run_codes_chunk(ix, s, s.codes.p, ix->n_trees, s.wide.p, ix->n_trees, nv, row0,
+                                                  k, flags, decimals, weights, o);
                        });
 }
 
@@ -1869,6 +2032,16 @@ int sknnr_hamming_kneighbors(sknnr_hamming_index *ix, const uint16_t *q_codes, i
                              int64_t ldq, int64_t row_offset, int32_t k, uint32_t flags,
                              int32_t decimals, double *out_dist, int64_t *out_idx,
                              int32_t weights, double *out_pred, void *stream) {
+    if (ix && ix->d_rwide) return fail(SKNNR_EINVAL, "a wide index takes u32 codes (sknnr_hamming_kneighbors_wide)");
+    return hamming_kneighbors_impl(ix, nullptr, q_codes, 0, n_q, ldq, row_offset, k, flags, decimals,
+                                   out_dist, out_idx, weights, out_pred, stream);
+}
+
+int sknnr_hamming_kneighbors_wide(sknnr_hamming_index *ix, const uint32_t *q_codes, int64_t n_q,
+                                  int64_t ldq, int64_t row_offset, int32_t k, uint32_t flags,
+                                  int32_t decimals, double *out_dist, int64_t *out_idx,
+                                  int32_t weights, double *out_pred, void *stream) {
+    if (ix && !ix->d_rwide) return fail(SKNNR_EINVAL, "not a wide index (sknnr_hamming_kneighbors takes its u16 codes)");
     return hamming_kneighbors_impl(ix, nullptr, q_codes, 0, n_q, ldq, row_offset, k, flags, decimals,
                                    out_dist, out_idx, weights, out_pred, stream);
 }

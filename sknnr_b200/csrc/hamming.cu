@@ -428,4 +428,104 @@ cudaError_t launch_hamming_finish(const int *cand_idx, const int *cand_cnt, int 
     return cudaGetLastError();
 }
 
+// ---- wide mode: exact 32-bit codes behind the 16-bit filter ---------------------------------
+// A tree with more than 31743 distinct node IDs has no dense 16-bit coding.  The index then keeps
+// exact u32 codes and runs the kernels above on their hashed image (wide mod 31743; 0xFFFFFFFF,
+// "matches nothing", -> 31743).  Hashing only merges distinct codes, so a hashed mismatch count (or
+// fixed-point sum) never exceeds the true one: every reference outside a filter list still has a
+// true value >= the list's boundary, and hamming_wide_refine_kernel certifies against that bound.
+__global__ void __launch_bounds__(256)
+hamming_hash_kernel(const uint32_t *__restrict__ wide, long long n, long long ldw, int n_trees,
+                    uint16_t *__restrict__ codes) {
+    const long long total = n * n_trees;
+    for (long long e = (long long)blockIdx.x * 256 + threadIdx.x; e < total; e += (long long)gridDim.x * 256) {
+        const long long r = e / n_trees;
+        const int t = (int)(e - r * n_trees);
+        codes[e] = hamming_filter_code(wide[r * ldw + t]);
+    }
+}
+
+cudaError_t launch_hamming_hash(const uint32_t *wide, long long n, long long ldw, int n_trees, uint16_t *codes,
+                                cudaStream_t st) {
+    if (n <= 0) return cudaSuccess;
+    long long blocks = (n * n_trees + 255) / 256;
+    if (blocks > 148 * 16) blocks = 148 * 16;
+    hamming_hash_kernel<<<(unsigned)blocks, 256, 0, st>>>(wide, n, ldw, n_trees, codes);
+    return cudaGetLastError();
+}
+
+// One warp per query, one filter candidate per lane.  Equal weights (a.lut != null): the true
+// mismatch counts over the exact codes, ranked by (count, index); every reference outside the list
+// has a true (count, index) above the list's last (hashed) entry, so the top k are final when the
+// k-th is below it - a k-th tie with the boundary is decided by the index, exactly as the ranking
+// decides it.  Unequal weights: hamming_refine_kernel's certificate on numerators recomputed from the
+// exact codes.  Either way a list with an empty slot holds every reference.
+__global__ void __launch_bounds__(256)
+hamming_wide_refine_kernel(HammingWideRefineArgs a, FinishParams fp) {
+    // (shuffle: the compiler then knows `warp` is warp-uniform and keeps what derives from it in uniform registers)
+    const int warp = __shfl_sync(SK_FULL, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
+    const long long q = (long long)blockIdx.x * 8 + warp;
+    if (q >= a.n_q) return;
+    int id = 0x7fffffff, c = 0x7fffffff;
+    if (lane < a.kc) {
+        id = a.cand_idx[q * a.kc + lane];
+        c = a.cand_cnt[q * a.kc + lane];
+    }
+    const bool valid = id != 0x7fffffff;
+    const bool whole = __ballot_sync(SK_FULL, lane < a.kc && !valid) != 0;   // the list holds every reference
+    // the list's boundary: its largest (filter value, index)
+    int bc = valid ? c : -1, bi = valid ? id : -1;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const int oc = __shfl_xor_sync(SK_FULL, bc, o), oi = __shfl_xor_sync(SK_FULL, bi, o);
+        if (pair_less<int>(bc, bi, oc, oi)) {
+            bc = oc;
+            bi = oi;
+        }
+    }
+    const uint32_t *qc = a.qcodes + q * a.ldq;
+    const uint32_t *rc = a.rcodes + (long long)(valid ? id : 0) * a.n_trees;
+    const int kk = fp.k + (fp.exclude_self ? 1 : 0);
+    bool ok;
+    double d = SK_INF_D;
+    if (a.lut) {
+        int m = 0x7fffffff;
+        if (valid) {
+            m = 0;
+            for (int t = 0; t < a.n_trees; ++t) m += qc[t] != rc[t];
+        }
+        warp_sort_pairs<int, 32>(m, id, lane);
+        const int kc_ = __shfl_sync(SK_FULL, m, kk - 1), ki = __shfl_sync(SK_FULL, id, kk - 1);
+        ok = whole || pair_less<int>(kc_, ki, bc, bi);
+        if (id != 0x7fffffff) d = a.lut[m];
+    } else {
+        double num = SK_INF_D;
+        if (valid) {
+            double s = 0.0;
+            for (int t = 0; t < a.n_trees; ++t)
+                if (qc[t] != rc[t]) s = __dadd_rn(s, a.w[t]);
+            num = s;
+        }
+        warp_sort_pairs<double, 32>(num, id, lane);
+        const double kth = __shfl_sync(SK_FULL, num, kk - 1);
+        ok = whole || kth < a.scale * (double)bc - a.err;
+        if (id != 0x7fffffff) d = num / a.wsum;
+    }
+    if (!ok) {
+        if (lane == 0) {
+            const int pos = atomicAdd(a.fb_count, 1);
+            a.fb_list[pos] = (int)q;
+        }
+        return;
+    }
+    finish_query(fp, q, d, id, lane);
+}
+
+cudaError_t launch_hamming_wide_refine(const HammingWideRefineArgs &a, const FinishParams &fp, cudaStream_t st) {
+    if (a.n_q <= 0) return cudaSuccess;
+    const long long grid = (a.n_q + 7) / 8;
+    hamming_wide_refine_kernel<<<(unsigned)grid, 256, 0, st>>>(a, fp);
+    return cudaGetLastError();
+}
+
 }  // namespace sk

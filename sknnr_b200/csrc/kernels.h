@@ -124,7 +124,8 @@ cudaError_t launch_refine_lp(const RefineArgs &a, int metric, const FinishParams
 // Exhaustive float64 search for the rows in list[0..*count) (or all rows when list==null):
 // one CTA per row, all references, exact (distance, index) top-k, then finish_query.
 struct ExactArgs {
-    int metric;             // 0 = Euclidean (z64/ref64), 1 = weighted Hamming (codes + w), 2 = Manhattan, 3 = Chebyshev
+    int metric;             // 0 = Euclidean (z64/ref64), 1 = weighted Hamming (codes + w), 2 = Manhattan, 3 = Chebyshev,
+                            // 4 = weighted Hamming on exact u32 codes (qwide / rwide + w; wide mode)
     const double *z64;
     const double *ref64;
     int d;
@@ -141,6 +142,8 @@ struct ExactArgs {
     double *scratch;        // [grid, n_ref]
     double *big;            // [grid, 4 * (k + exclude_self)] - only read when k (+1) > 32
     int grid;
+    const uint32_t *qwide;  // metric 4: [n_q, ldq]
+    const uint32_t *rwide;  // metric 4: [n_ref, n_trees]
 };
 cudaError_t launch_exact(const ExactArgs &a, const FinishParams &fp, cudaStream_t st);
 
@@ -181,6 +184,33 @@ cudaError_t launch_hamming_refine(const HammingRefineArgs &a, const FinishParams
 cudaError_t launch_hamming_finish(const int *cand_idx, const int *cand_cnt, int kc,
                                   const double *lut, long long n_q, const FinishParams &fp,
                                   cudaStream_t st);
+// Wide mode (trees with more than 31743 distinct node IDs): exact u32 codes, 0xFFFFFFFF = "matches
+// nothing"; the 16-bit kernels above run as a filter on the hashed image of the codes.
+constexpr uint32_t WIDE_NONE = 0xFFFFFFFFu;
+__host__ __device__ inline uint16_t hamming_filter_code(uint32_t wide) {
+    return wide == WIDE_NONE ? (uint16_t)31743 : (uint16_t)(wide % 31743u);
+}
+// codes [n, n_trees] <- filter codes of wide [n, ldw]
+cudaError_t launch_hamming_hash(const uint32_t *wide, long long n, long long ldw, int n_trees, uint16_t *codes,
+                                cudaStream_t st);
+// exact (count or float64 distance) re-rank of the filter's candidates, certificate, finish_query or fb_list
+struct HammingWideRefineArgs {
+    const int *cand_idx;    // [n_q, kc]
+    const int *cand_cnt;    // [n_q, kc] hashed mismatch counts (lut != null) or fixed-point weight sums
+    int kc;
+    const uint32_t *qcodes; // [n_q, ldq] exact codes
+    long long ldq;
+    const uint32_t *rcodes; // [n_ref, n_trees] exact codes
+    int n_trees;
+    const double *lut;      // equal weights: mismatch count -> float64 distance; null: unequal weights
+    const double *w;        // [n_trees]
+    double wsum;
+    double scale, err;      // as in HammingRefineArgs (unequal weights)
+    long long n_q;
+    int *fb_count;
+    int *fb_list;
+};
+cudaError_t launch_hamming_wide_refine(const HammingWideRefineArgs &a, const FinishParams &fp, cudaStream_t st);
 
 // ---- forest.cu (RFNodeTransformer.transform on the device) -------------------------------
 // One node of the flattened forests, 16 bytes (one LDG.128).  left < 0: leaf, `right` = the 16-bit

@@ -488,8 +488,9 @@ __device__ void finish_query_block(const FinishParams &p, long long q, double *s
     __syncthreads();
 }
 
-__global__ void __launch_bounds__(EXACT_THREADS)
-exact_kernel(ExactArgs a, FinishParams fp) {
+// The exhaustive search of exact_kernel / exact_wide_kernel; pair(q, j) is the float64 distance
+template <class Pair>
+__device__ __forceinline__ void exact_search(const ExactArgs &a, const FinishParams &fp, Pair pair) {
     __shared__ double red_d[EXACT_THREADS / 32];
     __shared__ int red_i[EXACT_THREADS / 32];
     __shared__ double sel_d_s[MAXK];
@@ -508,7 +509,7 @@ exact_kernel(ExactArgs a, FinishParams fp) {
 
     for (long long it = blockIdx.x; it < n_rows; it += gridDim.x) {
         const long long q = a.list ? (long long)a.list[it] : it;
-        for (int j = threadIdx.x; j < a.n_ref; j += EXACT_THREADS) scr[j] = exact_pair(a, q, j);
+        for (int j = threadIdx.x; j < a.n_ref; j += EXACT_THREADS) scr[j] = pair(q, j);
         __syncthreads();
         double last_d = -1.0;
         int last_i = -1;
@@ -568,9 +569,31 @@ exact_kernel(ExactArgs a, FinishParams fp) {
     }
 }
 
+__global__ void __launch_bounds__(EXACT_THREADS)
+exact_kernel(ExactArgs a, FinishParams fp) {
+    exact_search(a, fp, [&](long long q, int j) { return exact_pair(a, q, j); });
+}
+
+// metric 4: weighted Hamming on exact u32 codes, the same left-to-right float64 sum as exact_pair
+__global__ void __launch_bounds__(EXACT_THREADS)
+exact_wide_kernel(ExactArgs a, FinishParams fp) {
+    exact_search(a, fp, [&](long long q, int j) {
+        const uint32_t *qc = a.qwide + q * a.ldq;
+        const uint32_t *rc = a.rwide + (long long)j * a.n_trees;
+        double num = 0.0;
+        for (int t = 0; t < a.n_trees; ++t) {
+            if (qc[t] != rc[t]) num = __dadd_rn(num, a.w[t]);
+        }
+        return num / a.wsum;
+    });
+}
+
 cudaError_t launch_exact(const ExactArgs &a, const FinishParams &fp, cudaStream_t st) {
     if (a.grid <= 0) return cudaSuccess;
-    exact_kernel<<<a.grid, EXACT_THREADS, 0, st>>>(a, fp);
+    if (a.metric == 4)
+        exact_wide_kernel<<<a.grid, EXACT_THREADS, 0, st>>>(a, fp);
+    else
+        exact_kernel<<<a.grid, EXACT_THREADS, 0, st>>>(a, fp);
     return cudaGetLastError();
 }
 

@@ -15,6 +15,7 @@ import numpy as np
 from sklearn.utils.validation import check_is_fitted
 
 from . import _lib as L
+from ._base import _forest_tables
 
 __all__ = ["kneighbors_raster", "predict_raster"]
 
@@ -40,7 +41,7 @@ def _regressor_and_image(est, image):
             raise NotImplementedError("the estimator's transformer is not an affine map")
         query = ix.query_raster
     elif hasattr(est, "transformer_") and est._forest_fusable():
-        forest = est.transformer_._forest_index(reg.__dict__.get("_node_tables"))
+        forest = est.transformer_._forest_index(_forest_tables(reg.__dict__.get("_node_tables")))
         query = lambda bands, k, **kw: ix.query_raster_forest(forest, bands, k, **kw)  # noqa: E731
     else:
         raise NotImplementedError(
