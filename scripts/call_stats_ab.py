@@ -7,7 +7,8 @@ call run several chunks, so the host pipeline, its ramp, the slot rotation and t
 all take part.  Entry points: host-buffer and device-pointer kneighbors on float64 / float32 / int16
 rows, SKNNR_EXCLUDE_SELF, SKNNR_CHECK_FINITE (clean and with a NaN), a k beyond the filtered engines,
 raster calls of both index kinds, Hamming queries on node codes (host and device pointers, equal and
-unequal tree weights) and through a device forest walk, transform and both weighted averages.
+unequal tree weights, 16-bit and wide indexes of the same node IDs) and through a device forest walk,
+transform and both weighted averages.
 
     python scripts/call_stats_ab.py LIB_A LIB_B [--repeats N] [--out FILE]
 
@@ -24,6 +25,7 @@ from __future__ import annotations
 
 import argparse
 import hashlib
+import itertools
 import json
 import os
 import subprocess
@@ -123,14 +125,17 @@ def record() -> dict:
     Xf = rng.standard_normal((n_q, n_feat))
     qcodes = forest.apply(Xf).astype(np.uint16)
     out["forest_apply"] = {"out": digest(qcodes)}
-    for wname, w in (("equal", np.full(40, 1.0 / 40)), ("unequal", rng.uniform(0.5, 1.5, 40))):
-        hx = HammingIndex(codes, w, y)
+    tree_weights = (("equal", np.full(40, 1.0 / 40)), ("unequal", rng.uniform(0.5, 1.5, 40)))
+    # the wide legs: the same node IDs as exact u32 codes (wide mode's filter and re-rank)
+    for (wname, w), wide in itertools.product(tree_weights, (False, True)):
+        hq = qcodes.astype(np.uint32) if wide else qcodes
+        hx = HammingIndex(codes.astype(np.uint32) if wide else codes, w, y)
 
         def ham(name, call):
-            keep(f"hamming_{wname}_{name}", call(), hx, False)
+            keep(f"hamming_{'wide_' if wide else ''}{wname}_{name}", call(), hx, False)
 
-        ham("codes_host", lambda: hx.query(qcodes, k, weights="distance", with_pred=True))
-        qd = torch.from_numpy(qcodes.astype(np.int16)).cuda()
+        ham("codes_host", lambda: hx.query(hq, k, weights="distance", with_pred=True))
+        qd = torch.from_numpy(qcodes.astype(np.int32 if wide else np.int16)).cuda()
         res = [torch.empty((n_q, k), dtype=torch.float64, device="cuda"),
                torch.empty((n_q, k), dtype=torch.int64, device="cuda")]
 
@@ -147,7 +152,7 @@ def record() -> dict:
         fb = np.ascontiguousarray(rng.standard_normal((n_feat, 30_000)))
         fb[:, rng.random(30_000) < 0.1] = np.nan
         ham("raster_forest", lambda: hx.query_raster_forest(forest, fb, k, weights="distance", with_pred=True))
-        hd, hi, _ = hx.query(qcodes[:10_000], k)
+        hd, hi, _ = hx.query(hq[:10_000], k)
         ham("weighted_average", lambda: hx.weighted_average(hi, 1.0 / (1.0 + hd)))
         hx.close()
     forest.close()

@@ -1688,28 +1688,46 @@ int sknnr_hamming_index_cascade_counts(sknnr_hamming_index *ix, int64_t *out3) {
     return SKNNR_OK;
 }
 
-static int run_hamming_chunk(sknnr_hamming_index *ix, Slot &s, const uint16_t *dq, int64_t ldq,
-                             int64_t rows, int64_t row0, int k, uint32_t flags, int decimals,
-                             int weights, const ChunkOut &o) {
+// One chunk's query codes on the device: dq the 16-bit codes the search runs on (row stride ldq); in
+// wide mode dq holds the filter codes of dw, the exact codes (row stride ldw)
+struct QueryCodes {
+    const uint16_t *dq;
+    int64_t ldq;
+    const uint32_t *dw = nullptr;
+    int64_t ldw = 0;
+};
+
+// The search of one chunk.  Wide mode: the 16-bit search runs on the filter codes, and
+// hamming_refine_kernel re-ranks its candidates on the exact codes and certifies them.  The rows it
+// cannot certify (and every row when no filtered engine serves the call) go to the exhaustive kernel
+// on the exact codes.
+static int run_hamming_chunk(sknnr_hamming_index *ix, Slot &s, const QueryCodes &c, int64_t rows, int64_t row0,
+                             int k, uint32_t flags, int decimals, int weights, const ChunkOut &o) {
     const bool excl = flags & SKNNR_EXCLUDE_SELF;
     const int kk = k + (excl ? 1 : 0);
     cudaStream_t st = s.stream;
     const FinishParams fp = finish_params(ix, k, flags, decimals, weights, row0, o);
+    const bool wide = ix->d_rwide != nullptr;
 
-    // equal weights: integer counts are exact, kc = k suffices.  Unequal weights: the fixed-point
-    // filter keeps >= 8 spare candidates for the certificate of hamming_refine_kernel.
+    // equal weights: 16-bit counts are exact, kc = k suffices; wide mode's hashed counts need spare
+    // candidates for the certificate of hamming_refine_kernel, like the unequal weights' fixed-point
+    // filter: lists of >= k (+1) + 8.
     const bool exact_only = g_opt.engine == SKNNR_ENGINE_EXACT;
-    const int kc_u = pick_kc(kk, 0);
+    const int kc_u = pick_kc(kk, wide ? 8 : 0);
     const int kc_w = std::max(16, pick_kc(kk, 8));
     const bool fast_u = ix->uniform && kc_u != 0 && ix->n_chunks * HAM_WC <= 2048 && !exact_only;
     const bool fast_w = !fast_u && !ix->uniform && ix->wq_ok && pick_kc(kk, 8) != 0 && !exact_only;
     ix->stats.engine = (fast_u || fast_w) ? SKNNR_ENGINE_SIMT : SKNNR_ENGINE_EXACT;
 
+    // the exact codes: the searched codes themselves, or wide mode's u32 codes
+    const void *qx = wide ? (const void *)c.dw : c.dq;
+    const int64_t ldx = wide ? c.ldw : c.ldq;
+    const void *rx = wide ? (const void *)ix->d_rwide : ix->d_rcodes;
     ExactArgs ea{};
-    ea.metric = 1;
-    ea.qcodes = dq;
-    ea.ldq = ldq;
-    ea.rcodes = ix->d_rcodes;
+    ea.metric = wide ? 4 : 1;
+    ea.qcodes = qx;
+    ea.ldq = ldx;
+    ea.rcodes = rx;
     ea.n_trees = ix->n_trees;
     ea.w = ix->d_w;
     ea.wsum = ix->wsum;
@@ -1729,12 +1747,12 @@ static int run_hamming_chunk(sknnr_hamming_index *ix, Slot &s, const uint16_t *d
     CK(s.qimg_h.reserve((size_t)n_qtiles * ix->n_chunks * HAM_WC * QTILE));
     CK(s.cand_idx.reserve((size_t)rows * kc));
     CK(s.cand_cnt.reserve((size_t)rows * kc));
-    CK(launch_hamming_pack(dq, rows, ldq, ix->n_trees, ix->n_chunks, QTILE, 31743, s.qimg_h.p, st));
+    CK(launch_hamming_pack(c.dq, rows, c.ldq, ix->n_trees, ix->n_chunks, QTILE, 31743, s.qimg_h.p, st));
     if (g_opt.timing) CK(s.mark(st));
     CK(launch_hamming_search(s.qimg_h.p, ix->d_rimg, fast_w ? ix->d_wq : nullptr, ix->n_chunks, ix->n_rtiles,
                              rows, (int)ix->n_ref, kc, s.cand_idx.p, s.cand_cnt.p, st));
     if (g_opt.timing) CK(s.mark(st));
-    if (fast_u) {
+    if (fast_u && !wide) {
         CK(launch_hamming_finish(s.cand_idx.p, s.cand_cnt.p, kc, ix->d_lut, rows, fp, st));
         ix->stats.kernel_launches += 3;
         return SKNNR_OK;
@@ -1745,10 +1763,11 @@ static int run_hamming_chunk(sknnr_hamming_index *ix, Slot &s, const uint16_t *d
     ha.cand_idx = s.cand_idx.p;
     ha.cand_cnt = s.cand_cnt.p;
     ha.kc = kc;
-    ha.qcodes = dq;
-    ha.ldq = ldq;
-    ha.rcodes = ix->d_rcodes;
+    ha.qcodes = qx;
+    ha.ldq = ldx;
+    ha.rcodes = rx;
     ha.n_trees = ix->n_trees;
+    ha.lut = fast_u ? ix->d_lut : nullptr;
     ha.w = ix->d_w;
     ha.wsum = ix->wsum;
     ha.scale = ix->wq_scale;
@@ -1756,7 +1775,7 @@ static int run_hamming_chunk(sknnr_hamming_index *ix, Slot &s, const uint16_t *d
     ha.n_q = rows;
     ha.fb_count = s.fb.p;
     ha.fb_list = s.fb.p + 1;
-    CK(launch_hamming_refine(ha, fp, st));
+    CK(launch_hamming_refine(ha, wide, fp, st));
     // exhaustive float64 search of the uncertified rows
     ea.list = s.fb.p + 1;
     ea.count = s.fb.p;
@@ -1769,99 +1788,13 @@ static int run_hamming_chunk(sknnr_hamming_index *ix, Slot &s, const uint16_t *d
     return SKNNR_OK;
 }
 
-// Wide mode: the 16-bit search runs on the filter codes dq; hamming_wide_refine_kernel re-ranks its
-// candidates on the exact codes dw and certifies them; the rows it cannot certify (and every row when
-// k (+1) > 24) go to the exhaustive kernel on the exact codes.
-static int run_hamming_wide_chunk(sknnr_hamming_index *ix, Slot &s, const uint16_t *dq, int64_t ldq,
-                                  const uint32_t *dw, int64_t ldw, int64_t rows, int64_t row0, int k,
-                                  uint32_t flags, int decimals, int weights, const ChunkOut &o) {
-    const bool excl = flags & SKNNR_EXCLUDE_SELF;
-    const int kk = k + (excl ? 1 : 0);
-    cudaStream_t st = s.stream;
-    const FinishParams fp = finish_params(ix, k, flags, decimals, weights, row0, o);
-
-    // both certificates need spare candidates: lists of >= k (+1) + 8
-    const bool exact_only = g_opt.engine == SKNNR_ENGINE_EXACT;
-    const int kc8 = pick_kc(kk, 8);
-    const bool fast_u = ix->uniform && kc8 != 0 && ix->n_chunks * HAM_WC <= 2048 && !exact_only;
-    const bool fast_w = !fast_u && !ix->uniform && ix->wq_ok && kc8 != 0 && !exact_only;
-    ix->stats.engine = (fast_u || fast_w) ? SKNNR_ENGINE_SIMT : SKNNR_ENGINE_EXACT;
-
-    ExactArgs ea{};
-    ea.metric = 4;
-    ea.qwide = dw;
-    ea.ldq = ldw;
-    ea.rwide = ix->d_rwide;
-    ea.n_trees = ix->n_trees;
-    ea.w = ix->d_w;
-    ea.wsum = ix->wsum;
-    ea.n_q = rows;
-    ea.n_ref = (int)ix->n_ref;
-    ea.grid = ix->exact_ctas(rows);
-    if (!fast_u && !fast_w) {
-        if (g_opt.timing) CK(s.mark(st));
-        CK(ix->launch_exact_chained(ea, fp, kk, st));
-        if (g_opt.timing) CK(s.mark(st));
-        ix->stats.kernel_launches++;
-        ix->n_exact_rows += rows;
-        return SKNNR_OK;
-    }
-    const int kc = fast_u ? kc8 : std::max(16, kc8);
-    const int64_t n_qtiles = (rows + QTILE - 1) / QTILE;
-    CK(s.qimg_h.reserve((size_t)n_qtiles * ix->n_chunks * HAM_WC * QTILE));
-    CK(s.cand_idx.reserve((size_t)rows * kc));
-    CK(s.cand_cnt.reserve((size_t)rows * kc));
-    CK(launch_hamming_pack(dq, rows, ldq, ix->n_trees, ix->n_chunks, QTILE, 31743, s.qimg_h.p, st));
-    if (g_opt.timing) CK(s.mark(st));
-    CK(launch_hamming_search(s.qimg_h.p, ix->d_rimg, fast_w ? ix->d_wq : nullptr, ix->n_chunks, ix->n_rtiles,
-                             rows, (int)ix->n_ref, kc, s.cand_idx.p, s.cand_cnt.p, st));
-    if (g_opt.timing) CK(s.mark(st));
-    CK(s.fb.reserve((size_t)rows + 1));
-    CK(cudaMemsetAsync(s.fb.p, 0, sizeof(int), st));
-    HammingWideRefineArgs ha{};
-    ha.cand_idx = s.cand_idx.p;
-    ha.cand_cnt = s.cand_cnt.p;
-    ha.kc = kc;
-    ha.qcodes = dw;
-    ha.ldq = ldw;
-    ha.rcodes = ix->d_rwide;
-    ha.n_trees = ix->n_trees;
-    ha.lut = fast_u ? ix->d_lut : nullptr;
-    ha.w = ix->d_w;
-    ha.wsum = ix->wsum;
-    ha.scale = ix->wq_scale;
-    ha.err = ix->wq_err;
-    ha.n_q = rows;
-    ha.fb_count = s.fb.p;
-    ha.fb_list = s.fb.p + 1;
-    CK(launch_hamming_wide_refine(ha, fp, st));
-    ea.list = s.fb.p + 1;
-    ea.count = s.fb.p;
-    CK(ix->launch_exact_chained(ea, fp, kk, st));
-    CK(cudaMemcpyAsync(&s.h_fb[0], s.fb.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-    s.h_fb[1] = 0;
-    s.fb_pending = true;
-    s.rows_in_flight = 0;
-    ix->stats.kernel_launches += 4;
-    return SKNNR_OK;
-}
-
-// The search of one chunk of query codes: dq the 16-bit codes (row stride ldq); in wide mode dw the
-// exact codes (row stride ldw) and dq their filter codes
-static int run_codes_chunk(sknnr_hamming_index *ix, Slot &s, const uint16_t *dq, int64_t ldq,
-                           const uint32_t *dw, int64_t ldw, int64_t rows, int64_t row0, int k,
-                           uint32_t flags, int decimals, int weights, const ChunkOut &o) {
-    if (ix->d_rwide)
-        return run_hamming_wide_chunk(ix, s, dq, ldq, dw, ldw, rows, row0, k, flags, decimals, weights, o);
-    return run_hamming_chunk(ix, s, dq, ldq, rows, row0, k, flags, decimals, weights, o);
-}
-
-// Forest walk of `rows` feature rows x (row stride ldx) to the index's query codes, on s.stream:
+// Forest walk of `rows` feature rows x (row stride ldx) to the index's query codes c, on s.stream:
 // s.codes holds the 16-bit codes; in wide mode s.wide holds the node IDs (the exact codes) and
 // s.codes their filter codes
 static int walk_forest(sknnr_hamming_index *ix, sknnr_forest *forest, Slot &s, const void *x,
-                       int32_t x_dtype, int64_t ldx, int64_t rows) {
+                       int32_t x_dtype, int64_t ldx, int64_t rows, QueryCodes &c) {
     CK(s.codes.reserve((size_t)rows * ix->n_trees));
+    c = {s.codes.p, ix->n_trees};
     if (!ix->d_rwide) {
         CK(launch_forest_apply(x, x_dtype, ldx, rows, forest->n_features, forest->d_nodes, forest->d_roots,
                                forest->n_trees, s.codes.p, nullptr, ix->n_trees, s.stream));
@@ -1869,6 +1802,8 @@ static int walk_forest(sknnr_hamming_index *ix, sknnr_forest *forest, Slot &s, c
         return SKNNR_OK;
     }
     CK(s.wide.reserve((size_t)rows * ix->n_trees));
+    c.dw = s.wide.p;
+    c.ldw = ix->n_trees;
     CK(launch_forest_apply(x, x_dtype, ldx, rows, forest->n_features, forest->d_nodes, forest->d_roots,
                            forest->n_trees, nullptr, (int *)s.wide.p, ix->n_trees, s.stream));
     CK(launch_hamming_hash(s.wide.p, rows, ix->n_trees, ix->n_trees, s.codes.p, s.stream));
@@ -1924,12 +1859,9 @@ static int hamming_kneighbors_impl(sknnr_hamming_index *ix, sknnr_forest *forest
         const int64_t rows = std::min(chunk, n_q - r0);
         Slot &s = dev_ptrs ? ix->slots[0] : ix->slots[ci % IndexBase::kSlots];
         if (!dev_ptrs) CK(ix->finish_slot(s));
-        const uint16_t *dq;
-        int64_t dld = ldq;
-        const uint32_t *dw = nullptr;    // wide mode: exact codes
-        int64_t dldw = ldq;
+        QueryCodes c;
         if (forest) {
-            // raw feature rows -> device -> forest walk -> 16-bit node codes, all on s.stream
+            // raw feature rows -> device -> forest walk -> the index's query codes, all on s.stream
             const void *dX;
             int64_t dldx = ldq;
             if (q_on_device) {
@@ -1944,13 +1876,10 @@ static int hamming_kneighbors_impl(sknnr_hamming_index *ix, sknnr_forest *forest
                 dX = s.x.p;
                 dldx = cols;
             }
-            if ((rc = walk_forest(ix, forest, s, dX, x_dtype, dldx, rows)) != SKNNR_OK) return rc;
-            dq = s.codes.p;
-            dld = ix->n_trees;
-            dw = s.wide.p;
-            dldw = ix->n_trees;
+            if ((rc = walk_forest(ix, forest, s, dX, x_dtype, dldx, rows, c)) != SKNNR_OK) return rc;
         } else {
             const void *dcodes;
+            int64_t dld = ldq;
             if (q_on_device) {
                 dcodes = (const unsigned char *)q_codes + (size_t)r0 * ldq * code_bytes;
             } else {
@@ -1963,25 +1892,22 @@ static int hamming_kneighbors_impl(sknnr_hamming_index *ix, sknnr_forest *forest
                 dcodes = s.x.p;
                 dld = ix->n_trees;
             }
+            const uint32_t *dw = (const uint32_t *)dcodes;
             if (!wide) {
-                dq = (const uint16_t *)dcodes;
+                c = {(const uint16_t *)dcodes, dld};
             } else if (excl) {
-                dq = ix->d_rcodes + (size_t)r0 * ldq;   // (the reference's filter codes exist already)
-                dw = (const uint32_t *)dcodes;
+                c = {ix->d_rcodes + (size_t)r0 * ldq, ldq, dw, ldq};   // (the reference's filter codes exist already)
             } else {
-                dw = (const uint32_t *)dcodes;
-                dldw = dld;
                 CK(s.codes.reserve((size_t)rows * ix->n_trees));
-                CK(launch_hamming_hash(dw, rows, dldw, ix->n_trees, s.codes.p, s.stream));
+                CK(launch_hamming_hash(dw, rows, dld, ix->n_trees, s.codes.p, s.stream));
                 ix->stats.kernel_launches++;
-                dq = s.codes.p;
-                dld = ix->n_trees;
+                c = {s.codes.p, ix->n_trees, dw, dld};
             }
         }
         ChunkOut o;
         rc = chunk_outputs(ix, s, dev_ptrs, r0, rows, k, weights, out_dist, out_idx, out_pred, o);
         if (rc != SKNNR_OK) return rc;
-        rc = run_codes_chunk(ix, s, dq, dld, dw, dldw, rows, row_offset + r0, k, flags, decimals, weights, o);
+        rc = run_hamming_chunk(ix, s, c, rows, row_offset + r0, k, flags, decimals, weights, o);
         if (rc != SKNNR_OK) return rc;
         if (!dev_ptrs) {
             if (out_dist) {
@@ -2021,10 +1947,10 @@ int sknnr_hamming_raster_kneighbors_forest(sknnr_hamming_index *ix, sknnr_forest
     return raster_impl(ix, forest->n_features, bands, x_dtype, n_pix, band_stride, use_nodata, nodata, k, flags,
                        weights, out_dist, out_idx, out_pred, fill_dist, fill_idx, fill_pred, n_valid_out,
                        [&](Slot &s, const void *xc, int64_t nv, int64_t row0, const ChunkOut &o) -> int {
-                           const int r = walk_forest(ix, forest, s, xc, x_dtype, forest->n_features, nv);
+                           QueryCodes c;
+                           const int r = walk_forest(ix, forest, s, xc, x_dtype, forest->n_features, nv, c);
                            if (r != SKNNR_OK) return r;
-                           return run_codes_chunk(ix, s, s.codes.p, ix->n_trees, s.wide.p, ix->n_trees, nv, row0,
-                                                  k, flags, decimals, weights, o);
+                           return run_hamming_chunk(ix, s, c, nv, row0, k, flags, decimals, weights, o);
                        });
 }
 

@@ -472,4 +472,16 @@ __device__ __forceinline__ void finish_query(const FinishParams &p, long long q,
     finish_query_w<32>(p, q, dist, id, lane, true);
 }
 
+// Numerator of SciPy's weighted Hamming distance: the left-to-right float64 sum of w_t over the
+// trees whose codes differ ($SP/scipy/spatial/distance.py:1718-1723 -> cdist_hamming).  Code is
+// uint16_t (dense node codes) or uint32_t (wide mode's exact codes).
+template <class Code>
+__device__ __forceinline__ double hamming_numerator(const Code *qc, const Code *rc, int n_trees,
+                                                    const double *w) {
+    double s = 0.0;
+    for (int t = 0; t < n_trees; ++t)
+        if (qc[t] != rc[t]) s = __dadd_rn(s, w[t]);
+    return s;
+}
+
 }  // namespace sk

@@ -350,57 +350,6 @@ cudaError_t launch_hamming_search(const uint32_t *qimg, const uint32_t *rimg, co
     }
 }
 
-// ---- unequal weights: float64 distances of the candidates + certificate --------------------
-// One warp per query, one candidate per lane.  The distance is SciPy's: left-to-right float64 sum
-// of w_t over the mismatching trees, divided by the left-to-right sum of all w_t.  Every reference
-// outside the list has a fixed-point sum >= the largest one in the list (amax), hence a true
-// numerator >= scale * amax - err; the top k are final when the k-th exact numerator is below that.
-__global__ void __launch_bounds__(256)
-hamming_refine_kernel(HammingRefineArgs a, FinishParams fp) {
-    // (shuffle: the compiler then knows `warp` is warp-uniform and keeps what derives from it in uniform registers)
-    const int warp = __shfl_sync(SK_FULL, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
-    const long long q = (long long)blockIdx.x * 8 + warp;
-    if (q >= a.n_q) return;
-    int id = 0x7fffffff, aq = 0;
-    if (lane < a.kc) {
-        id = a.cand_idx[q * a.kc + lane];
-        aq = a.cand_cnt[q * a.kc + lane];
-    }
-    const bool valid = id != 0x7fffffff;
-    double num = SK_INF_D;
-    if (valid) {
-        const uint16_t *qc = a.qcodes + q * a.ldq;
-        const uint16_t *rc = a.rcodes + (long long)id * a.n_trees;
-        double s = 0.0;
-        for (int t = 0; t < a.n_trees; ++t)
-            if (qc[t] != rc[t]) s = __dadd_rn(s, a.w[t]);
-        num = s;
-    }
-    int amax = valid ? aq : 0;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) amax = max(amax, __shfl_xor_sync(SK_FULL, amax, o));
-    const bool whole = __ballot_sync(SK_FULL, lane < a.kc && !valid) != 0;   // the list holds every reference
-    warp_sort_pairs<double, 32>(num, id, lane);
-    const int kk = fp.k + (fp.exclude_self ? 1 : 0);
-    const double kth = __shfl_sync(SK_FULL, num, kk - 1);
-    const bool ok = whole || kth < a.scale * (double)amax - a.err;
-    if (!ok) {
-        if (lane == 0) {
-            const int pos = atomicAdd(a.fb_count, 1);
-            a.fb_list[pos] = (int)q;
-        }
-        return;
-    }
-    finish_query(fp, q, id != 0x7fffffff ? num / a.wsum : SK_INF_D, id, lane);
-}
-
-cudaError_t launch_hamming_refine(const HammingRefineArgs &a, const FinishParams &fp, cudaStream_t st) {
-    if (a.n_q <= 0) return cudaSuccess;
-    const long long grid = (a.n_q + 7) / 8;
-    hamming_refine_kernel<<<(unsigned)grid, 256, 0, st>>>(a, fp);
-    return cudaGetLastError();
-}
-
 // ---- counts -> float64 distances, then the common epilogue ------------------------------
 __global__ void __launch_bounds__(256)
 hamming_finish_kernel(const int *__restrict__ cand_idx, const int *__restrict__ cand_cnt, int kc,
@@ -433,7 +382,7 @@ cudaError_t launch_hamming_finish(const int *cand_idx, const int *cand_cnt, int 
 // exact u32 codes and runs the kernels above on their hashed image (wide mod 31743; 0xFFFFFFFF,
 // "matches nothing", -> 31743).  Hashing only merges distinct codes, so a hashed mismatch count (or
 // fixed-point sum) never exceeds the true one: every reference outside a filter list still has a
-// true value >= the list's boundary, and hamming_wide_refine_kernel certifies against that bound.
+// true value >= the list's boundary, and hamming_refine_kernel certifies against that bound.
 __global__ void __launch_bounds__(256)
 hamming_hash_kernel(const uint32_t *__restrict__ wide, long long n, long long ldw, int n_trees,
                     uint16_t *__restrict__ codes) {
@@ -454,14 +403,22 @@ cudaError_t launch_hamming_hash(const uint32_t *wide, long long n, long long ldw
     return cudaGetLastError();
 }
 
-// One warp per query, one filter candidate per lane.  Equal weights (a.lut != null): the true
-// mismatch counts over the exact codes, ranked by (count, index); every reference outside the list
-// has a true (count, index) above the list's last (hashed) entry, so the top k are final when the
-// k-th is below it - a k-th tie with the boundary is decided by the index, exactly as the ranking
-// decides it.  Unequal weights: hamming_refine_kernel's certificate on numerators recomputed from the
-// exact codes.  Either way a list with an empty slot holds every reference.
+// ---- re-rank of the filter's candidates on the exact codes + certificate -------------------
+// One warp per query, one filter candidate per lane; Code is the type of the exact codes (uint16_t:
+// the searched codes themselves, uint32_t: wide mode).  The list's boundary is its largest (filter
+// value, index).
+// Unequal weights: the distance is SciPy's, the left-to-right float64 sum of w_t over the mismatching
+// trees divided by the left-to-right sum of all w_t.  Every reference outside the list has a
+// fixed-point sum >= the boundary's (bc), hence a true numerator >= scale * bc - err; the top k are
+// final when the k-th exact numerator is below that.
+// Equal weights (a.lut != null, wide mode only; 16-bit counts are exact and go to
+// hamming_finish_kernel): the true mismatch counts, ranked by (count, index); every reference outside
+// the list has a true (count, index) above the boundary, so the top k are final when the k-th is
+// below it - a k-th tie with the boundary is decided by the index, exactly as the ranking decides it.
+// Either way a list with an empty slot holds every reference.
+template <class Code>
 __global__ void __launch_bounds__(256)
-hamming_wide_refine_kernel(HammingWideRefineArgs a, FinishParams fp) {
+hamming_refine_kernel(HammingRefineArgs a, FinishParams fp) {
     // (shuffle: the compiler then knows `warp` is warp-uniform and keeps what derives from it in uniform registers)
     const int warp = __shfl_sync(SK_FULL, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
     const long long q = (long long)blockIdx.x * 8 + warp;
@@ -483,8 +440,8 @@ hamming_wide_refine_kernel(HammingWideRefineArgs a, FinishParams fp) {
             bi = oi;
         }
     }
-    const uint32_t *qc = a.qcodes + q * a.ldq;
-    const uint32_t *rc = a.rcodes + (long long)(valid ? id : 0) * a.n_trees;
+    const Code *qc = static_cast<const Code *>(a.qcodes) + q * a.ldq;
+    const Code *rc = static_cast<const Code *>(a.rcodes) + (long long)(valid ? id : 0) * a.n_trees;
     const int kk = fp.k + (fp.exclude_self ? 1 : 0);
     bool ok;
     double d = SK_INF_D;
@@ -500,12 +457,7 @@ hamming_wide_refine_kernel(HammingWideRefineArgs a, FinishParams fp) {
         if (id != 0x7fffffff) d = a.lut[m];
     } else {
         double num = SK_INF_D;
-        if (valid) {
-            double s = 0.0;
-            for (int t = 0; t < a.n_trees; ++t)
-                if (qc[t] != rc[t]) s = __dadd_rn(s, a.w[t]);
-            num = s;
-        }
+        if (valid) num = hamming_numerator(qc, rc, a.n_trees, a.w);
         warp_sort_pairs<double, 32>(num, id, lane);
         const double kth = __shfl_sync(SK_FULL, num, kk - 1);
         ok = whole || kth < a.scale * (double)bc - a.err;
@@ -521,10 +473,13 @@ hamming_wide_refine_kernel(HammingWideRefineArgs a, FinishParams fp) {
     finish_query(fp, q, d, id, lane);
 }
 
-cudaError_t launch_hamming_wide_refine(const HammingWideRefineArgs &a, const FinishParams &fp, cudaStream_t st) {
+cudaError_t launch_hamming_refine(const HammingRefineArgs &a, bool wide, const FinishParams &fp, cudaStream_t st) {
     if (a.n_q <= 0) return cudaSuccess;
     const long long grid = (a.n_q + 7) / 8;
-    hamming_wide_refine_kernel<<<(unsigned)grid, 256, 0, st>>>(a, fp);
+    if (wide)
+        hamming_refine_kernel<uint32_t><<<(unsigned)grid, 256, 0, st>>>(a, fp);
+    else
+        hamming_refine_kernel<uint16_t><<<(unsigned)grid, 256, 0, st>>>(a, fp);
     return cudaGetLastError();
 }
 

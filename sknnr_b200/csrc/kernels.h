@@ -124,13 +124,13 @@ cudaError_t launch_refine_lp(const RefineArgs &a, int metric, const FinishParams
 // Exhaustive float64 search for the rows in list[0..*count) (or all rows when list==null):
 // one CTA per row, all references, exact (distance, index) top-k, then finish_query.
 struct ExactArgs {
-    int metric;             // 0 = Euclidean (z64/ref64), 1 = weighted Hamming (codes + w), 2 = Manhattan, 3 = Chebyshev,
-                            // 4 = weighted Hamming on exact u32 codes (qwide / rwide + w; wide mode)
+    int metric;             // 0 = Euclidean (z64/ref64), 2 = Manhattan, 3 = Chebyshev; weighted Hamming
+                            // (codes + w): 1 = uint16_t codes, 4 = uint32_t codes (wide mode)
     const double *z64;
     const double *ref64;
     int d;
-    const uint16_t *qcodes; // [n_q, ldq]
-    const uint16_t *rcodes; // [n_ref, n_trees]
+    const void *qcodes;     // [n_q, ldq]
+    const void *rcodes;     // [n_ref, n_trees]
     int n_trees;
     long long ldq;
     const double *w;        // [n_trees]
@@ -142,8 +142,6 @@ struct ExactArgs {
     double *scratch;        // [grid, n_ref]
     double *big;            // [grid, 4 * (k + exclude_self)] - only read when k (+1) > 32
     int grid;
-    const uint32_t *qwide;  // metric 4: [n_q, ldq]
-    const uint32_t *rwide;  // metric 4: [n_ref, n_trees]
 };
 cudaError_t launch_exact(const ExactArgs &a, const FinishParams &fp, cudaStream_t st);
 
@@ -163,23 +161,6 @@ cudaError_t launch_hamming_pack(const uint16_t *codes, long long n, long long ld
 cudaError_t launch_hamming_search(const uint32_t *qimg, const uint32_t *rimg, const uint32_t *wq,
                                   int n_chunks, int n_rtiles, long long n_q, int n_ref, int kc,
                                   int *cand_idx, int *cand_cnt, cudaStream_t st);
-// unequal weights: exact float64 distances of the candidates, certificate, finish_query or fb_list
-struct HammingRefineArgs {
-    const int *cand_idx;    // [n_q, kc]
-    const int *cand_cnt;    // [n_q, kc] fixed-point weight sums
-    int kc;
-    const uint16_t *qcodes; // [n_q, ldq]
-    long long ldq;
-    const uint16_t *rcodes; // [n_ref, n_trees]
-    int n_trees;
-    const double *w;        // [n_trees]
-    double wsum;            // left-to-right float64 sum of w
-    double scale, err;      // w_t = scale * wq_t + e_t, err >= sum |e_t| + float64 summation slack
-    long long n_q;
-    int *fb_count;
-    int *fb_list;
-};
-cudaError_t launch_hamming_refine(const HammingRefineArgs &a, const FinishParams &fp, cudaStream_t st);
 // mismatch counts -> float64 distances through the host-built table, then finish_query
 cudaError_t launch_hamming_finish(const int *cand_idx, const int *cand_cnt, int kc,
                                   const double *lut, long long n_q, const FinishParams &fp,
@@ -194,23 +175,24 @@ __host__ __device__ inline uint16_t hamming_filter_code(uint32_t wide) {
 cudaError_t launch_hamming_hash(const uint32_t *wide, long long n, long long ldw, int n_trees, uint16_t *codes,
                                 cudaStream_t st);
 // exact (count or float64 distance) re-rank of the filter's candidates, certificate, finish_query or fb_list
-struct HammingWideRefineArgs {
+struct HammingRefineArgs {
     const int *cand_idx;    // [n_q, kc]
-    const int *cand_cnt;    // [n_q, kc] hashed mismatch counts (lut != null) or fixed-point weight sums
+    const int *cand_cnt;    // [n_q, kc] fixed-point weight sums, or hashed mismatch counts (lut != null)
     int kc;
-    const uint32_t *qcodes; // [n_q, ldq] exact codes
+    const void *qcodes;     // [n_q, ldq] exact codes: uint16_t, or uint32_t in wide mode
     long long ldq;
-    const uint32_t *rcodes; // [n_ref, n_trees] exact codes
+    const void *rcodes;     // [n_ref, n_trees] exact codes, the same type
     int n_trees;
-    const double *lut;      // equal weights: mismatch count -> float64 distance; null: unequal weights
+    const double *lut;      // wide mode, equal weights: mismatch count -> float64 distance; null: unequal weights
     const double *w;        // [n_trees]
-    double wsum;
-    double scale, err;      // as in HammingRefineArgs (unequal weights)
+    double wsum;            // left-to-right float64 sum of w
+    double scale, err;      // w_t = scale * wq_t + e_t, err >= sum |e_t| + float64 summation slack
     long long n_q;
     int *fb_count;
     int *fb_list;
 };
-cudaError_t launch_hamming_wide_refine(const HammingWideRefineArgs &a, const FinishParams &fp, cudaStream_t st);
+// wide: the codes are uint32_t
+cudaError_t launch_hamming_refine(const HammingRefineArgs &a, bool wide, const FinishParams &fp, cudaStream_t st);
 
 // ---- forest.cu (RFNodeTransformer.transform on the device) -------------------------------
 // One node of the flattened forests, 16 bytes (one LDG.128).  left < 0: leaf, `right` = the 16-bit

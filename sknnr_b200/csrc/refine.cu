@@ -7,7 +7,8 @@
 //                    same for lists of <= 16 candidates with two queries per warp;
 //   refine_lp_kernel - the same for Manhattan / Chebyshev indexes, one lane per candidate;
 //   exact_kernel   - exhaustive float64 search for the rows whose certificate failed (and the
-//                    engine for shapes the fast kernels do not cover / unequal Hamming weights);
+//                    engine for shapes the fast kernels do not cover); exact_hamming_kernel is the
+//                    same for the weighted Hamming distance of node codes;
 //   weighted_average_kernel - seam S3 with caller-supplied weights.
 //
 // The reference computes distances from the float64 expansion |x|^2 - 2x.y + |y|^2
@@ -390,23 +391,13 @@ cudaError_t launch_refine_lp(const RefineArgs &a, int metric, const FinishParams
 // ---------------------------------------------------------------------------------------
 constexpr int EXACT_THREADS = 256;
 
+// metric 0, 2 or 3
 __device__ __forceinline__ double exact_pair(const ExactArgs &a, long long q, int j) {
-    if (a.metric != 1) {
-        const double *zq = a.z64 + q * a.d;
-        const double *r = a.ref64 + (long long)j * a.d;
-        if (a.metric == 2) return dist_lp<METRIC_L1>(zq, r, a.d);
-        if (a.metric == 3) return dist_lp<METRIC_LINF>(zq, r, a.d);
-        return dist2_serial(zq, r, a.d);
-    }
-    // weighted Hamming: left-to-right float64 sum of w_t over mismatching trees / sum(w)
-    // ($SP/scipy/spatial/distance.py:1718-1723 -> cdist_hamming)
-    const uint16_t *qc = a.qcodes + q * a.ldq;
-    const uint16_t *rc = a.rcodes + (long long)j * a.n_trees;
-    double num = 0.0;
-    for (int t = 0; t < a.n_trees; ++t) {
-        if (qc[t] != rc[t]) num = __dadd_rn(num, a.w[t]);
-    }
-    return num / a.wsum;
+    const double *zq = a.z64 + q * a.d;
+    const double *r = a.ref64 + (long long)j * a.d;
+    if (a.metric == 2) return dist_lp<METRIC_L1>(zq, r, a.d);
+    if (a.metric == 3) return dist_lp<METRIC_LINF>(zq, r, a.d);
+    return dist2_serial(zq, r, a.d);
 }
 
 // finish_query for k (+1) > 32, by the whole CTA: the kk selected neighbours arrive ascending by
@@ -488,7 +479,7 @@ __device__ void finish_query_block(const FinishParams &p, long long q, double *s
     __syncthreads();
 }
 
-// The exhaustive search of exact_kernel / exact_wide_kernel; pair(q, j) is the float64 distance
+// The exhaustive search of exact_kernel / exact_hamming_kernel; pair(q, j) is the float64 distance
 template <class Pair>
 __device__ __forceinline__ void exact_search(const ExactArgs &a, const FinishParams &fp, Pair pair) {
     __shared__ double red_d[EXACT_THREADS / 32];
@@ -574,24 +565,23 @@ exact_kernel(ExactArgs a, FinishParams fp) {
     exact_search(a, fp, [&](long long q, int j) { return exact_pair(a, q, j); });
 }
 
-// metric 4: weighted Hamming on exact u32 codes, the same left-to-right float64 sum as exact_pair
+// metric 1 (Code = uint16_t) or 4 (uint32_t): SciPy's weighted Hamming distance
+template <class Code>
 __global__ void __launch_bounds__(EXACT_THREADS)
-exact_wide_kernel(ExactArgs a, FinishParams fp) {
+exact_hamming_kernel(ExactArgs a, FinishParams fp) {
     exact_search(a, fp, [&](long long q, int j) {
-        const uint32_t *qc = a.qwide + q * a.ldq;
-        const uint32_t *rc = a.rwide + (long long)j * a.n_trees;
-        double num = 0.0;
-        for (int t = 0; t < a.n_trees; ++t) {
-            if (qc[t] != rc[t]) num = __dadd_rn(num, a.w[t]);
-        }
-        return num / a.wsum;
+        return hamming_numerator(static_cast<const Code *>(a.qcodes) + q * a.ldq,
+                                 static_cast<const Code *>(a.rcodes) + (long long)j * a.n_trees, a.n_trees,
+                                 a.w) / a.wsum;
     });
 }
 
 cudaError_t launch_exact(const ExactArgs &a, const FinishParams &fp, cudaStream_t st) {
     if (a.grid <= 0) return cudaSuccess;
-    if (a.metric == 4)
-        exact_wide_kernel<<<a.grid, EXACT_THREADS, 0, st>>>(a, fp);
+    if (a.metric == 1)
+        exact_hamming_kernel<uint16_t><<<a.grid, EXACT_THREADS, 0, st>>>(a, fp);
+    else if (a.metric == 4)
+        exact_hamming_kernel<uint32_t><<<a.grid, EXACT_THREADS, 0, st>>>(a, fp);
     else
         exact_kernel<<<a.grid, EXACT_THREADS, 0, st>>>(a, fp);
     return cudaGetLastError();

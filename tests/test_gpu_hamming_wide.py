@@ -1,7 +1,7 @@
 """Wide Hamming mode on the device: trees with more than 31,743 distinct node IDs keep exact 32-bit
 codes, the 16-bit search runs as a filter on their hashed image, and a float64 re-rank certifies its
 candidates.  Every result is compared bit for bit with SciPy's weighted Hamming distances ranked by
-stable (distance, index), then sknnr's ordering."""
+stable (distance, index), then sknnr's ordering, or with a 16-bit index of the same codes."""
 
 import numpy as np
 import pytest
@@ -209,6 +209,52 @@ def test_forest_raster_int16_equals_row_query(forest_fit):
     assert (i.reshape(5, -1)[:, ~valid] == -1).all()
     p = predict_raster(est, img, nodata=-999)
     assert np.array_equal(p.reshape(1, -1)[:, valid].ravel(), est.predict(rows))
+
+
+@pytest.fixture(scope="module")
+def small_forest():
+    from sklearn.ensemble import RandomForestRegressor
+
+    from sknnr_b200._engine import ForestIndex
+
+    rng = np.random.default_rng(8)
+    X = rng.standard_normal((6000, 6))
+    y = X[:, :2] @ rng.standard_normal((2, 2)) + 0.1 * rng.standard_normal((6000, 2))
+    rf = RandomForestRegressor(n_estimators=24, max_depth=9, random_state=0).fit(X[:5000], y[:5000])
+    forest = ForestIndex([e.tree_ for e in rf.estimators_], 6)   # no code tables: leaves carry their node IDs
+    yield forest, X[:5000], y[:5000], X[5000:]
+    forest.close()
+
+
+@pytest.mark.parametrize("k", [1, 7, 40])
+@pytest.mark.parametrize("unequal", [False, True])
+def test_wide_index_of_16_bit_codes_equals_16_bit_index(small_forest, unequal, k):
+    """Node IDs that all fit 16 bits, searched by a 16-bit index and by a wide index of the same IDs as
+    u32: distances, indices and predictions are bit-identical, for node-code queries, X=None and the
+    forest walk."""
+    from sknnr_b200._engine import HammingIndex
+
+    forest, Xr, y, Xq = small_forest
+    codes, qcodes = forest.apply(Xr), forest.apply(Xq)
+    assert codes.max() < 31743
+    T = codes.shape[1]
+    w = np.random.default_rng(3).uniform(0.5, 1.5, T) if unequal else np.full(T, 1.0 / T)
+    narrow = HammingIndex(codes.astype(np.uint16), w, y)
+    wide = HammingIndex(codes.astype(np.uint32), w, y)
+    assert wide.wide and not narrow.wide
+    try:
+        calls = [
+            lambda ix, c: ix.query(qcodes.astype(c), k, weights="distance", with_pred=True),
+            lambda ix, c: ix.query(None, k, exclude_self=True, weights="uniform", with_pred=True),
+            lambda ix, c: ix.query_forest(forest, Xq, k, weights="distance", with_pred=True),
+        ]
+        for call in calls:
+            a, b = call(narrow, np.uint16), call(wide, np.uint32)
+            for u, v in zip(a, b):
+                assert np.array_equal(u, v)
+    finally:
+        narrow.close()
+        wide.close()
 
 
 def test_forest_two_devices_equal_one(forest_fit, monkeypatch):
